@@ -3,7 +3,7 @@
 
     python bench.py [--gpus N] [--steps K] [--warmup W] [--impl ours|reference]
                     [--n 1000000] [--dim 128] [--nq 10000] [--k 10] [--ef 64] [--m 16]
-                    [--graph reference|quality] [--sweep]
+                    [--graph reference|quality] [--sweep] [--dump-outputs DIR]
 
 A "step" is one pass of the hot path (zvdb_search_batch_device: one launch of the layer-0
 best-first kernel) over one batch of nq synthetic Gaussian queries against an index of n
@@ -30,6 +30,7 @@ import numpy as np
 ROOT = os.path.dirname(os.path.abspath(__file__))
 if ROOT not in sys.path:
     sys.path.insert(0, ROOT)
+sys.dont_write_bytecode = True      # the benchmark leaves the tree as it found it (it may be read-only)
 
 METRIC = "batched search QPS at recall@10 (1M x 128 fp32)"
 QUERY_BATCHES = 4   # distinct query batches rotated over the steps
@@ -100,7 +101,15 @@ def parse_args():
                                                            "ef sweep) and the K4 timing that the default line carries")
     p.add_argument("--parity-queries", type=int, default=1000, help="queries of batch 0 checked bit for bit against the oracle "
                                                                     "(at N>1: N oracle shard indexes + the oracle merge) after the timed region")
-    return p.parse_args()
+    p.add_argument("--dump-outputs", metavar="DIR", default=None,
+                   help="write what the last timed step returned (ids, dist, counts; at N=1 also pops, evals) as DIR/<name>.npy "
+                        "in float32 / float64, so that two builds can be compared output for output on the same seeded inputs")
+    args = p.parse_args()
+    if args.steps < 1 or args.warmup < 0:
+        p.error("--steps must be >= 1 and --warmup >= 0")
+    if args.dump_outputs and args.impl != "ours":
+        p.error("--dump-outputs writes the GPU path's results; it applies to --impl ours")
+    return args
 
 
 def make_data(n, dim, nq, seed_x=1, seed_q=2):
@@ -207,6 +216,27 @@ def recall_at_k(ids, gt):
     return hit / (len(gt) * k)
 
 
+DUMP_BYTES = 64 << 20
+
+
+def dump_outputs(path, outs):
+    """Write each per-query array of `outs` as path/<name>.npy: float32 arrays as they are, integer ones as float64
+    (exact below 2**53; an empty id slot, -1, stays -1). When that would pass DUMP_BYTES, the same rows of every array
+    are written for a fixed, seeded sample of the queries, and their indexes as rows.npy."""
+    arrs = {name: np.asarray(a, np.float32 if a.dtype == np.float32 else np.float64) for name, a in outs.items()}
+    nq = len(next(iter(arrs.values())))
+    row_bytes = sum(a[:1].nbytes for a in arrs.values())
+    budget = DUMP_BYTES - 4096 * (len(arrs) + 1)          # headroom for the .npy headers
+    if row_bytes * nq > budget:
+        rows = np.sort(np.random.default_rng(0).choice(nq, size=budget // (row_bytes + 8), replace=False))
+        arrs = {name: a[rows] for name, a in arrs.items()}
+        arrs["rows"] = rows.astype(np.float64)
+    os.makedirs(path, exist_ok=True)
+    for name, a in arrs.items():
+        np.save(os.path.join(path, name + ".npy"), a)
+    log(f"[dump] {', '.join(f'{n}{list(a.shape)}' for n, a in arrs.items())} -> {path}")
+
+
 def algorithmic_bytes(evals, pops, row_bytes, m, dim, k):
     """SURVEY 8d: gathered rows + adjacency rows + query + output, per query, summed."""
     return int(evals.astype(np.int64).sum()) * row_bytes + int(pops.astype(np.int64).sum()) * m * 4 + \
@@ -271,7 +301,7 @@ def run_reference(args):
         return
     world = max(1, int(os.environ.get("WORLD_SIZE", str(args.gpus))))
     from oracle import oracle as O
-    O.build()
+    O.lib()
     threads = host_threads()
     X, Qs = make_data(args.n, args.dim, args.nq)
     t0 = time.time()
@@ -624,6 +654,9 @@ def run_ours(args):
         ends[s].record()
     barrier()
     wall = time.perf_counter() - t_wall
+    if args.dump_outputs and rank == 0:       # the last timed step's results, before later passes reuse these buffers
+        outs = (m_ids, m_dist, m_cnt) if world > 1 else (d_ids, d_dist, d_cnt, d_pops, d_evals)
+        dump_outputs(args.dump_outputs, {name: t_.cpu().numpy() for name, t_ in zip(("ids", "dist", "counts", "pops", "evals"), outs)})
     dev_ms = starts[0].elapsed_time(ends[-1])             # device time of the whole K-step region
     kern_ms = [starts[s].elapsed_time(ends[s]) for s in range(args.steps)]
     step_ms = list(kern_ms)                               # per-step device times on rank 0 (min / median go into config)
@@ -763,7 +796,7 @@ def run_ours(args):
     kw = {}
     if not args.shard_gen and args.parity_queries > 0:
         from oracle import oracle as O
-        O.build()
+        O.lib()
         chk = min(args.parity_queries, nq)
         if args.descent:
             lv_, ub_, ua_ = h.export_upper_layers()
@@ -801,7 +834,7 @@ def run_ours(args):
     if world == 1 and not args.no_cpu and not args.shard_gen:
         if O is None:
             from oracle import oracle as O
-            O.build()
+            O.lib()
             if args.descent:
                 lv_, ub_, ua_ = h.export_upper_layers()
                 kw["upper"] = (lv_, ub_, ua_, h.max_level, h.descent_start)
