@@ -157,6 +157,30 @@ ZVDB_API int zvdb_export_upper_layers(const zvdb_index *ix, uint8_t *levels, uin
 ZVDB_API int zvdb_load_upper_layers(zvdb_index *ix, const uint8_t *levels, const uint32_t *upper_adj,
                                     uint64_t n_lists, uint64_t start);
 
+/* ---- vector storage of the graph search --------------------------------------------------------
+ * ZVDB_STORAGE_F16: the graph search gathers an fp16 copy of the rows (half the bytes per evaluated
+ * row) and re-ranks what it found in fp32. The device then holds the fp32 rows AND a __half copy
+ * (cap_rows x row_floats x 2 bytes, rounded to nearest even, filled by one kernel from the fp32 rows
+ * when a search finds rows it does not cover); exact k-NN, save / load and zvdb_get_point keep using
+ * the fp32 rows. Under F16 every plain search entry point (zvdb_search, zvdb_search_batch on pageable
+ * or page-locked buffers, zvdb_search_batch_device, zvdb_search_batch_packed_device):
+ *   - traverses exactly as search(q, ef) does on the f16-rounded rows (the descent too): pops and
+ *     evals are that traversal's;
+ *   - re-scores the whole popped set (count = min(ef, reachable) ids) with the fp32 distance on the
+ *     fp32 rows, orders it by (exact distance, id) -- the order of exact k-NN and of the shard merge --
+ *     and returns the first min(k, count): distances are the fp32 distances of those (query, id).
+ * Coordinates that round to +-inf in fp16 (|x| >= 65520) fail the search with ZVDB_ERR_UNSUPPORTED
+ * naming the first such row; setting ZVDB_STORAGE_F32 recovers the handle. Coordinates below the fp16
+ * normal range (|x| < 6.1e-5) become subnormal or zero in the copy: a precision loss of the traversal
+ * only, the returned distances stay exact. Refused with ZVDB_ERR_UNSUPPORTED: F16 on an f64 / i32
+ * index, and zvdb_search_batch_exchange / _exchange_host on an F16 handle. The setting may change at
+ * any time and applies from the next search; ZVDB_STORAGE_F32 frees the copy. zvdb_save does not
+ * store it (nor the descent or the kernel variant): zvdb_load keeps the handle's setting, a new handle starts at F32. */
+#define ZVDB_STORAGE_F32 0   /* default: the search gathers the fp32 rows */
+#define ZVDB_STORAGE_F16 1   /* the search gathers an fp16 copy of the rows; results are re-ranked in fp32 */
+ZVDB_API int zvdb_set_storage(zvdb_index *ix, int storage);
+ZVDB_API int zvdb_storage(const zvdb_index *ix);
+
 /* ---- on-disk format (SURVEY 8f rank 3; the reference has no persistence) --------------------------
  * zvdb_save writes the whole index -- vectors in the device layout, every layer, entry point, level
  * generator state -- to one file ending in a checksum; zvdb_load replaces the contents of `ix` (which

@@ -29,6 +29,8 @@ extern fn zvdb_search_typed(ix: *zvdb_index, query: *const anyopaque, dim: u32, 
 extern fn zvdb_search_batch_typed(ix: *zvdb_index, queries: *const anyopaque, nq: u64, dim: u32, dtype: c_int, k: u32, ef: u32, ids: [*]u64, dist: [*]f32, counts: [*]u32) c_int;
 extern fn zvdb_get_point_typed(ix: *const zvdb_index, id: u64) ?*const anyopaque;
 extern fn zvdb_set_descent(ix: *zvdb_index, on: c_int) c_int;
+extern fn zvdb_set_storage(ix: *zvdb_index, storage: c_int) c_int;
+extern fn zvdb_storage(ix: *const zvdb_index) c_int;
 extern fn zvdb_save(ix: *const zvdb_index, path: [*:0]const u8) c_int;
 extern fn zvdb_load(ix: *zvdb_index, path: [*:0]const u8) c_int;
 extern fn zvdb_alloc_host(bytes: usize) ?*anyopaque;
@@ -139,6 +141,19 @@ pub fn HNSW(comptime T: type) type {
         pub fn setDescent(self: *Self, on: bool) !void {
             const h = self.handle orelse return error.CudaError;
             try check(zvdb_set_descent(h, @intFromBool(on)));
+        }
+
+        /// Extension: which rows the graph search gathers. `.f16` = an fp16 copy of the rows (half the bytes per
+        /// evaluated row); the popped set is re-scored in fp32, so returned distances are exact. Takes effect at the
+        /// next search; not stored by `save`.
+        pub const Storage = enum(c_int) { f32 = 0, f16 = 1 };
+        pub fn setStorage(self: *Self, storage: Storage) !void {
+            const h = self.handle orelse return error.CudaError;
+            try check(zvdb_set_storage(h, @intFromEnum(storage)));
+        }
+        pub fn storage(self: *const Self) Storage {
+            const h = self.handle orelse return .f32;
+            return if (zvdb_storage(h) == 1) .f16 else .f32;
         }
 
         /// Extension: the whole index to / from one file (the reference has no persistence).

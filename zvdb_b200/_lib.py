@@ -14,6 +14,7 @@ LIB_PATH = os.environ.get("ZVDB_B200_LIB") or os.path.join(_HERE, "lib", "libzvd
 
 OK, ERR_OOM, ERR_NODE_NOT_FOUND, ERR_DIM_MISMATCH, ERR_CUDA, ERR_INVALID, ERR_UNSUPPORTED = range(7)
 METRIC_L2, METRIC_COSINE, METRIC_DOT = 0, 1, 2
+STORAGE_F32, STORAGE_F16 = 0, 1
 INVALID_ID = 0xFFFFFFFFFFFFFFFF
 
 _u32, _u64, _i32, _i64, _vp = C.c_uint32, C.c_uint64, C.c_int, C.c_int64, C.c_void_p
@@ -44,6 +45,8 @@ SIGNATURES = {
     "zvdb_build_from_candidates": (_i32, [_vp, _pf, _u64, _u32, _vp, _u32, _i32]),
     "zvdb_set_descent": (_i32, [_vp, _i32]),
     "zvdb_descent_start": (_i64, [_vp]),
+    "zvdb_set_storage": (_i32, [_vp, _i32]),
+    "zvdb_storage": (_i32, [_vp]),
     "zvdb_export_upper_layers": (_i32, [_vp, _vp, _vp, _vp, _pu64]),
     "zvdb_load_upper_layers": (_i32, [_vp, _vp, _vp, _u64, _u64]),
     "zvdb_save": (_i32, [_vp, C.c_char_p]),

@@ -1,6 +1,9 @@
 """Build libzvdb_b200.so in-tree with nvcc for sm_100a (explicit -gencode, -lineinfo).
 
-    python -m zvdb_b200.build [--force] [--verbose]
+    python -m zvdb_b200.build [--force] [--verbose] [--define NAME=VALUE ...] [--out PATH]
+
+--define / --out build a variant of the library for an A/B run (e.g. --define ZVDB_F16_UNROLL=2 --out build/u2/libzvdb_b200.so,
+then ZVDB_B200_LIB=build/u2/libzvdb_b200.so points the binding at it); without them the in-tree library is built.
 
 The library is plain CUDA C++ behind a C ABI (include/zvdb_b200.h); it does not link torch.
 """
@@ -41,24 +44,32 @@ def _stale() -> bool:
     return any(os.path.getmtime(d) > t for d in deps)
 
 
-def build(force: bool = False, verbose: bool = False) -> str:
-    if not force and not _stale():
+def build(force: bool = False, verbose: bool = False, defines=(), out: str = "") -> str:
+    out = os.path.abspath(out) if out else LIB_PATH
+    if out == LIB_PATH and not defines and not force and not _stale():
         return LIB_PATH
-    os.makedirs(LIB_DIR, exist_ok=True)
-    cmd = [_nvcc(), *NVCC_FLAGS]
+    os.makedirs(os.path.dirname(out), exist_ok=True)
+    cmd = [_nvcc(), *NVCC_FLAGS] + [f"-D{d}" for d in defines]
     if verbose:
         cmd += ["-Xptxas", "-v"]
     # the image's CC/CXX point at a wrapper; let nvcc use the system g++
     if os.path.exists("/usr/bin/g++"):
         cmd += ["-ccbin", "/usr/bin/g++"]
-    cmd += ["-o", LIB_PATH] + [os.path.join(CSRC, s) for s in SOURCES]
+    cmd += ["-o", out] + [os.path.join(CSRC, s) for s in SOURCES]
     r = subprocess.run(cmd, capture_output=True, text=True)
     if verbose or r.returncode:
         sys.stderr.write(r.stdout + r.stderr)
     if r.returncode:
         raise RuntimeError("nvcc failed building libzvdb_b200.so")
-    return LIB_PATH
+    return out
 
 
 if __name__ == "__main__":
-    print(build(force="--force" in sys.argv, verbose="--verbose" in sys.argv))
+    import argparse
+    ap = argparse.ArgumentParser()
+    ap.add_argument("--force", action="store_true")
+    ap.add_argument("--verbose", action="store_true")
+    ap.add_argument("--define", action="append", default=[], metavar="NAME=VALUE", help="preprocessor definition (variant builds)")
+    ap.add_argument("--out", default="", help="where to write the library (default: the in-tree zvdb_b200/lib/libzvdb_b200.so)")
+    a = ap.parse_args()
+    print(build(force=a.force, verbose=a.verbose, defines=a.define, out=a.out))

@@ -49,6 +49,22 @@ __global__ void scatter_adj_rows_kernel(uint32_t *__restrict__ adj, const uint32
     }
 }
 
+// F16 storage: rows [r0, r1) of the fp32 arena rounded to nearest even into the f16 copy (pitch row_floats in both). The
+// one range check of the f16 path: the first row with a coordinate that rounds to +-inf (|x| >= 65520) goes to *bad_row
+// (atomicMin; ~0 = none), and the search that triggered the conversion refuses to run.
+__global__ void arena_to_f16_kernel(uint2 *__restrict__ dst, const float4 *__restrict__ src, uint64_t r0, uint64_t r1,
+                                    uint32_t row_chunks, uint32_t *__restrict__ bad_row) {
+    const uint64_t begin = r0 * row_chunks, end = r1 * row_chunks;
+    for (uint64_t i = begin + blockIdx.x * static_cast<uint64_t>(blockDim.x) + threadIdx.x; i < end;
+         i += static_cast<uint64_t>(gridDim.x) * blockDim.x) {
+        const float4 v = src[i];
+        const __half2 a = __floats2half2_rn(v.x, v.y), b = __floats2half2_rn(v.z, v.w);
+        if (__hisinf(__low2half(a)) | __hisinf(__high2half(a)) | __hisinf(__low2half(b)) | __hisinf(__high2half(b)))
+            atomicMin(bad_row, static_cast<uint32_t>(i / row_chunks));
+        dst[i] = make_uint2(*reinterpret_cast<const uint32_t *>(&a), *reinterpret_cast<const uint32_t *>(&b));
+    }
+}
+
 template <typename T>
 struct DevBuf {
     T *p = nullptr;
@@ -89,6 +105,10 @@ struct zvdb_index {
     uint32_t *d_adj = nullptr;      // [cap_rows][m]
     uint64_t cap_rows = 0, n_dev = 0;
     uint32_t cap_row_floats = 0, cap_m = 0;   // row layout d_arena / d_adj were sized for (a load may change dim)
+    int storage = ZVDB_STORAGE_F32; // rows the graph search gathers (zvdb_set_storage)
+    uint2 *d_arena16 = nullptr;     // ZVDB_STORAGE_F16: [cap_rows][row_floats] __half copy of d_arena, rows [0, f16_rows) current
+    uint64_t f16_rows = 0;
+    DevBuf<uint32_t> f16_bad;       // first row the conversion found out of the f16 range (~0 = none)
     DevBuf<float> q_buf, dist_buf;
     DevBuf<uint64_t> ids_buf;
     DevBuf<uint32_t> cnt_buf, pops_buf, evals_buf, scat_rows, scat_ids, bitmap_buf, vlog_buf;
@@ -134,6 +154,10 @@ static int ensure_capacity(zvdb_index *ix, uint64_t rows) {
         ix->d_arena = nullptr; ix->d_adj = nullptr; ix->cap_rows = 0; ix->n_dev = 0; ix->bf_rows = 0;
         ix->cap_row_floats = g.row_floats; ix->cap_m = g.m;
     }
+    if (ix->d_arena16) {                                  // the f16 copy is sized like the arena: the next F16 search rebuilds it
+        ZV_CUDA(cudaDeviceSynchronize());
+        cudaFree(ix->d_arena16); ix->d_arena16 = nullptr; ix->f16_rows = 0;
+    }
     uint64_t nc = std::max<uint64_t>(rows, std::max<uint64_t>(ix->cap_rows * 2, 1024));
     float *na = nullptr; uint32_t *nj = nullptr;
     ZV_CUDA(cudaMalloc(&na, nc * g.row_floats * sizeof(float)));
@@ -160,6 +184,7 @@ static int sync_device_locked(zvdb_index *ix) {
     if (ix->n_dev) ZV_CUDA(cudaDeviceSynchronize());
     int rc = ensure_capacity(ix, g.n);
     if (rc) return rc;
+    ix->f16_rows = std::min<uint64_t>(ix->f16_rows, g.rows_uploaded);   // rows from rows_uploaded on are (re)written now
     for (uint64_t r = g.rows_uploaded; r < g.n;) {
         const uint64_t chunk = r / g.rows_per_chunk;
         const uint64_t end = std::min<uint64_t>(g.n, (chunk + 1) * g.rows_per_chunk);
@@ -195,6 +220,38 @@ static int sync_device_locked(zvdb_index *ix) {
     return ZVDB_OK;
 }
 
+// ZVDB_STORAGE_F16: bring the f16 copy of the arena up to the device rows (after sync_device_locked): allocated at the
+// arena's capacity, rows [f16_rows, n_dev) converted by one kernel. A row out of the f16 range fails the search that got
+// here (and every later one under F16, since f16_rows stays behind it); zvdb_set_storage(F32) recovers the handle.
+static int sync_f16_locked(zvdb_index *ix) {
+    const HostGraph &g = ix->g;
+    if (g.dtype != 0) return fail(ZVDB_ERR_UNSUPPORTED, "f16 storage: the index holds f64 / i32 rows; set ZVDB_STORAGE_F32");
+    if (ix->f16_rows >= ix->n_dev) return ZVDB_OK;
+    if (!ix->d_arena16) {
+        ZV_CUDA(cudaMalloc(&ix->d_arena16, ix->cap_rows * g.row_floats * 2));
+        ix->f16_rows = 0;
+    }
+    ZV_CUDA(ix->f16_bad.reserve(1));
+    ZV_CUDA(cudaMemsetAsync(ix->f16_bad.p, 0xFF, sizeof(uint32_t), ix->stream));
+    const uint32_t row_chunks = g.row_floats / 4;
+    const uint64_t total = (ix->n_dev - ix->f16_rows) * row_chunks;
+    const unsigned blocks = static_cast<unsigned>(std::min<uint64_t>((total + 255) / 256, static_cast<uint64_t>(ix->num_sms) * 8));
+    arena_to_f16_kernel<<<blocks, 256, 0, ix->stream>>>(ix->d_arena16, reinterpret_cast<const float4 *>(ix->d_arena), ix->f16_rows,
+                                                        ix->n_dev, row_chunks, ix->f16_bad.p);
+    ix->launches++;
+    ZV_CUDA(cudaGetLastError());
+    uint32_t bad = ~0u;
+    ZV_CUDA(cudaMemcpyAsync(&bad, ix->f16_bad.p, sizeof bad, cudaMemcpyDeviceToHost, ix->stream));
+    ZV_CUDA(cudaStreamSynchronize(ix->stream));
+    if (bad != ~0u) {
+        char buf[200];
+        snprintf(buf, sizeof buf, "f16 storage: row %u has a coordinate that rounds to +-inf in fp16 (|x| >= 65520); set ZVDB_STORAGE_F32 to search this index", bad);
+        return fail(ZVDB_ERR_UNSUPPORTED, buf);
+    }
+    ix->f16_rows = ix->n_dev;
+    return ZVDB_OK;
+}
+
 // Device copy of layers >= 1 for the descent (K2): levels[n], upper_base[n], upper_adj[n_lists][m].
 // Re-sent whole whenever a list above layer 0 changed (half the nodes have one; the reference links
 // one neighbour per layer and insert, hnsw.zig:106-108).
@@ -222,9 +279,9 @@ static int sync_upper_locked(zvdb_index *ix) {
 
 // ---- K1 launch ------------------------------------------------------------------------------
 
-template <int CPL, int METRIC, int VIS, bool EXCH>
+template <int CPL, int METRIC, int VIS, bool EXCH, int ROWF>
 static cudaError_t launch_search_inst(const SearchParams &p, unsigned grid, size_t smem, cudaStream_t s) {
-    auto kern = search_layer0_kernel<CPL, METRIC, VIS, EXCH>;
+    auto kern = search_layer0_kernel<CPL, METRIC, VIS, EXCH, ROWF>;
     if (smem > 48 * 1024) {
         cudaError_t e = cudaFuncSetAttribute(kern, cudaFuncAttributeMaxDynamicSharedMemorySize, static_cast<int>(smem));
         if (e != cudaSuccess) return e;
@@ -233,57 +290,64 @@ static cudaError_t launch_search_inst(const SearchParams &p, unsigned grid, size
     return cudaGetLastError();
 }
 
-template <int METRIC, int VIS, bool EXCH>
+template <int METRIC, int VIS, bool EXCH, int ROWF>
 static cudaError_t launch_search_metric(int cpl, const SearchParams &p, unsigned grid, size_t smem, cudaStream_t s) {
     switch (cpl) {
-        case 1: return launch_search_inst<1, METRIC, VIS, EXCH>(p, grid, smem, s);
-        case 2: return launch_search_inst<2, METRIC, VIS, EXCH>(p, grid, smem, s);
-        case 4: return launch_search_inst<4, METRIC, VIS, EXCH>(p, grid, smem, s);
-        case 6: return launch_search_inst<6, METRIC, VIS, EXCH>(p, grid, smem, s);
-        case 8: return launch_search_inst<8, METRIC, VIS, EXCH>(p, grid, smem, s);
+        case 1: return launch_search_inst<1, METRIC, VIS, EXCH, ROWF>(p, grid, smem, s);
+        case 2: return launch_search_inst<2, METRIC, VIS, EXCH, ROWF>(p, grid, smem, s);
+        case 4: return launch_search_inst<4, METRIC, VIS, EXCH, ROWF>(p, grid, smem, s);
+        case 6: return launch_search_inst<6, METRIC, VIS, EXCH, ROWF>(p, grid, smem, s);
+        case 8: return launch_search_inst<8, METRIC, VIS, EXCH, ROWF>(p, grid, smem, s);
     }
     return cudaErrorInvalidValue;
 }
 
-template <int VIS, bool EXCH>
+template <int VIS, bool EXCH, int ROWF>
 static cudaError_t launch_search_vis2(int metric, int cpl, const SearchParams &p, unsigned grid, size_t smem, cudaStream_t s) {
     switch (metric) {
-        case 0: return launch_search_metric<kMetricL2, VIS, EXCH>(cpl, p, grid, smem, s);
-        case 1: return launch_search_metric<kMetricCos, VIS, EXCH>(cpl, p, grid, smem, s);
-        default: return launch_search_metric<kMetricDot, VIS, EXCH>(cpl, p, grid, smem, s);
+        case 0: return launch_search_metric<kMetricL2, VIS, EXCH, ROWF>(cpl, p, grid, smem, s);
+        case 1: return launch_search_metric<kMetricCos, VIS, EXCH, ROWF>(cpl, p, grid, smem, s);
+        default: return launch_search_metric<kMetricDot, VIS, EXCH, ROWF>(cpl, p, grid, smem, s);
     }
 }
 
-// exch = any sharded form of the step (peer stores, records, flags, merge tail): its own instantiation, see the kernel
+// exch = any sharded form of the step (peer stores, records, flags, merge tail): its own instantiation, see the kernel.
+// f16 = the plain search over the f16 copy with the exact re-rank (never together with exch: the entry points refuse it).
 template <int VIS>
-static cudaError_t launch_search_vis(bool exch, int metric, int cpl, const SearchParams &p, unsigned grid, size_t smem, cudaStream_t s) {
-    return exch ? launch_search_vis2<VIS, true>(metric, cpl, p, grid, smem, s) : launch_search_vis2<VIS, false>(metric, cpl, p, grid, smem, s);
+static cudaError_t launch_search_vis(bool exch, bool f16, int metric, int cpl, const SearchParams &p, unsigned grid, size_t smem, cudaStream_t s) {
+    if (f16) return launch_search_vis2<VIS, false, kRowF16>(metric, cpl, p, grid, smem, s);
+    return exch ? launch_search_vis2<VIS, true, kRowF32>(metric, cpl, p, grid, smem, s) : launch_search_vis2<VIS, false, kRowF32>(metric, cpl, p, grid, smem, s);
 }
 
-template <int METRIC>
+template <int METRIC, int ROWF>
 static cudaError_t launch_descend_metric(int cpl, const SearchParams &p, unsigned grid, cudaStream_t s) {
     switch (cpl) {
-        case 1: descend_kernel<1, METRIC><<<grid, 128, 0, s>>>(p); break;
-        case 2: descend_kernel<2, METRIC><<<grid, 128, 0, s>>>(p); break;
-        case 4: descend_kernel<4, METRIC><<<grid, 128, 0, s>>>(p); break;
-        case 6: descend_kernel<6, METRIC><<<grid, 128, 0, s>>>(p); break;
-        case 8: descend_kernel<8, METRIC><<<grid, 128, 0, s>>>(p); break;
+        case 1: descend_kernel<1, METRIC, ROWF><<<grid, 128, 0, s>>>(p); break;
+        case 2: descend_kernel<2, METRIC, ROWF><<<grid, 128, 0, s>>>(p); break;
+        case 4: descend_kernel<4, METRIC, ROWF><<<grid, 128, 0, s>>>(p); break;
+        case 6: descend_kernel<6, METRIC, ROWF><<<grid, 128, 0, s>>>(p); break;
+        case 8: descend_kernel<8, METRIC, ROWF><<<grid, 128, 0, s>>>(p); break;
         default: return cudaErrorInvalidValue;
     }
     return cudaGetLastError();
 }
-static cudaError_t launch_descend(int metric, int cpl, const SearchParams &p, unsigned grid, cudaStream_t s) {
+template <int ROWF>
+static cudaError_t launch_descend_rowf(int metric, int cpl, const SearchParams &p, unsigned grid, cudaStream_t s) {
     switch (metric) {
-        case 0: return launch_descend_metric<kMetricL2>(cpl, p, grid, s);
-        case 1: return launch_descend_metric<kMetricCos>(cpl, p, grid, s);
-        default: return launch_descend_metric<kMetricDot>(cpl, p, grid, s);
+        case 0: return launch_descend_metric<kMetricL2, ROWF>(cpl, p, grid, s);
+        case 1: return launch_descend_metric<kMetricCos, ROWF>(cpl, p, grid, s);
+        default: return launch_descend_metric<kMetricDot, ROWF>(cpl, p, grid, s);
     }
+}
+// f16 = the descent walks the f16 copy, like the layer-0 search it seeds
+static cudaError_t launch_descend(bool f16, int metric, int cpl, const SearchParams &p, unsigned grid, cudaStream_t s) {
+    return f16 ? launch_descend_rowf<kRowF16>(metric, cpl, p, grid, s) : launch_descend_rowf<kRowF32>(metric, cpl, p, grid, s);
 }
 
 // K1L, the latency form: one CTA of 8 (or 4) warps per query (search_team_kernel.cuh)
-template <int CPL, int METRIC, bool ADJC, int MC, int T>
+template <int CPL, int METRIC, bool ADJC, int MC, int T, int ROWF>
 static cudaError_t launch_team_inst3(const SearchParams &p, unsigned grid, size_t smem, cudaStream_t s) {
-    auto kern = search_team_kernel<CPL, METRIC, ADJC, MC, T>;
+    auto kern = ROWF == kRowF16 ? search_team_f16_kernel<CPL, METRIC, ADJC, MC, T> : search_team_kernel<CPL, METRIC, ADJC, MC, T>;
     if (smem > 48 * 1024) {
         cudaError_t e = cudaFuncSetAttribute(kern, cudaFuncAttributeMaxDynamicSharedMemorySize, static_cast<int>(smem));
         if (e != cudaSuccess) return e;
@@ -294,30 +358,35 @@ static cudaError_t launch_team_inst3(const SearchParams &p, unsigned grid, size_
 // Full teams (256 threads): m = 16 (BASELINE's M) with the adjacency cache is compiled with m as a constant, everything else
 // reads m from the parameters. Half teams (128 threads) exist without the cache only: they are what a batch runs on that is too
 // large for full teams to be resident at once.
-template <int CPL, int METRIC>
+template <int CPL, int METRIC, int ROWF>
 static cudaError_t launch_team_inst(bool adjc, unsigned threads, const SearchParams &p, unsigned grid, size_t smem, cudaStream_t s) {
-    if (threads == 128) return launch_team_inst3<CPL, METRIC, false, 0, 128>(p, grid, smem, s);
-    if (adjc && p.m == 16) return launch_team_inst3<CPL, METRIC, true, 16, 256>(p, grid, smem, s);
-    return adjc ? launch_team_inst3<CPL, METRIC, true, 0, 256>(p, grid, smem, s) : launch_team_inst3<CPL, METRIC, false, 0, 256>(p, grid, smem, s);
+    if (threads == 128) return launch_team_inst3<CPL, METRIC, false, 0, 128, ROWF>(p, grid, smem, s);
+    if (adjc && p.m == 16) return launch_team_inst3<CPL, METRIC, true, 16, 256, ROWF>(p, grid, smem, s);
+    return adjc ? launch_team_inst3<CPL, METRIC, true, 0, 256, ROWF>(p, grid, smem, s) : launch_team_inst3<CPL, METRIC, false, 0, 256, ROWF>(p, grid, smem, s);
 }
-template <int METRIC>
+template <int METRIC, int ROWF>
 static cudaError_t launch_team_metric(int cpl, bool adjc, unsigned threads, const SearchParams &p, unsigned grid, size_t smem, cudaStream_t s) {
     switch (cpl) {
-        case 1: return launch_team_inst<1, METRIC>(adjc, threads, p, grid, smem, s);
-        case 2: return launch_team_inst<2, METRIC>(adjc, threads, p, grid, smem, s);
-        case 4: return launch_team_inst<4, METRIC>(adjc, threads, p, grid, smem, s);
-        case 6: return launch_team_inst<6, METRIC>(adjc, threads, p, grid, smem, s);
-        case 8: return launch_team_inst<8, METRIC>(adjc, threads, p, grid, smem, s);
+        case 1: return launch_team_inst<1, METRIC, ROWF>(adjc, threads, p, grid, smem, s);
+        case 2: return launch_team_inst<2, METRIC, ROWF>(adjc, threads, p, grid, smem, s);
+        case 4: return launch_team_inst<4, METRIC, ROWF>(adjc, threads, p, grid, smem, s);
+        case 6: return launch_team_inst<6, METRIC, ROWF>(adjc, threads, p, grid, smem, s);
+        case 8: return launch_team_inst<8, METRIC, ROWF>(adjc, threads, p, grid, smem, s);
     }
     return cudaErrorInvalidValue;
 }
-// adjc = every candidate's adjacency row kept in shared memory (no dependent adjacency fetch at a pop)
-static cudaError_t launch_team(int metric, int cpl, bool adjc, unsigned threads, const SearchParams &p, unsigned grid, size_t smem, cudaStream_t s) {
+template <int ROWF>
+static cudaError_t launch_team_rowf(int metric, int cpl, bool adjc, unsigned threads, const SearchParams &p, unsigned grid, size_t smem, cudaStream_t s) {
     switch (metric) {
-        case 0: return launch_team_metric<kMetricL2>(cpl, adjc, threads, p, grid, smem, s);
-        case 1: return launch_team_metric<kMetricCos>(cpl, adjc, threads, p, grid, smem, s);
-        default: return launch_team_metric<kMetricDot>(cpl, adjc, threads, p, grid, smem, s);
+        case 0: return launch_team_metric<kMetricL2, ROWF>(cpl, adjc, threads, p, grid, smem, s);
+        case 1: return launch_team_metric<kMetricCos, ROWF>(cpl, adjc, threads, p, grid, smem, s);
+        default: return launch_team_metric<kMetricDot, ROWF>(cpl, adjc, threads, p, grid, smem, s);
     }
+}
+// adjc = every candidate's adjacency row kept in shared memory (no dependent adjacency fetch at a pop); f16 = over the f16 copy
+static cudaError_t launch_team(bool f16, int metric, int cpl, bool adjc, unsigned threads, const SearchParams &p, unsigned grid, size_t smem, cudaStream_t s) {
+    return f16 ? launch_team_rowf<kRowF16>(metric, cpl, adjc, threads, p, grid, smem, s)
+               : launch_team_rowf<kRowF32>(metric, cpl, adjc, threads, p, grid, smem, s);
 }
 
 // Where the exact visited set of a search with pop budget `ef` lives (see launch_search).
@@ -374,8 +443,16 @@ static int launch_search(zvdb_index *ix, const float *d_q, uint64_t nq, uint32_t
     const HostGraph &g = ix->g;
     if (nq == 0) return ZVDB_OK;
     if (nq > 0x7FFFFFFFull) return fail(ZVDB_ERR_UNSUPPORTED, "nq exceeds 2^31-1 queries per launch");
+    // F16 storage: the plain search gathers the f16 copy (brought up to date here) and re-ranks on the fp32 arena
+    const bool f16 = ix->storage == ZVDB_STORAGE_F16 && g.n > 0;
+    if (f16 && (fx || n_peers)) return fail(ZVDB_ERR_UNSUPPORTED, "f16 storage: the sharded exchange forms gather fp32 rows only");
+    if (f16) {
+        int rcf = sync_f16_locked(ix);
+        if (rcf) return rcf;
+    }
     SearchParams p{};
     p.arena = reinterpret_cast<const float4 *>(ix->d_arena);
+    p.arena16 = f16 ? ix->d_arena16 : nullptr;
     p.adj = ix->d_adj;
     p.queries = d_q;
     p.ids = d_ids; p.dist = d_dist; p.counts = d_counts; p.pops = d_pops; p.evals = d_evals;
@@ -438,14 +515,14 @@ static int launch_search(zvdb_index *ix, const float *d_q, uint64_t nq, uint32_t
             cudaError_t e;
             if (p.seeds) {                                    // K2 first (its seeds are per-handle scratch: ordered across streams)
                 ZV_CUDA(cudaStreamWaitEvent(s, ix->bitmap_ev, 0));
-                e = launch_descend(g.metric, cpl, p, static_cast<unsigned>((nq + 3) / 4), s);
+                e = launch_descend(f16, g.metric, cpl, p, static_cast<unsigned>((nq + 3) / 4), s);
                 ix->launches++;
                 ZV_CUDA(e);
             }
             p.slots = static_cast<uint32_t>(slots); p.hash_words = static_cast<uint32_t>(hash_words);
             p.cand_cap = static_cast<uint32_t>(team_cap);
             if (ix->mailbox_dev && nq == 1) { p.done_flag = ix->mailbox_dev; p.done_seq = ix->mailbox_seq; ix->mailbox_armed = true; }
-            e = launch_team(g.metric, cpl, adjc, threads, p, static_cast<unsigned>(nq), static_cast<size_t>(team_smem), s);
+            e = launch_team(f16, g.metric, cpl, adjc, threads, p, static_cast<unsigned>(nq), static_cast<size_t>(team_smem), s);
             ix->launches++;
             ZV_CUDA(e);
             if (p.seeds) ZV_CUDA(cudaEventRecord(ix->bitmap_ev, s));
@@ -548,14 +625,14 @@ static int launch_search(zvdb_index *ix, const float *d_q, uint64_t nq, uint32_t
     if (p.seeds) {                                        // K2 first: one warp per query, 4 per CTA
         // the seeds are per-handle scratch like the tables: order launches from different streams
         if (vis == kVisSmemHash) ZV_CUDA(cudaStreamWaitEvent(s, ix->bitmap_ev, 0));
-        e = launch_descend(g.metric, cpl, p, static_cast<unsigned>((nq + 3) / 4), s);
+        e = launch_descend(f16, g.metric, cpl, p, static_cast<unsigned>((nq + 3) / 4), s);
         ix->launches++;
         ZV_CUDA(e);
     }
     const bool exch = n_peers != 0 || fx != nullptr;
-    if (vis == kVisSmemHash) e = launch_search_vis<kVisSmemHash>(exch, g.metric, cpl, p, grid, smem, s);
-    else if (vis == kVisGlobalBitmap) e = launch_search_vis<kVisGlobalBitmap>(exch, g.metric, cpl, p, grid, smem, s);
-    else e = launch_search_vis<kVisGlobalHash>(exch, g.metric, cpl, p, grid, smem, s);
+    if (vis == kVisSmemHash) e = launch_search_vis<kVisSmemHash>(exch, f16, g.metric, cpl, p, grid, smem, s);
+    else if (vis == kVisGlobalBitmap) e = launch_search_vis<kVisGlobalBitmap>(exch, f16, g.metric, cpl, p, grid, smem, s);
+    else e = launch_search_vis<kVisGlobalHash>(exch, f16, g.metric, cpl, p, grid, smem, s);
     ix->launches++;
     ZV_CUDA(e);
     if (vis != kVisSmemHash || p.seeds) ZV_CUDA(cudaEventRecord(ix->bitmap_ev, s));
@@ -965,8 +1042,9 @@ void zvdb_destroy(zvdb_index *ix) {
     for (int i = 0; i < 8; ++i) if (ix->in_ev[i]) cudaEventDestroy(ix->in_ev[i]);
     if (ix->bitmap_ev) cudaEventDestroy(ix->bitmap_ev);
     if (ix->bf_ev) cudaEventDestroy(ix->bf_ev);
-    cudaFree(ix->d_arena); cudaFree(ix->d_adj);
+    cudaFree(ix->d_arena); cudaFree(ix->d_adj); cudaFree(ix->d_arena16);
     if (ix->h_stage) cudaFreeHost(ix->h_stage);
+    ix->f16_bad.free_();
     ix->q_buf.free_(); ix->dist_buf.free_(); ix->ids_buf.free_(); ix->cnt_buf.free_();
     ix->pops_buf.free_(); ix->evals_buf.free_(); ix->scat_rows.free_(); ix->scat_ids.free_(); ix->bitmap_buf.free_(); ix->vlog_buf.free_(); ix->res_buf.free_(); ix->gtable_buf.free_();
     ix->d_level.free_(); ix->d_upper_base.free_(); ix->d_upper_adj.free_(); ix->seeds_buf.free_();
@@ -1174,7 +1252,7 @@ static int set_points_locked(zvdb_index *ix, const float *points, uint64_t n, ui
     }
     g.has_entry = n > 0; g.entry = entry; g.max_level = 0;
     g.rows_uploaded = 0; g.adj_all_dirty = true;
-    ix->n_dev = 0; ix->bf_rows = 0;
+    ix->n_dev = 0; ix->bf_rows = 0; ix->f16_rows = 0;
     return ZVDB_OK;
 }
 
@@ -1281,7 +1359,7 @@ int zvdb_load(zvdb_index *ix, const char *path) {
         g.dim = 0; g.row_floats = 0; g.rows_per_chunk = 0;
         if (hd.dim) g.fix_dim(hd.dim);
         g.ef_construction = hd.ef_construction; g.rng = hd.rng; g.dtype = 0;
-        ix->n_dev = 0; ix->bf_rows = 0;
+        ix->n_dev = 0; ix->bf_rows = 0; ix->f16_rows = 0;
         return ZVDB_OK;
     }
     if (hd.dim == 0 || hd.dim > 1024 || hd.row_floats != (hd.dim + 31u) / 32u * 32u || hd.n >= 0xFFFFFFFEull || hd.max_level > 31 ||
@@ -1358,7 +1436,7 @@ int zvdb_load(zvdb_index *ix, const char *path) {
     g.upper_off.swap(fresh.upper_off); g.upper.swap(fresh.upper);
     g.has_entry = fresh.has_entry; g.entry = fresh.entry; g.max_level = fresh.max_level; g.top_node = fresh.top_node; g.rng = fresh.rng;
     ++g.upper_version; g.rows_uploaded = 0; g.dirty.clear(); g.adj_all_dirty = true;
-    ix->n_dev = 0; ix->bf_rows = 0;
+    ix->n_dev = 0; ix->bf_rows = 0; ix->f16_rows = 0;
     return ZVDB_OK;
 }
 
@@ -1368,6 +1446,23 @@ int zvdb_set_descent(zvdb_index *ix, int on) {
     ix->descent = on != 0;
     return ZVDB_OK;
 }
+
+int zvdb_set_storage(zvdb_index *ix, int storage) {
+    if (!ix) return fail(ZVDB_ERR_INVALID, "null index");
+    if (storage != ZVDB_STORAGE_F32 && storage != ZVDB_STORAGE_F16) return fail(ZVDB_ERR_INVALID, "set_storage: storage must be ZVDB_STORAGE_F32 or ZVDB_STORAGE_F16");
+    std::lock_guard<std::mutex> lk(ix->mu);
+    if (storage == ZVDB_STORAGE_F16 && ix->g.dtype != 0)
+        return fail(ZVDB_ERR_UNSUPPORTED, "set_storage: f16 storage is built for f32 indexes only (this one holds f64 / i32 rows)");
+    ix->storage = storage;
+    if (storage == ZVDB_STORAGE_F32 && ix->d_arena16) {      // searches enqueued on caller streams may still read it
+        ZV_CUDA(cudaSetDevice(ix->device));
+        ZV_CUDA(cudaDeviceSynchronize());
+        cudaFree(ix->d_arena16); ix->d_arena16 = nullptr; ix->f16_rows = 0;
+    }
+    return ZVDB_OK;
+}
+
+int zvdb_storage(const zvdb_index *ix) { if (!ix) return ZVDB_STORAGE_F32; ZV_LOCKED(ix); return ix->storage; }
 
 int64_t zvdb_descent_start(const zvdb_index *ix) {
     if (!ix) return -1;
@@ -1500,7 +1595,7 @@ int zvdb_build_from_candidates(zvdb_index *ix, const float *points, uint64_t n, 
         // becomes empty (the error string of the failing step is kept).
         const std::string why = g_last_error;
         g.reset_nodes();
-        ix->n_dev = 0; ix->bf_rows = 0;
+        ix->n_dev = 0; ix->bf_rows = 0; ix->f16_rows = 0;
         return fail(rc, why);
     }
     // the table was produced on the device and copied back: both sides are current
@@ -1900,6 +1995,7 @@ int zvdb_search_batch_exchange(zvdb_index *ix, zvdb_exchange *ex, const float *d
     const uint64_t block = zvdb_shard_block_bytes(nq, k);
     if (block * ex->world > ex->cap_bytes) return fail(ZVDB_ERR_INVALID, "exchange: nq * k exceeds the capacity the exchange was created with");
     std::lock_guard<std::mutex> lk(ix->mu);
+    if (ix->storage == ZVDB_STORAGE_F16) return fail(ZVDB_ERR_UNSUPPORTED, "exchange: f16 storage is not built into the sharded forms; set ZVDB_STORAGE_F32");
     ZV_CUDA(cudaSetDevice(ix->device));
     cudaStream_t s = static_cast<cudaStream_t>(stream);
     const uint32_t epoch = ++ex->epoch;
@@ -1961,6 +2057,7 @@ int zvdb_search_batch_exchange_host(zvdb_index *ix, zvdb_exchange *ex, const flo
     const uint64_t block = zvdb_shard_block_bytes(nq, k);
     if (block * ex->world > ex->cap_bytes) return fail(ZVDB_ERR_INVALID, "exchange: nq * k exceeds the capacity the exchange was created with");
     std::lock_guard<std::mutex> lk(ix->mu);
+    if (ix->storage == ZVDB_STORAGE_F16) return fail(ZVDB_ERR_UNSUPPORTED, "exchange: f16 storage is not built into the sharded forms; set ZVDB_STORAGE_F32");
     ZV_CUDA(cudaSetDevice(ix->device));
     const bool empty = ix->g.n == 0 || !ix->g.has_entry;
     if (!empty && dim != ix->g.dim) return fail(ZVDB_ERR_DIM_MISMATCH, "Mismatched dimensions in distance calculation");

@@ -27,6 +27,8 @@
 // Memory traffic per query (the HBM-gather roofline numerator, SURVEY 8d):
 //   evals * row_bytes (row gathers) + pops * m * 4 (adjacency rows) + dim*4 (query) + k*12 (output).
 #pragma once
+#include <cuda_fp16.h>
+#include <type_traits>
 #include "common.cuh"
 
 namespace zvdb {
@@ -115,17 +117,44 @@ struct SearchParams {
     // the host call returns on seeing it instead of waiting for the stream to report the kernel's completion.
     uint32_t *done_flag;
     uint32_t done_seq;
+    // F16 row format (zvdb_set_storage): the rows the traversal gathers, [n][row_chunks] 8-byte chunks of four halves (the
+    // fp32 arena rounded to nearest even); `arena` stays the fp32 rows the popped set is re-scored on.
+    const uint2 *arena16;
 };
 
 enum : int { kMetricL2 = 0, kMetricCos = 1, kMetricDot = 2 };
 constexpr uint32_t kPoolCap = 64;   // pending pool slots
 
+// Row format of the gathered rows. A lane owns the same four elements of a 128-element chunk in both: 16 bytes of fp32
+// (float4) or 8 bytes of fp16 (uint2, two __half2). fp16 -> fp32 is exact, so the FFMA2 chain and the butterfly see the
+// same operands as an fp32 row holding the rounded values: a search over f16 rows is bit for bit the oracle's search on
+// the f16-rounded rows.
+enum : int { kRowF32 = 0, kRowF16 = 1 };
+template <int ROWF> using RowChunk = std::conditional_t<ROWF == kRowF16, uint2, float4>;
+__device__ __forceinline__ float4 chunk_f32(const float4 v) { return v; }
+__device__ __forceinline__ float4 chunk_f32(const uint2 w) {
+    const float2 a = __half22float2(*reinterpret_cast<const __half2 *>(&w.x));
+    const float2 b = __half22float2(*reinterpret_cast<const __half2 *>(&w.y));
+    return make_float4(a.x, a.y, b.x, b.y);
+}
+template <int ROWF> __device__ __forceinline__ RowChunk<ROWF> zero_chunk() {
+    if constexpr (ROWF == kRowF16) return make_uint2(0u, 0u); else return make_float4(0.f, 0.f, 0.f, 0.f);
+}
+// The rows a search gathers: the fp32 arena, or its f16 copy.
+template <int ROWF> __device__ __forceinline__ const RowChunk<ROWF> *search_rows(const SearchParams &p) {
+    if constexpr (ROWF == kRowF16) return p.arena16; else return p.arena;
+}
+
 // Rows a warp fetches before it starts reducing (loads in flight per lane = U * CPL float4).
 // WIDE is used when shared memory already limits residency to <= 16 warps per SM, so each thread
 // may hold twice the registers.
-template <int CPL, bool WIDE> struct Unroll {
+// F16 rows cost half the registers in flight; ZVDB_F16_UNROLL scales U for them (1 = the fp32 value).
+#ifndef ZVDB_F16_UNROLL
+#define ZVDB_F16_UNROLL 1
+#endif
+template <int CPL, bool WIDE, int ROWF = kRowF32> struct Unroll {
     static constexpr int narrow = CPL <= 1 ? 8 : (CPL <= 2 ? 4 : 2);
-    static constexpr int value = WIDE ? (CPL <= 4 ? narrow * 2 : narrow) : narrow;
+    static constexpr int value = (WIDE ? (CPL <= 4 ? narrow * 2 : narrow) : narrow) * (ROWF == kRowF16 ? ZVDB_F16_UNROLL : 1);
 };
 
 // Packed f32x2 arithmetic (Blackwell FFMA2: PTX fma.rn.f32x2, sm_100+). A 16-byte chunk (x,y,z,w)
@@ -226,17 +255,19 @@ __device__ __forceinline__ void transposed_reduce(float (&d)[R], uint32_t lane, 
 // ids[u] for u >= nrows must still be valid row ids (callers pad with a hot row): a full-width
 // batch runs without per-row predicates. Returns, in every lane l, the distance of row l / (32/U)
 // (meaningless for rows >= nrows).
-template <int CPL, int METRIC, int U>
-__device__ __forceinline__ float rows_distance(const float4 *__restrict__ arena, uint32_t row_chunks,
+// ROWF = kRowF16: the same with 8-byte chunks (ld.global.nc.v2), converted exactly before the FMAs.
+template <int CPL, int METRIC, int U, int ROWF = kRowF32>
+__device__ __forceinline__ float rows_distance(const RowChunk<ROWF> *__restrict__ arena, uint32_t row_chunks,
                                                const uint32_t (&ids)[U], const Chunk2 (&qv)[CPL], uint32_t lane) {
-    float4 v[U][CPL];
-    const float4 *__restrict__ base = arena + lane;
+    using T = RowChunk<ROWF>;
+    T v[U][CPL];
+    const T *__restrict__ base = arena + lane;
     if (row_chunks == 32u * CPL) {                       // every lane owns CPL chunks (dim a multiple of 128*CPL... the common case)
         // byte address = base + id * (compile-time row bytes): one IMAD.WIDE per row instead of multiply + 64-bit shift-add
         const char *__restrict__ bbase = reinterpret_cast<const char *>(base);
 #pragma unroll
         for (int u = 0; u < U; ++u) {
-            const float4 *__restrict__ row = reinterpret_cast<const float4 *>(bbase + static_cast<uint64_t>(ids[u]) * (512u * CPL));
+            const T *__restrict__ row = reinterpret_cast<const T *>(bbase + static_cast<uint64_t>(ids[u]) * (32u * sizeof(T) * CPL));
 #pragma unroll
             for (int c = 0; c < CPL; ++c) v[u][c] = __ldg(row + 32 * c);
         }
@@ -245,7 +276,7 @@ __device__ __forceinline__ float rows_distance(const float4 *__restrict__ arena,
         for (int u = 0; u < U; ++u) {
 #pragma unroll
             for (int c = 0; c < CPL; ++c) {
-                v[u][c] = make_float4(0.f, 0.f, 0.f, 0.f);
+                v[u][c] = zero_chunk<ROWF>();
                 if (lane + 32u * c < row_chunks) v[u][c] = __ldg(base + static_cast<size_t>(ids[u]) * row_chunks + 32 * c);
             }
         }
@@ -255,7 +286,7 @@ __device__ __forceinline__ float rows_distance(const float4 *__restrict__ arena,
     for (int u = 0; u < U; ++u) {
         uint64_t a2 = 0;                                 // (+0.0f, +0.0f)
 #pragma unroll
-        for (int c = 0; c < CPL; ++c) a2 = accumulate_chunk<METRIC>(a2, qv[c], v[u][c]);
+        for (int c = 0; c < CPL; ++c) a2 = accumulate_chunk<METRIC>(a2, qv[c], chunk_f32(v[u][c]));
         acc[u] = lane_partial(a2);
     }
     transposed_reduce<U>(acc, lane, 16);
@@ -265,12 +296,13 @@ __device__ __forceinline__ float rows_distance(const float4 *__restrict__ arena,
 // Ask for one whole arena row to be brought into L2, one request per 128-byte line, no register and no
 // scoreboard behind it (fire and forget). Per-lane addresses: the bulk form (cp.async.bulk.prefetch.L2)
 // takes its address from a uniform register and compiles to a lane-by-lane loop, ~7 issue slots per row.
-template <int CPL>
-__device__ __forceinline__ void prefetch_row_l2(const float4 *__restrict__ arena, uint32_t row_chunks, uint32_t id) {
-    const float4 *row = arena + static_cast<size_t>(id) * row_chunks;
+template <int CPL, typename T>
+__device__ __forceinline__ void prefetch_row_l2(const T *__restrict__ arena, uint32_t row_chunks, uint32_t id) {
+    constexpr uint32_t kLine = 128 / sizeof(T);          // chunks per 128-byte line
+    const T *row = arena + static_cast<size_t>(id) * row_chunks;
 #pragma unroll
-    for (int i = 0; i < CPL * 4; ++i)
-        if (static_cast<uint32_t>(i) * 8u < row_chunks) asm volatile("prefetch.global.L2 [%0];" ::"l"(row + i * 8));
+    for (int i = 0; i < CPL * 32 / static_cast<int>(kLine); ++i)
+        if (static_cast<uint32_t>(i) * kLine < row_chunks) asm volatile("prefetch.global.L2 [%0];" ::"l"(row + i * kLine));
 }
 
 // Ask for the head of node `id`'s adjacency row (its first 128-byte line: the whole row for m <= 32).
@@ -279,16 +311,16 @@ __device__ __forceinline__ void prefetch_adj_l2(const uint32_t *__restrict__ adj
 }
 
 // Distance of ONE row, every lane returns it (plain butterfly; same bits as rows_distance).
-template <int CPL, int METRIC>
-__device__ __forceinline__ float row_distance(const float4 *__restrict__ arena, uint32_t row_chunks, uint32_t id,
+template <int CPL, int METRIC, int ROWF = kRowF32>
+__device__ __forceinline__ float row_distance(const RowChunk<ROWF> *__restrict__ arena, uint32_t row_chunks, uint32_t id,
                                               const Chunk2 (&qv)[CPL], uint32_t lane) {
     uint64_t a2 = 0;
 #pragma unroll
     for (int c = 0; c < CPL; ++c) {
         const uint32_t chunk = lane + 32u * c;
-        float4 v = make_float4(0.f, 0.f, 0.f, 0.f);
+        RowChunk<ROWF> v = zero_chunk<ROWF>();
         if (chunk < row_chunks) v = __ldg(arena + static_cast<size_t>(id) * row_chunks + chunk);
-        a2 = accumulate_chunk<METRIC>(a2, qv[c], v);
+        a2 = accumulate_chunk<METRIC>(a2, qv[c], chunk_f32(v));
     }
     float acc = lane_partial(a2);
 #pragma unroll
@@ -378,19 +410,20 @@ __device__ __forceinline__ uint32_t merge_pool(uint64_t *win, uint32_t ns, uint3
 // that beats where it stood); repeat until a scan moves nothing. A node that does not have the layer is
 // not scanned (:93). Here the layers are taken top down and the node reached on layer 1 seeds the
 // layer-0 beam of search_layer0_kernel instead of entry_point. A kernel of its own so that the beam's
-// register budget (64 per thread, 32 warps per SM) is untouched.
-template <int CPL, int METRIC>
+// register budget (64 per thread, 32 warps per SM) is untouched. ROWF = the rows the layer-0 search gathers (its seeds
+// carry distances of the same rows).
+template <int CPL, int METRIC, int ROWF = kRowF32>
 __global__ void __launch_bounds__(128) descend_kernel(const SearchParams p) {
-    constexpr int U = Unroll<CPL, false>::value;
+    constexpr int U = Unroll<CPL, false, ROWF>::value;
     constexpr uint32_t LPR = 32 / U;
     const uint32_t lane = threadIdx.x & 31;
     const uint32_t q = blockIdx.x * (blockDim.x >> 5) + (threadIdx.x >> 5);
     if (q >= p.nq) return;
-    const float4 *__restrict__ arena = p.arena;
+    const RowChunk<ROWF> *__restrict__ arena = search_rows<ROWF>(p);
     Chunk2 qv[CPL];
     load_query<CPL>(qv, p.queries + static_cast<size_t>(q) * p.dim, p.dim, lane);
     uint32_t entry = p.descent_start, ndesc = 0;
-    float d0 = row_distance<CPL, METRIC>(arena, p.row_chunks, entry, qv, lane);
+    float d0 = row_distance<CPL, METRIC, ROWF>(arena, p.row_chunks, entry, qv, lane);
     for (uint32_t layer = p.max_level; layer >= 1; --layer) {
         for (;;) {
             if (layer > __ldg(p.levels + entry)) break;                                           // :93
@@ -408,7 +441,7 @@ __global__ void __launch_bounds__(128) descend_kernel(const SearchParams p) {
                         const uint32_t x = __shfl_sync(kFullMask, nb, (c0 + u) & 31);
                         ids[u] = x == kInvalidId ? entry : x;
                     }
-                    const float d = rows_distance<CPL, METRIC, U>(arena, p.row_chunks, ids, qv, lane);
+                    const float d = rows_distance<CPL, METRIC, U, ROWF>(arena, p.row_chunks, ids, qv, lane);
                     const uint32_t j = c0 + lane / LPR;
                     if ((lane % LPR) == 0 && j < nvalid)
                         best = min(best, (static_cast<uint64_t>(float_to_ordered(d)) << 32) | (base + j));
@@ -547,10 +580,14 @@ __device__ __noinline__ void merge_one_query(const SearchParams &p, uint32_t q, 
 // EXCH = the sharded forms of the step (peer stores, records, flags, the merge tail). The plain search is a separate
 // instantiation with none of that code in it: in round 2 every piece of exchange code added behind a run-time test still
 // cost the global-visited modes 8-10 % (the 64-register pop loop is allocated together with whatever surrounds it).
-template <int CPL, int METRIC, int VIS, bool EXCH>
+// ROWF = the format of the rows the traversal gathers. kRowF16 (plain search only, EXCH = false) adds the exact re-rank
+// epilogue: the popped set is re-scored on the fp32 arena and ordered by (exact distance, id). It exists only in those
+// instantiations, for the same reason as EXCH.
+template <int CPL, int METRIC, int VIS, bool EXCH, int ROWF = kRowF32>
 __global__ void __launch_bounds__(32, (CPL <= 2 ? 32 : 16))
 search_layer0_kernel(const __grid_constant__ SearchParams p) {
-    constexpr int U = Unroll<CPL, false>::value;
+    static_assert(ROWF == kRowF32 || !EXCH, "the sharded forms gather fp32 rows only");
+    constexpr int U = Unroll<CPL, false, ROWF>::value;
     constexpr uint32_t LPR = 32 / U;                            // lanes holding the same row after the reduce
     constexpr bool GLOBAL_VIS = VIS != kVisSmemHash;
     const uint32_t x_world = EXCH ? p.ex_world : 0u, x_qper = EXCH ? p.q_per : 0u, x_lines = EXCH ? p.ll_lines : 0u, x_peers = EXCH ? p.n_peers : 0u;
@@ -598,7 +635,7 @@ search_layer0_kernel(const __grid_constant__ SearchParams p) {
     };
 
     const uint32_t lane = threadIdx.x;
-    const float4 *__restrict__ arena = p.arena;
+    const RowChunk<ROWF> *__restrict__ arena = search_rows<ROWF>(p);
     const uint32_t pass_w = min(p.m, 32u);
     if (x_qper && blockIdx.x == 0 && lane < x_world && lane != p.ex_rank)   // our slice of the queries is in place (copied before this launch)
         asm volatile("st.release.sys.global.u32 [%0], %1;" ::"l"(p.peer_sflags[lane] + static_cast<size_t>(p.ex_rank) * p.sflag_pitch), "r"(p.ex_epoch) : "memory");
@@ -636,7 +673,7 @@ search_layer0_kernel(const __grid_constant__ SearchParams p) {
         uint32_t entry = p.entry;
         float d0;
         if (p.seeds == nullptr) {
-            d0 = row_distance<CPL, METRIC>(arena, p.row_chunks, entry, qv, lane);
+            d0 = row_distance<CPL, METRIC, ROWF>(arena, p.row_chunks, entry, qv, lane);
         } else {                                           // K2 ran first: start where the descent landed
             const uint4 sd = __ldg(p.seeds + q);
             entry = sd.x; d0 = __uint_as_float(sd.y);
@@ -754,7 +791,7 @@ search_layer0_kernel(const __grid_constant__ SearchParams p) {
                     uint32_t ids[U];
 #pragma unroll
                     for (int u = 0; u < U; ++u) ids[u] = __shfl_sync(kFullMask, nb_row, c0 + u);
-                    const float d = rows_distance<CPL, METRIC, U>(arena, p.row_chunks, ids, qv, lane);
+                    const float d = rows_distance<CPL, METRIC, U, ROWF>(arena, p.row_chunks, ids, qv, lane);
                     if (!resolved) { resolve(); if (((fmask >> c0) & kChunkMask) == 0) continue; }
                     const uint32_t j = c0 + lane / LPR;                   // the neighbour slot whose row this lane holds
                     const uint32_t rid = __shfl_sync(kFullMask, nb, j);
@@ -793,7 +830,7 @@ search_layer0_kernel(const __grid_constant__ SearchParams p) {
 #pragma unroll
                     for (int u = 0; u < U; ++u) ids[u] = todo[j0 + u];
                 }
-                const float d = rows_distance<CPL, METRIC, U>(arena, p.row_chunks, ids, qv, lane);
+                const float d = rows_distance<CPL, METRIC, U, ROWF>(arena, p.row_chunks, ids, qv, lane);
                 const uint32_t r = lane / LPR;                   // the row this lane holds
                 uint64_t key = ~0ull;
                 if ((lane % LPR) == 0 && r < static_cast<uint32_t>(nrows)) key = pack_key(d, todo[j0 + r]);
@@ -811,8 +848,25 @@ search_layer0_kernel(const __grid_constant__ SearchParams p) {
     __syncwarp();
     uint64_t *sorted = cand;                                     // the window is dead now
     const uint32_t p2 = next_pow2(np);
+    if constexpr (ROWF == kRowF16) {
+        // Re-rank: every popped id re-scored with the fp32 distance on the fp32 arena (the K1 / K4 distance of the pair),
+        // keys (exact distance, id) sorted directly; sorted[] then holds keys, not pop indices.
+        constexpr int U32 = Unroll<CPL, false>::value;
+        constexpr uint32_t LPR32 = 32 / U32;
+        const uint32_t first = key_id(*res_at(0));               // padding rows of the last batch: a valid, hot row
+        for (uint32_t j0 = 0; j0 < np; j0 += U32) {
+            uint32_t ids[U32];
+#pragma unroll
+            for (int u = 0; u < U32; ++u) ids[u] = j0 + u < np ? key_id(*res_at(j0 + u)) : first;
+            const float d = rows_distance<CPL, METRIC, U32>(p.arena, p.row_chunks, ids, qv, lane);
+            const uint32_t r = lane / LPR32;
+            if ((lane % LPR32) == 0 && j0 + r < np) sorted[j0 + r] = pack_key(d, key_id(*res_at(j0 + r)));
+        }
+        for (uint32_t i = np + lane; i < p2; i += 32) sorted[i] = ~0ull;
+    } else {
     for (uint32_t i = lane; i < p2; i += 32)
         sorted[i] = i < np ? ((*res_at(i) & 0xFFFFFFFF00000000ull) | i) : ~0ull;
+    }
     bitonic_sort_u64(sorted, p2);
     const uint32_t nres = min(np, p.k);
     // receivers of this query's shard-local top-k: every rank (all-gather), or only the query's owner
@@ -852,7 +906,7 @@ search_layer0_kernel(const __grid_constant__ SearchParams p) {
         const size_t o = static_cast<size_t>(q) * p.k + r;
         uint64_t oid = ~0ull; float od = 0.0f;
         if (r < nres) {
-            const uint64_t key = x_world ? sorted[r] : *res_at(static_cast<uint32_t>(sorted[r]));
+            const uint64_t key = (x_world || ROWF == kRowF16) ? sorted[r] : *res_at(static_cast<uint32_t>(sorted[r]));
             oid = static_cast<uint64_t>(key_id(key)) * p.id_stride + p.id_base;
             od = key_dist(key);
         }

@@ -56,36 +56,38 @@ __host__ __device__ inline uint64_t team_smem_bytes(uint64_t cand_cap, uint64_t 
     return (b + 15) & ~15ull;
 }
 
-template <int CPL, int METRIC>
-__device__ __forceinline__ void half_row_load(float4 (&vlo)[CPL], float4 (&vhi)[CPL], const float4 *__restrict__ arena,
+// Lane j of a half-warp loads chunks j and j + 16 of every 32: 16-byte chunks of an fp32 row, 8-byte chunks of an f16 row.
+template <int CPL, int METRIC, int ROWF = kRowF32>
+__device__ __forceinline__ void half_row_load(RowChunk<ROWF> (&vlo)[CPL], RowChunk<ROWF> (&vhi)[CPL], const RowChunk<ROWF> *__restrict__ arena,
                                               uint32_t row_chunks, uint32_t id, uint32_t j) {
+    using T = RowChunk<ROWF>;
     if (row_chunks == 32u * CPL) {
-        const char *__restrict__ b = reinterpret_cast<const char *>(arena + j) + static_cast<uint64_t>(id) * (512u * CPL);
+        const char *__restrict__ b = reinterpret_cast<const char *>(arena + j) + static_cast<uint64_t>(id) * (32u * sizeof(T) * CPL);
 #pragma unroll
         for (int c = 0; c < CPL; ++c) {
-            vlo[c] = __ldg(reinterpret_cast<const float4 *>(b) + 32 * c);
-            vhi[c] = __ldg(reinterpret_cast<const float4 *>(b) + 32 * c + 16);
+            vlo[c] = __ldg(reinterpret_cast<const T *>(b) + 32 * c);
+            vhi[c] = __ldg(reinterpret_cast<const T *>(b) + 32 * c + 16);
         }
     } else {
-        const float4 *__restrict__ row = arena + static_cast<size_t>(id) * row_chunks;
+        const T *__restrict__ row = arena + static_cast<size_t>(id) * row_chunks;
 #pragma unroll
         for (int c = 0; c < CPL; ++c) {
             const uint32_t lo = j + 32u * c, hi = lo + 16u;
-            vlo[c] = make_float4(0.f, 0.f, 0.f, 0.f); vhi[c] = make_float4(0.f, 0.f, 0.f, 0.f);
+            vlo[c] = zero_chunk<ROWF>(); vhi[c] = zero_chunk<ROWF>();
             if (lo < row_chunks) vlo[c] = __ldg(row + lo);
             if (hi < row_chunks) vhi[c] = __ldg(row + hi);
         }
     }
 }
 // Distance of the loaded row to the query by one half-warp; every lane of the half returns it.
-template <int CPL, int METRIC>
-__device__ __forceinline__ float half_row_reduce(const float4 (&vlo)[CPL], const float4 (&vhi)[CPL], const Chunk2 (&qlo)[CPL],
+template <int CPL, int METRIC, typename T>
+__device__ __forceinline__ float half_row_reduce(const T (&vlo)[CPL], const T (&vhi)[CPL], const Chunk2 (&qlo)[CPL],
                                                  const Chunk2 (&qhi)[CPL]) {
     uint64_t alo = 0, ahi = 0;                               // (+0.0f, +0.0f)
 #pragma unroll
     for (int c = 0; c < CPL; ++c) {
-        alo = accumulate_chunk<METRIC>(alo, qlo[c], vlo[c]);
-        ahi = accumulate_chunk<METRIC>(ahi, qhi[c], vhi[c]);
+        alo = accumulate_chunk<METRIC>(alo, qlo[c], chunk_f32(vlo[c]));
+        ahi = accumulate_chunk<METRIC>(ahi, qhi[c], chunk_f32(vhi[c]));
     }
     float s = __fadd_rn(lane_partial(alo), lane_partial(ahi));           // butterfly level xor 16
 #pragma unroll
@@ -101,10 +103,10 @@ __device__ __forceinline__ uint64_t warp_min_key(uint64_t key) {
     return (static_cast<uint64_t>(dmin) << 32) | imin;
 }
 
-// MC = m when it is known at compile time (16: BASELINE's M), 0 = read it from the parameters.
-template <int CPL, int METRIC, bool ADJC, int MC, int T>
-__global__ void __launch_bounds__(T, (T == 256 ? (CPL <= 2 ? 2 : 1) : (CPL <= 4 ? 4 : 2)))
-search_team_kernel(const __grid_constant__ SearchParams p) {
+// MC = m when it is known at compile time (16: BASELINE's M), 0 = read it from the parameters. ROWF = the format of the
+// rows the traversal gathers; kRowF16 adds the exact re-rank of the popped set (as in search_layer0_kernel).
+template <int CPL, int METRIC, bool ADJC, int MC, int T, int ROWF>
+__device__ __forceinline__ void search_team_body(const SearchParams &p) {
     constexpr uint32_t TT = T, TW = T / 32, TR = T / 16;            // threads, warps, rows (half-warps) per pass
     extern __shared__ __align__(16) unsigned char smem_raw[];
     const uint32_t m = MC ? static_cast<uint32_t>(MC) : p.m;
@@ -120,7 +122,7 @@ search_team_kernel(const __grid_constant__ SearchParams p) {
     const uint32_t tid = threadIdx.x, lane = tid & 31u, warp = tid >> 5, j = lane & 15u;
     const uint32_t half = warp * 2u + (lane >> 4);                  // the neighbour position of a pass this half-warp evaluates
     const uint32_t q = blockIdx.x;
-    const float4 *__restrict__ arena = p.arena;
+    const RowChunk<ROWF> *__restrict__ arena = search_rows<ROWF>(p);
 
     // query -> shared memory once (it may live in page-locked HOST memory: every load is a PCIe read), then registers
     {
@@ -146,8 +148,8 @@ search_team_kernel(const __grid_constant__ SearchParams p) {
         uint32_t entry = p.entry;
         float d0;
         if (p.seeds == nullptr) {
-            float4 vlo[CPL], vhi[CPL];
-            half_row_load<CPL, METRIC>(vlo, vhi, arena, p.row_chunks, entry, j);
+            RowChunk<ROWF> vlo[CPL], vhi[CPL];
+            half_row_load<CPL, METRIC, ROWF>(vlo, vhi, arena, p.row_chunks, entry, j);
             d0 = half_row_reduce<CPL, METRIC>(vlo, vhi, qlo, qhi);
         } else {                                                    // K2 ran first: start where the descent landed
             const uint4 sd = __ldg(p.seeds + q);
@@ -172,10 +174,10 @@ search_team_kernel(const __grid_constant__ SearchParams p) {
             if (pos < m) nb = ADJC ? cadj[cur_slot * m + pos] : __ldg(p.adj + static_cast<size_t>(cur) * m + pos);
             const bool valid = nb != kInvalidId;
             const bool active = __any_sync(kFullMask, valid);       // (per warp) some half of this warp has a neighbour in this pass
-            float4 vlo[CPL], vhi[CPL];
+            RowChunk<ROWF> vlo[CPL], vhi[CPL];
             bool fresh = false;
             if (active) {
-                half_row_load<CPL, METRIC>(vlo, vhi, arena, p.row_chunks, valid ? nb : cur, j);   // (padding: a hot, valid row)
+                half_row_load<CPL, METRIC, ROWF>(vlo, vhi, arena, p.row_chunks, valid ? nb : cur, j);   // (padding: a hot, valid row)
                 if (ADJC && valid) {                                // the neighbour's own adjacency row, in the same trip, straight into its slot
                     for (uint32_t w = j; w < m; w += 16u) {
                         const uint32_t dst = static_cast<uint32_t>(__cvta_generic_to_shared(cadj + slot * m + w));
@@ -226,15 +228,29 @@ search_team_kernel(const __grid_constant__ SearchParams p) {
     __syncthreads();
     uint64_t *sorted = cand;                                        // the candidates are dead now
     const uint32_t p2 = next_pow2(np);
+    if constexpr (ROWF == kRowF16) {
+        // Re-rank: half-warp h re-scores popped entries h, h + T / 16, ... with the fp32 distance on the fp32 arena; sorted[]
+        // then holds (exact distance, id) keys, not pop indices.
+        for (uint32_t i0 = 0; i0 < np; i0 += TR) {                  // (uniform bound: the reduction shuffles take whole warps)
+            const uint32_t i = i0 + half;
+            const uint32_t id = key_id(res[i < np ? i : 0u]);
+            float4 vlo[CPL], vhi[CPL];
+            half_row_load<CPL, METRIC>(vlo, vhi, p.arena, p.row_chunks, id, j);
+            const float d = half_row_reduce<CPL, METRIC>(vlo, vhi, qlo, qhi);
+            if (j == 0 && i < np) sorted[i] = pack_key(d, id);
+        }
+        for (uint32_t i = np + tid; i < p2; i += TT) sorted[i] = ~0ull;
+    } else {
     for (uint32_t i = tid; i < p2; i += TT)
         sorted[i] = i < np ? ((res[i] & 0xFFFFFFFF00000000ull) | i) : ~0ull;
+    }
     bitonic_sort_u64(sorted, p2);
     const uint32_t nres = min(np, p.k);
     for (uint32_t r = tid; r < p.k; r += TT) {
         const size_t o = static_cast<size_t>(q) * p.k + r;
         uint64_t oid = ~0ull; float od = 0.0f;
         if (r < nres) {
-            const uint64_t key = res[static_cast<uint32_t>(sorted[r])];
+            const uint64_t key = ROWF == kRowF16 ? sorted[r] : res[static_cast<uint32_t>(sorted[r])];
             oid = static_cast<uint64_t>(key_id(key)) * p.id_stride + p.id_base;
             od = key_dist(key);
         }
@@ -252,6 +268,20 @@ search_team_kernel(const __grid_constant__ SearchParams p) {
             *reinterpret_cast<volatile uint32_t *>(p.done_flag) = p.done_seq;
         }
     }
+}
+
+template <int CPL, int METRIC, bool ADJC, int MC, int T>
+__global__ void __launch_bounds__(T, (T == 256 ? (CPL <= 2 ? 2 : 1) : (CPL <= 4 ? 4 : 2)))
+search_team_kernel(const __grid_constant__ SearchParams p) {
+    search_team_body<CPL, METRIC, ADJC, MC, T, kRowF32>(p);
+}
+
+// The same over f16 rows with the exact re-rank (zvdb_set_storage): a kernel of its own name, so the fp32 kernels and their
+// instantiation count stay what they are.
+template <int CPL, int METRIC, bool ADJC, int MC, int T>
+__global__ void __launch_bounds__(T, (T == 256 ? (CPL <= 2 ? 2 : 1) : (CPL <= 4 ? 4 : 2)))
+search_team_f16_kernel(const __grid_constant__ SearchParams p) {
+    search_team_body<CPL, METRIC, ADJC, MC, T, kRowF16>(p);
 }
 
 }  // namespace zvdb

@@ -221,6 +221,20 @@ class HNSW:
         """Walk layers max_level..1 greedily before the layer-0 search (zvdb_set_descent)."""
         L.check(L.lib().zvdb_set_descent(self._h, 1 if on else 0))
 
+    # -- vector storage of the graph search (zvdb_set_storage) --------------------------------------
+    _STORAGE = {"f32": L.STORAGE_F32, "f16": L.STORAGE_F16}
+
+    def set_storage(self, storage: str = "f32") -> None:
+        """"f16": the graph search gathers an fp16 copy of the rows and re-ranks the popped set exactly in fp32
+        (distances returned are the fp32 ones); "f32" (default): it gathers the fp32 rows. Takes effect at the next search."""
+        if storage not in self._STORAGE:
+            raise ValueError('storage must be "f32" or "f16"')
+        L.check(L.lib().zvdb_set_storage(self._h, self._STORAGE[storage]))
+
+    @property
+    def storage(self) -> str:
+        return "f16" if int(L.lib().zvdb_storage(self._h)) == L.STORAGE_F16 else "f32"
+
     @property
     def descent_start(self) -> Optional[int]:
         e = int(L.lib().zvdb_descent_start(self._h))
