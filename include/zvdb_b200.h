@@ -178,8 +178,35 @@ ZVDB_API int zvdb_load_upper_layers(zvdb_index *ix, const uint8_t *levels, const
  * store it (nor the descent or the kernel variant): zvdb_load keeps the handle's setting, a new handle starts at F32. */
 #define ZVDB_STORAGE_F32 0   /* default: the search gathers the fp32 rows */
 #define ZVDB_STORAGE_F16 1   /* the search gathers an fp16 copy of the rows; results are re-ranked in fp32 */
+/* ZVDB_STORAGE_SQ8: the graph search gathers 8-bit codes of the rows (a quarter of the fp32 bytes per
+ * evaluated row: one 128-byte line per 128 dimensions), with the same contract as F16 wherever it can:
+ *   - codebook: one (scale s_d, offset o_d) fp32 pair per dimension, trained on the fp32 device rows
+ *     (normalised under cosine): o_d = min_d, s_d = (max_d - min_d) / 255 (round to nearest, each a
+ *     single IEEE operation; min / max order -0 below +0). Padding elements up to the row pitch get (0, 0);
+ *   - encode: c = clamp(rint((x - o_d) / s_d), 0, 255) as uint8 (rint: to nearest even), c = 0 where s_d == 0;
+ *   - decode: x' = fmaf((float)c, s_d, o_d), one rounding. The traversal runs the fp32 arithmetic on x', so
+ *     pops and evals are those of search(q, ef) on the decoded rows (the descent too);
+ *   - results: as F16, the popped set re-scored in fp32 on the fp32 rows, ordered by (exact distance, id),
+ *     first min(k, count): the distances are exact.
+ * The codebook is trained at the first SQ8 search after zvdb_set_storage(ix, ZVDB_STORAGE_SQ8) (setting it
+ * again retrains: the way to refresh it after many inserts), after a call that replaces the contents
+ * (zvdb_load, zvdb_load_graph, zvdb_build_from_candidates) and after a dim change. Inserts never retrain:
+ * later rows are encoded with the codebook there is, out-of-range coordinates saturate to 0 / 255 (a loss
+ * of traversal quality only; results stay exact), and capacity growth re-encodes with the same codebook.
+ * A non-finite coordinate fails the search with ZVDB_ERR_UNSUPPORTED naming the first such row; setting
+ * ZVDB_STORAGE_F32 recovers the handle. Refused with ZVDB_ERR_UNSUPPORTED like F16: SQ8 on an f64 / i32
+ * index, and the two exchange entry points on an SQ8 handle; and SQ8 searches of rows wider than 768
+ * dimensions (the kernels are built for up to 768). The device holds the fp32 rows AND the codes
+ * (cap_rows x row_floats bytes); switching storage frees the compact copy the new setting does not use
+ * (F32 frees both, and leaving SQ8 drops the codebook). Exact k-NN, zvdb_get_point and save / load use the
+ * fp32 rows; zvdb_save stores neither the setting nor the codebook. */
+#define ZVDB_STORAGE_SQ8 2   /* the search gathers 8-bit scalar-quantised codes; results are re-ranked in fp32 */
 ZVDB_API int zvdb_set_storage(zvdb_index *ix, int storage);
 ZVDB_API int zvdb_storage(const zvdb_index *ix);
+/* The SQ8 codebook in use: dim scales and dim offsets (dim = the index's, else ZVDB_ERR_DIM_MISMATCH).
+ * ZVDB_ERR_INVALID when none is trained (the storage is not SQ8, or no SQ8 search ran since it was set or
+ * the contents were replaced). code c of dimension d decodes to fmaf((float)c, scale[d], offset[d]). */
+ZVDB_API int zvdb_storage_codebook(const zvdb_index *ix, float *scale, float *offset, uint32_t dim);
 
 /* ---- on-disk format (SURVEY 8f rank 3; the reference has no persistence) --------------------------
  * zvdb_save writes the whole index -- vectors in the device layout, every layer, entry point, level

@@ -144,16 +144,21 @@ pub fn HNSW(comptime T: type) type {
         }
 
         /// Extension: which rows the graph search gathers. `.f16` = an fp16 copy of the rows (half the bytes per
-        /// evaluated row); the popped set is re-scored in fp32, so returned distances are exact. Takes effect at the
-        /// next search; not stored by `save`.
-        pub const Storage = enum(c_int) { f32 = 0, f16 = 1 };
+        /// evaluated row); `.sq8` = 8-bit codes with a per-dimension codebook (a quarter), trained at the next search.
+        /// The popped set is re-scored in fp32, so returned distances are exact. Takes effect at the next search; not
+        /// stored by `save`.
+        pub const Storage = enum(c_int) { f32 = 0, f16 = 1, sq8 = 2 };
         pub fn setStorage(self: *Self, storage: Storage) !void {
             const h = self.handle orelse return error.CudaError;
             try check(zvdb_set_storage(h, @intFromEnum(storage)));
         }
         pub fn storage(self: *const Self) Storage {
             const h = self.handle orelse return .f32;
-            return if (zvdb_storage(h) == 1) .f16 else .f32;
+            return switch (zvdb_storage(h)) {
+                1 => .f16,
+                2 => .sq8,
+                else => .f32,
+            };
         }
 
         /// Extension: the whole index to / from one file (the reference has no persistence).

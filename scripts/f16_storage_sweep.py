@@ -1,19 +1,25 @@
 #!/usr/bin/env python
-"""F32 vs F16 vector storage of the graph search (zvdb_set_storage) on one B200. JSON lines, one per point.
+"""F32 vs F16 vs SQ8 vector storage of the graph search (zvdb_set_storage) on one B200. JSON lines, one per point.
 
-    python scripts/f16_storage_sweep.py [--out profiles/r03_f16_storage.jsonl] [--parts throughput,c3,small] [--tag NAME]
+    python scripts/f16_storage_sweep.py [--out profiles/r03_storage.jsonl] [--parts goal,throughput,small,c3] [--tag NAME]
+        [--storages f32,f16,sq8]
 
+goal        The curve that answers the project's target (>= 1 M QPS at recall@10 >= 0.95 on 1M x 128): the incremental
+            quality graph at M = 32, ef 32..2048, QPS and recall@10 against K4 per storage, then one "goal_summary" line per
+            storage with the best recall among its points at >= 1 M QPS.
 throughput  1M x 128 L2 (bench.py's rows and queries: N(0,1) seeds 1 / 2), 10 000 queries, ef 32..512, on the reference
-            graph (insert) and on the search-driven incremental quality graph (bench.py's throughput track). F32 and F16
-            alternate in one process, three rounds; ms per launch = median over the rounds of CUDA-event time per launch.
-            recall@10 against K4's exact k-NN. Algorithmic bytes per query: evals x row bytes (512 fp32 / 256 f16)
-            + pops x 512 (F16: the fp32 re-rank of the popped set) + pops x m x 4 + dim x 4 + k x 12, and their rate as a
-            fraction of the device-to-device copy bandwidth measured in the same process. 1M rows are 512 MB (fp32) /
-            256 MB (f16): both exceed the 126 MB L2.
+            graph (insert) and on the search-driven incremental quality graph (bench.py's throughput track), M = 16.
+            The storages alternate in one process, three rounds; ms per launch = median over the rounds of CUDA-event time
+            per launch. recall@10 against K4's exact k-NN. Algorithmic bytes per query: evals x gathered row bytes (512 fp32,
+            256 f16, 128 SQ8 codes at 128-d: row_chunks x 4) + pops x dim x 4 (F16 / SQ8: the fp32 re-rank of the popped set)
+            + pops x m x 4 + dim x 4 + k x 12, and their rate as a fraction of the device-to-device copy bandwidth measured
+            in the same process. 1M rows are 512 MB (fp32) / 256 MB (f16): both exceed the 126 MB L2. The SQ8 codes are
+            128 MB, about the L2's size: much of their traffic may be served from L2, so a DRAM fraction must not be
+            inferred from the algorithmic bytes of SQ8 lines.
 c3          1M x 768 cosine, M = 32, k = 100, low-rank rows (scripts/configs_c3_c5.py "lowrank32"), quality graph from K4
             candidates, ef 100 / 256 / 512; recall@100 against K4.
 small       nq = 1 and 64 at ef = 64 on the reference graph: device time per launch of K1L (the kernel such batches run on)
-            under F32 and F16.
+            under each storage.
 unroll      F16 only, ef 128 / 256 on the incremental graph, for an A/B of the F16 unroll between two builds of the library
             (ZVDB_B200_LIB points at the other build, made by
             `python -m zvdb_b200.build --define ZVDB_F16_UNROLL=2 --out build/f16_unroll2/libzvdb_b200.so`); each line carries
@@ -109,13 +115,19 @@ def checksum(*arrays):
     return hsh.hexdigest()[:16]
 
 
-def sweep(torch, h, dq, nq, k, dim, m, efs, gt, stream, dev, base, emit, rounds=3, storages=("f32", "f16")):
+def gathered_row_bytes(storage, dim):
+    row_floats = (dim + 31) // 32 * 32
+    return {"f32": row_floats * 4, "f16": row_floats * 2, "sq8": row_floats}[storage]
+
+
+def sweep(torch, h, dq, nq, k, dim, m, efs, gt, stream, dev, base, emit, rounds=3, storages=("f32", "f16", "sq8")):
     b = Bufs(torch, dev, nq, k)
     bw = base.get("copy_gbs")
+    lines = []
     for ef in efs:
         ms = {s: [] for s in storages}
         out = {}
-        for _ in range(rounds):                             # F32 and F16 alternate
+        for _ in range(rounds):                             # the storages alternate
             for s in storages:
                 h.set_storage(s)
                 ms[s].append(time_search(torch, h, dq, nq, k, ef, b, stream))
@@ -123,10 +135,9 @@ def sweep(torch, h, dq, nq, k, dim, m, efs, gt, stream, dev, base, emit, rounds=
         for s in storages:
             ids, dist, cnt, pops, evals = out[s]
             t = float(np.median(ms[s]))
-            row_bytes = dim * 2 if s == "f16" else dim * 4
-            by = int(evals.astype(np.int64).sum()) * row_bytes + int(pops.astype(np.int64).sum()) * m * 4 + nq * (dim * 4 + k * 12)
-            if s == "f16":                                  # the re-rank reads the fp32 row of every popped node
-                by += int(pops.astype(np.int64).sum()) * dim * 4
+            by = int(evals.astype(np.int64).sum()) * gathered_row_bytes(s, dim) + int(pops.astype(np.int64).sum()) * m * 4 + nq * (dim * 4 + k * 12)
+            if s != "f32":                                  # the re-rank reads the fp32 row of every popped node
+                by += int(pops.astype(np.int64).sum()) * gathered_row_bytes("f32", dim)
             line = dict(base, storage=s, ef=ef, ms=round(t, 4), ms_rounds=[round(x, 4) for x in ms[s]], qps=nq / (t * 1e-3),
                         **{f"recall_at_{k}": recall(ids, gt)}, evals_per_query=float(evals.mean()), pops_per_query=float(pops.mean()),
                         algorithmic_bytes_per_query=by / nq, algorithmic_gbs=by / (t * 1e-3) / 1e9,
@@ -134,7 +145,9 @@ def sweep(torch, h, dq, nq, k, dim, m, efs, gt, stream, dev, base, emit, rounds=
             if bw:
                 line["frac_of_copy_bw"] = line["algorithmic_gbs"] / bw
             emit(line)
+            lines.append(line)
     h.set_storage("f32")
+    return lines
 
 
 def ground_truth(torch, h, dq, nq, k, dev, stream):
@@ -146,8 +159,9 @@ def ground_truth(torch, h, dq, nq, k, dev, stream):
 
 def main():
     ap = argparse.ArgumentParser()
-    ap.add_argument("--out", default=os.path.join(ROOT, "profiles", "r03_f16_storage.jsonl"))
-    ap.add_argument("--parts", default="throughput,c3,small")
+    ap.add_argument("--out", default=os.path.join(ROOT, "profiles", "r03_storage.jsonl"))
+    ap.add_argument("--parts", default="goal,throughput,small,c3")
+    ap.add_argument("--storages", default="f32,f16,sq8")
     ap.add_argument("--tag", default="", help="label of this run (e.g. which build of the library)")
     args = ap.parse_args()
     import torch
@@ -156,6 +170,7 @@ def main():
     dev = torch.device("cuda", 0)
     stream = torch.cuda.current_stream().cuda_stream
     parts = args.parts.split(",")
+    storages = tuple(args.storages.split(","))
     base = dict(card(), tag=args.tag, lib=os.environ.get("ZVDB_B200_LIB", "zvdb_b200/lib/libzvdb_b200.so"))
     base["copy_gbs"] = copy_gbs(torch, dev)
     os.makedirs(os.path.dirname(os.path.abspath(args.out)), exist_ok=True)
@@ -167,6 +182,31 @@ def main():
         fout.write(s + "\n"); fout.flush()
 
     n, dim, nq, k, m = 1_000_000, 128, 10_000, 10, 16
+    l2_note = "rows 512 MB fp32 / 256 MB f16 > 126 MB L2; SQ8 codes 128 MB ~ L2 size: no DRAM fraction from SQ8 algorithmic bytes"
+    if "goal" in parts:
+        X = np.random.default_rng(1).standard_normal((n, dim), dtype=np.float32)
+        Q = np.random.default_rng(2).standard_normal((nq, dim), dtype=np.float32)
+        dq = torch.from_numpy(Q).to(dev)
+        mg = 32
+        h = zvdb_b200.HNSW(mg, 200)
+        t0 = time.time()
+        builder.build_quality_graph_incremental(h, X, mg)
+        h.sync_device()
+        b = dict(base, part="goal", data="1M x 128 N(0,1), L2", graph="incremental", n=n, dim=dim, nq=nq, k=k, m=mg,
+                 build_s=round(time.time() - t0, 1), l2_note=l2_note)
+        gt = ground_truth(torch, h, dq, nq, k, dev, stream)
+        lines = sweep(torch, h, dq, nq, k, dim, mg, (32, 64, 128, 256, 512, 1024, 2048), gt, stream, dev, b, emit,
+                      storages=storages)
+        for s in storages:
+            fast = [ln for ln in lines if ln["storage"] == s and ln["qps"] >= 1e6]
+            best = max(fast, key=lambda ln: ln[f"recall_at_{k}"]) if fast else None
+            emit(dict(base, part="goal_summary", graph="incremental", m=mg, storage=s, target="recall@10 >= 0.95 at >= 1 M QPS",
+                      best_recall_at_1M_qps=best[f"recall_at_{k}"] if best else None, at_ef=best["ef"] if best else None,
+                      qps=best["qps"] if best else None,
+                      target_met=bool(best and best[f"recall_at_{k}"] >= 0.95)))
+        h.deinit()
+        del X, dq
+
     if any(p in parts for p in ("throughput", "small", "unroll")):
         X = np.random.default_rng(1).standard_normal((n, dim), dtype=np.float32)
         Q = np.random.default_rng(2).standard_normal((nq, dim), dtype=np.float32)
@@ -183,11 +223,11 @@ def main():
                 builder.build_quality_graph_incremental(h, X, m)
             h.sync_device()
             b = dict(base, part="throughput", data="1M x 128 N(0,1), L2", graph=graph, n=n, dim=dim, nq=nq, k=k, m=m,
-                     build_s=round(time.time() - t0, 1), l2_note="rows 512 MB fp32 / 256 MB f16 > 126 MB L2")
+                     build_s=round(time.time() - t0, 1), l2_note=l2_note)
             if gt is None:
                 gt = ground_truth(torch, h, dq, nq, k, dev, stream)
             if "throughput" in parts:
-                sweep(torch, h, dq, nq, k, dim, m, (32, 64, 128, 256, 512), gt, stream, dev, b, emit)
+                sweep(torch, h, dq, nq, k, dim, m, (32, 64, 128, 256, 512), gt, stream, dev, b, emit, storages=storages)
             if "unroll" in parts and graph == "incremental":
                 sweep(torch, h, dq, nq, k, dim, m, (128, 256), gt, stream, dev, dict(b, part="unroll"), emit, rounds=5, storages=("f16",))
             if "small" in parts and graph == "reference":
@@ -195,7 +235,7 @@ def main():
                     sb = Bufs(torch, dev, 64 * bs, k)
                     us = {}
                     for _ in range(3):
-                        for s in ("f32", "f16"):
+                        for s in storages:
                             h.set_storage(s)
                             h.set_kernel_variant(2 << 14)           # K1L (what batches this small run on by default)
                             def launch(i):
@@ -213,7 +253,7 @@ def main():
                             us.setdefault(s, []).append(e0.elapsed_time(e1) / 128 * 1e3)
                     h.set_kernel_variant(0)
                     h.set_storage("f32")
-                    for s in ("f32", "f16"):
+                    for s in storages:
                         emit(dict(base, part="small_batch", graph=graph, kernel="K1L (variant bits 14-15 = 2)", nq=bs, ef=64, k=k,
                                   storage=s, device_us=float(np.median(us[s])), device_us_rounds=[round(x, 2) for x in us[s]]))
             h.deinit()
@@ -230,8 +270,8 @@ def main():
         dq = torch.from_numpy(Q).to(dev)
         gt = ground_truth(torch, h, dq, nq3, k3, dev, stream)
         b = dict(base, part="c3", data="1M x 768 lowrank32, cosine", graph="quality (exact K4 candidates)", n=n3, dim=dim3, nq=nq3,
-                 k=k3, m=m3, build_s=round(time.time() - t0, 1), l2_note="rows 3.07 GB fp32 / 1.54 GB f16 > 126 MB L2")
-        sweep(torch, h, dq, nq3, k3, dim3, m3, (100, 256, 512), gt, stream, dev, b, emit)
+                 k=k3, m=m3, build_s=round(time.time() - t0, 1), l2_note="rows 3.07 GB fp32 / 1.54 GB f16 / 0.77 GB SQ8 > 126 MB L2")
+        sweep(torch, h, dq, nq3, k3, dim3, m3, (100, 256, 512), gt, stream, dev, b, emit, storages=storages)
         h.deinit()
     fout.close()
 

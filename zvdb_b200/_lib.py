@@ -14,7 +14,7 @@ LIB_PATH = os.environ.get("ZVDB_B200_LIB") or os.path.join(_HERE, "lib", "libzvd
 
 OK, ERR_OOM, ERR_NODE_NOT_FOUND, ERR_DIM_MISMATCH, ERR_CUDA, ERR_INVALID, ERR_UNSUPPORTED = range(7)
 METRIC_L2, METRIC_COSINE, METRIC_DOT = 0, 1, 2
-STORAGE_F32, STORAGE_F16 = 0, 1
+STORAGE_F32, STORAGE_F16, STORAGE_SQ8 = 0, 1, 2
 INVALID_ID = 0xFFFFFFFFFFFFFFFF
 
 _u32, _u64, _i32, _i64, _vp = C.c_uint32, C.c_uint64, C.c_int, C.c_int64, C.c_void_p
@@ -47,6 +47,7 @@ SIGNATURES = {
     "zvdb_descent_start": (_i64, [_vp]),
     "zvdb_set_storage": (_i32, [_vp, _i32]),
     "zvdb_storage": (_i32, [_vp]),
+    "zvdb_storage_codebook": (_i32, [_vp, _pf, _pf, _u32]),
     "zvdb_export_upper_layers": (_i32, [_vp, _vp, _vp, _vp, _pu64]),
     "zvdb_load_upper_layers": (_i32, [_vp, _vp, _vp, _u64, _u64]),
     "zvdb_save": (_i32, [_vp, C.c_char_p]),

@@ -65,6 +65,45 @@ __global__ void arena_to_f16_kernel(uint2 *__restrict__ dst, const float4 *__res
     }
 }
 
+// SQ8 storage, training: per-dimension min and max over rows [0, n) of the fp32 arena, as order-preserving words
+// (float_to_ordered, -0 < +0), and the first row holding a non-finite coordinate (*bad_row, atomicMin; ~0 = none). Min
+// and max do not depend on the order the rows are seen in, so the codebook is deterministic. One thread per element of
+// a row (blockDim.x = row_floats), each block a stripe of rows.
+__global__ void sq8_minmax_kernel(uint32_t *__restrict__ mn, uint32_t *__restrict__ mx, const float *__restrict__ src, uint64_t n,
+                                  uint32_t row_floats, uint32_t dim, uint32_t *__restrict__ bad_row) {
+    const uint32_t d = threadIdx.x;
+    if (d >= dim) return;
+    uint32_t lo = ~0u, hi = 0u, bad = ~0u;
+    for (uint64_t r = blockIdx.x; r < n; r += gridDim.x) {
+        const float x = src[r * row_floats + d];
+        if (!isfinite(x)) bad = min(bad, static_cast<uint32_t>(r));
+        const uint32_t o = float_to_ordered(x);
+        lo = min(lo, o); hi = max(hi, o);
+    }
+    atomicMin(mn + d, lo); atomicMax(mx + d, hi);
+    if (bad != ~0u) atomicMin(bad_row, bad);
+}
+
+// The SQ8 code of one element: clamp(rint((x - o) / s), 0, 255), 0 when s == 0 (a constant dimension, or padding).
+__device__ __forceinline__ uint32_t sq8_code(float x, float s, float o) {
+    if (s == 0.f) return 0u;
+    return static_cast<uint32_t>(fminf(fmaxf(rintf(__fdiv_rn(__fsub_rn(x, o), s)), 0.f), 255.f));
+}
+// SQ8 storage: rows [r0, r1) of the fp32 arena encoded with the codebook cb ([2][row_chunks]: scales, offsets) into the
+// code copy (one 4-byte word per 4-float chunk). The first row with a non-finite coordinate goes to *bad_row.
+__global__ void arena_to_sq8_kernel(uint32_t *__restrict__ dst, const float4 *__restrict__ src, const float4 *__restrict__ cb,
+                                    uint64_t r0, uint64_t r1, uint32_t row_chunks, uint32_t *__restrict__ bad_row) {
+    const uint64_t begin = r0 * row_chunks, end = r1 * row_chunks;
+    for (uint64_t i = begin + blockIdx.x * static_cast<uint64_t>(blockDim.x) + threadIdx.x; i < end;
+         i += static_cast<uint64_t>(gridDim.x) * blockDim.x) {
+        const uint32_t c = static_cast<uint32_t>(i % row_chunks);
+        const float4 v = src[i], sc = cb[c], of = cb[row_chunks + c];
+        if (!(isfinite(v.x) && isfinite(v.y) && isfinite(v.z) && isfinite(v.w))) atomicMin(bad_row, static_cast<uint32_t>(i / row_chunks));
+        dst[i] = sq8_code(v.x, sc.x, of.x) | (sq8_code(v.y, sc.y, of.y) << 8) | (sq8_code(v.z, sc.z, of.z) << 16) |
+                 (sq8_code(v.w, sc.w, of.w) << 24);
+    }
+}
+
 template <typename T>
 struct DevBuf {
     T *p = nullptr;
@@ -108,7 +147,14 @@ struct zvdb_index {
     int storage = ZVDB_STORAGE_F32; // rows the graph search gathers (zvdb_set_storage)
     uint2 *d_arena16 = nullptr;     // ZVDB_STORAGE_F16: [cap_rows][row_floats] __half copy of d_arena, rows [0, f16_rows) current
     uint64_t f16_rows = 0;
-    DevBuf<uint32_t> f16_bad;       // first row the conversion found out of the f16 range (~0 = none)
+    DevBuf<uint32_t> f16_bad;       // first row the conversion found out of the f16 range, or (SQ8) non-finite (~0 = none)
+    // ZVDB_STORAGE_SQ8: one allocation, the codebook [2][row_floats] fp32 (scales, then offsets) followed by the 8-bit codes
+    // of d_arena [cap_rows][row_floats], rows [0, sq8_rows) current (the kernels find the codebook in front of the codes)
+    unsigned char *d_sq8 = nullptr;
+    uint64_t sq8_rows = 0;
+    bool sq8_trained = false;       // the codebook belongs to these contents (else the next SQ8 search trains it)
+    std::vector<float> sq8_scale, sq8_offset;   // the codebook, [row_floats] each (zero for the padding elements)
+    DevBuf<uint32_t> sq8_minmax;    // training scratch, [2][row_floats] ordered min / max
     DevBuf<float> q_buf, dist_buf;
     DevBuf<uint64_t> ids_buf;
     DevBuf<uint32_t> cnt_buf, pops_buf, evals_buf, scat_rows, scat_ids, bitmap_buf, vlog_buf;
@@ -153,10 +199,15 @@ static int ensure_capacity(zvdb_index *ix, uint64_t rows) {
         cudaFree(ix->d_arena); cudaFree(ix->d_adj);
         ix->d_arena = nullptr; ix->d_adj = nullptr; ix->cap_rows = 0; ix->n_dev = 0; ix->bf_rows = 0;
         ix->cap_row_floats = g.row_floats; ix->cap_m = g.m;
+        ix->sq8_trained = false;                          // a new row pitch: the next SQ8 search trains a codebook for it
     }
     if (ix->d_arena16) {                                  // the f16 copy is sized like the arena: the next F16 search rebuilds it
         ZV_CUDA(cudaDeviceSynchronize());
         cudaFree(ix->d_arena16); ix->d_arena16 = nullptr; ix->f16_rows = 0;
+    }
+    if (ix->d_sq8) {                                      // so is the code copy: re-encoded (same codebook) by the next SQ8 search
+        ZV_CUDA(cudaDeviceSynchronize());
+        cudaFree(ix->d_sq8); ix->d_sq8 = nullptr; ix->sq8_rows = 0;
     }
     uint64_t nc = std::max<uint64_t>(rows, std::max<uint64_t>(ix->cap_rows * 2, 1024));
     float *na = nullptr; uint32_t *nj = nullptr;
@@ -185,6 +236,7 @@ static int sync_device_locked(zvdb_index *ix) {
     int rc = ensure_capacity(ix, g.n);
     if (rc) return rc;
     ix->f16_rows = std::min<uint64_t>(ix->f16_rows, g.rows_uploaded);   // rows from rows_uploaded on are (re)written now
+    ix->sq8_rows = std::min<uint64_t>(ix->sq8_rows, g.rows_uploaded);
     for (uint64_t r = g.rows_uploaded; r < g.n;) {
         const uint64_t chunk = r / g.rows_per_chunk;
         const uint64_t end = std::min<uint64_t>(g.n, (chunk + 1) * g.rows_per_chunk);
@@ -252,6 +304,74 @@ static int sync_f16_locked(zvdb_index *ix) {
     return ZVDB_OK;
 }
 
+// ZVDB_STORAGE_SQ8: bring the code copy up to the device rows (after sync_device_locked). Without a codebook for these
+// contents, one is trained first on rows [0, n_dev): o = min, s = (max - min) / 255 per dimension, each a single IEEE
+// operation on the host; then every row is (re-)encoded. Later rows [sq8_rows, n_dev) are encoded with the codebook
+// they find. A non-finite coordinate fails the search that got here and every later one under SQ8 (nothing moves past
+// the row); zvdb_set_storage(F32) recovers the handle.
+static int sync_sq8_locked(zvdb_index *ix) {
+    const HostGraph &g = ix->g;
+    if (g.dtype != 0) return fail(ZVDB_ERR_UNSUPPORTED, "sq8 storage: the index holds f64 / i32 rows; set ZVDB_STORAGE_F32");
+    if (ix->sq8_trained && ix->sq8_rows >= ix->n_dev) return ZVDB_OK;
+    const uint32_t rf = g.row_floats, row_chunks = rf / 4;
+    uint32_t bad = ~0u;
+    ZV_CUDA(ix->f16_bad.reserve(1));
+    ZV_CUDA(cudaMemsetAsync(ix->f16_bad.p, 0xFF, sizeof(uint32_t), ix->stream));
+    if (!ix->sq8_trained) {
+        ZV_CUDA(cudaDeviceSynchronize());                 // searches enqueued on caller streams may still read the codebook and codes
+        ZV_CUDA(ix->sq8_minmax.reserve(2ull * rf));
+        ZV_CUDA(cudaMemsetAsync(ix->sq8_minmax.p, 0xFF, rf * sizeof(uint32_t), ix->stream));   // min: above every word
+        ZV_CUDA(cudaMemsetAsync(ix->sq8_minmax.p + rf, 0, rf * sizeof(uint32_t), ix->stream)); // max: below every word
+        const unsigned blocks = static_cast<unsigned>(std::min<uint64_t>(ix->n_dev, static_cast<uint64_t>(ix->num_sms) * 8));
+        sq8_minmax_kernel<<<blocks, rf, 0, ix->stream>>>(ix->sq8_minmax.p, ix->sq8_minmax.p + rf, ix->d_arena, ix->n_dev, rf, g.dim,
+                                                         ix->f16_bad.p);
+        ix->launches++;
+        ZV_CUDA(cudaGetLastError());
+        std::vector<uint32_t> mm(2ull * rf);
+        ZV_CUDA(cudaMemcpyAsync(mm.data(), ix->sq8_minmax.p, mm.size() * sizeof(uint32_t), cudaMemcpyDeviceToHost, ix->stream));
+        ZV_CUDA(cudaMemcpyAsync(&bad, ix->f16_bad.p, sizeof bad, cudaMemcpyDeviceToHost, ix->stream));
+        ZV_CUDA(cudaStreamSynchronize(ix->stream));
+        if (bad == ~0u) {
+            ix->sq8_scale.assign(rf, 0.0f); ix->sq8_offset.assign(rf, 0.0f);   // padding elements (d >= dim): (s, o) = (0, 0)
+            for (uint32_t d = 0; d < g.dim; ++d) {
+                const float lo = ordered_to_float(mm[d]), hi = ordered_to_float(mm[rf + d]);
+                ix->sq8_scale[d] = (hi - lo) / 255.0f;    // (built without contraction: two IEEE operations)
+                ix->sq8_offset[d] = lo;
+            }
+            ix->sq8_trained = true; ix->sq8_rows = 0;
+            if (ix->d_sq8) {                              // a copy from an earlier codebook: every row is re-encoded below
+                ZV_CUDA(cudaMemcpyAsync(ix->d_sq8, ix->sq8_scale.data(), rf * sizeof(float), cudaMemcpyHostToDevice, ix->stream));
+                ZV_CUDA(cudaMemcpyAsync(ix->d_sq8 + rf * sizeof(float), ix->sq8_offset.data(), rf * sizeof(float), cudaMemcpyHostToDevice, ix->stream));
+            }
+        }
+    }
+    if (bad == ~0u && !ix->d_sq8) {                       // (first SQ8 search, or after capacity growth: same codebook)
+        ZV_CUDA(cudaMalloc(&ix->d_sq8, 8ull * rf + ix->cap_rows * rf));
+        ZV_CUDA(cudaMemcpyAsync(ix->d_sq8, ix->sq8_scale.data(), rf * sizeof(float), cudaMemcpyHostToDevice, ix->stream));
+        ZV_CUDA(cudaMemcpyAsync(ix->d_sq8 + rf * sizeof(float), ix->sq8_offset.data(), rf * sizeof(float), cudaMemcpyHostToDevice, ix->stream));
+        ix->sq8_rows = 0;
+    }
+    if (bad == ~0u && ix->sq8_rows < ix->n_dev) {
+        const uint64_t total = (ix->n_dev - ix->sq8_rows) * row_chunks;
+        const unsigned blocks = static_cast<unsigned>(std::min<uint64_t>((total + 255) / 256, static_cast<uint64_t>(ix->num_sms) * 8));
+        arena_to_sq8_kernel<<<blocks, 256, 0, ix->stream>>>(reinterpret_cast<uint32_t *>(ix->d_sq8 + 8ull * rf),
+                                                            reinterpret_cast<const float4 *>(ix->d_arena),
+                                                            reinterpret_cast<const float4 *>(ix->d_sq8), ix->sq8_rows, ix->n_dev,
+                                                            row_chunks, ix->f16_bad.p);
+        ix->launches++;
+        ZV_CUDA(cudaGetLastError());
+        ZV_CUDA(cudaMemcpyAsync(&bad, ix->f16_bad.p, sizeof bad, cudaMemcpyDeviceToHost, ix->stream));
+        ZV_CUDA(cudaStreamSynchronize(ix->stream));
+    }
+    if (bad != ~0u) {
+        char buf[200];
+        snprintf(buf, sizeof buf, "sq8 storage: row %u has a non-finite coordinate; set ZVDB_STORAGE_F32 to search this index", bad);
+        return fail(ZVDB_ERR_UNSUPPORTED, buf);
+    }
+    ix->sq8_rows = ix->n_dev;
+    return ZVDB_OK;
+}
+
 // Device copy of layers >= 1 for the descent (K2): levels[n], upper_base[n], upper_adj[n_lists][m].
 // Re-sent whole whenever a list above layer 0 changed (half the nodes have one; the reference links
 // one neighbour per layer and insert, hnsw.zig:106-108).
@@ -297,7 +417,7 @@ static cudaError_t launch_search_metric(int cpl, const SearchParams &p, unsigned
         case 2: return launch_search_inst<2, METRIC, VIS, EXCH, ROWF>(p, grid, smem, s);
         case 4: return launch_search_inst<4, METRIC, VIS, EXCH, ROWF>(p, grid, smem, s);
         case 6: return launch_search_inst<6, METRIC, VIS, EXCH, ROWF>(p, grid, smem, s);
-        case 8: return launch_search_inst<8, METRIC, VIS, EXCH, ROWF>(p, grid, smem, s);
+        case 8: if constexpr (ROWF != kRowSQ8) return launch_search_inst<8, METRIC, VIS, EXCH, ROWF>(p, grid, smem, s); break;
     }
     return cudaErrorInvalidValue;
 }
@@ -312,10 +432,12 @@ static cudaError_t launch_search_vis2(int metric, int cpl, const SearchParams &p
 }
 
 // exch = any sharded form of the step (peer stores, records, flags, merge tail): its own instantiation, see the kernel.
-// f16 = the plain search over the f16 copy with the exact re-rank (never together with exch: the entry points refuse it).
+// rowf = the rows the search gathers: kRowF16 / kRowSQ8 = the plain search over the compact copy with the exact re-rank
+// (never together with exch: the entry points refuse it).
 template <int VIS>
-static cudaError_t launch_search_vis(bool exch, bool f16, int metric, int cpl, const SearchParams &p, unsigned grid, size_t smem, cudaStream_t s) {
-    if (f16) return launch_search_vis2<VIS, false, kRowF16>(metric, cpl, p, grid, smem, s);
+static cudaError_t launch_search_vis(bool exch, int rowf, int metric, int cpl, const SearchParams &p, unsigned grid, size_t smem, cudaStream_t s) {
+    if (rowf == kRowF16) return launch_search_vis2<VIS, false, kRowF16>(metric, cpl, p, grid, smem, s);
+    if (rowf == kRowSQ8) return launch_search_vis2<VIS, false, kRowSQ8>(metric, cpl, p, grid, smem, s);
     return exch ? launch_search_vis2<VIS, true, kRowF32>(metric, cpl, p, grid, smem, s) : launch_search_vis2<VIS, false, kRowF32>(metric, cpl, p, grid, smem, s);
 }
 
@@ -326,7 +448,7 @@ static cudaError_t launch_descend_metric(int cpl, const SearchParams &p, unsigne
         case 2: descend_kernel<2, METRIC, ROWF><<<grid, 128, 0, s>>>(p); break;
         case 4: descend_kernel<4, METRIC, ROWF><<<grid, 128, 0, s>>>(p); break;
         case 6: descend_kernel<6, METRIC, ROWF><<<grid, 128, 0, s>>>(p); break;
-        case 8: descend_kernel<8, METRIC, ROWF><<<grid, 128, 0, s>>>(p); break;
+        case 8: if constexpr (ROWF != kRowSQ8) { descend_kernel<8, METRIC, ROWF><<<grid, 128, 0, s>>>(p); break; } else return cudaErrorInvalidValue;
         default: return cudaErrorInvalidValue;
     }
     return cudaGetLastError();
@@ -339,15 +461,19 @@ static cudaError_t launch_descend_rowf(int metric, int cpl, const SearchParams &
         default: return launch_descend_metric<kMetricDot, ROWF>(cpl, p, grid, s);
     }
 }
-// f16 = the descent walks the f16 copy, like the layer-0 search it seeds
-static cudaError_t launch_descend(bool f16, int metric, int cpl, const SearchParams &p, unsigned grid, cudaStream_t s) {
-    return f16 ? launch_descend_rowf<kRowF16>(metric, cpl, p, grid, s) : launch_descend_rowf<kRowF32>(metric, cpl, p, grid, s);
+// rowf = the rows the descent walks: those of the layer-0 search it seeds
+static cudaError_t launch_descend(int rowf, int metric, int cpl, const SearchParams &p, unsigned grid, cudaStream_t s) {
+    if (rowf == kRowF16) return launch_descend_rowf<kRowF16>(metric, cpl, p, grid, s);
+    if (rowf == kRowSQ8) return launch_descend_rowf<kRowSQ8>(metric, cpl, p, grid, s);
+    return launch_descend_rowf<kRowF32>(metric, cpl, p, grid, s);
 }
 
 // K1L, the latency form: one CTA of 8 (or 4) warps per query (search_team_kernel.cuh)
 template <int CPL, int METRIC, bool ADJC, int MC, int T, int ROWF>
 static cudaError_t launch_team_inst3(const SearchParams &p, unsigned grid, size_t smem, cudaStream_t s) {
-    auto kern = ROWF == kRowF16 ? search_team_f16_kernel<CPL, METRIC, ADJC, MC, T> : search_team_kernel<CPL, METRIC, ADJC, MC, T>;
+    auto kern = search_team_kernel<CPL, METRIC, ADJC, MC, T>;     // (if constexpr: only the format's own kernel is instantiated)
+    if constexpr (ROWF == kRowF16) kern = search_team_f16_kernel<CPL, METRIC, ADJC, MC, T>;
+    else if constexpr (ROWF == kRowSQ8) kern = search_team_sq8_kernel<CPL, METRIC, ADJC, MC, T>;
     if (smem > 48 * 1024) {
         cudaError_t e = cudaFuncSetAttribute(kern, cudaFuncAttributeMaxDynamicSharedMemorySize, static_cast<int>(smem));
         if (e != cudaSuccess) return e;
@@ -371,7 +497,7 @@ static cudaError_t launch_team_metric(int cpl, bool adjc, unsigned threads, cons
         case 2: return launch_team_inst<2, METRIC, ROWF>(adjc, threads, p, grid, smem, s);
         case 4: return launch_team_inst<4, METRIC, ROWF>(adjc, threads, p, grid, smem, s);
         case 6: return launch_team_inst<6, METRIC, ROWF>(adjc, threads, p, grid, smem, s);
-        case 8: return launch_team_inst<8, METRIC, ROWF>(adjc, threads, p, grid, smem, s);
+        case 8: if constexpr (ROWF != kRowSQ8) return launch_team_inst<8, METRIC, ROWF>(adjc, threads, p, grid, smem, s); break;
     }
     return cudaErrorInvalidValue;
 }
@@ -383,10 +509,11 @@ static cudaError_t launch_team_rowf(int metric, int cpl, bool adjc, unsigned thr
         default: return launch_team_metric<kMetricDot, ROWF>(cpl, adjc, threads, p, grid, smem, s);
     }
 }
-// adjc = every candidate's adjacency row kept in shared memory (no dependent adjacency fetch at a pop); f16 = over the f16 copy
-static cudaError_t launch_team(bool f16, int metric, int cpl, bool adjc, unsigned threads, const SearchParams &p, unsigned grid, size_t smem, cudaStream_t s) {
-    return f16 ? launch_team_rowf<kRowF16>(metric, cpl, adjc, threads, p, grid, smem, s)
-               : launch_team_rowf<kRowF32>(metric, cpl, adjc, threads, p, grid, smem, s);
+// adjc = every candidate's adjacency row kept in shared memory (no dependent adjacency fetch at a pop); rowf = the rows gathered
+static cudaError_t launch_team(int rowf, int metric, int cpl, bool adjc, unsigned threads, const SearchParams &p, unsigned grid, size_t smem, cudaStream_t s) {
+    if (rowf == kRowF16) return launch_team_rowf<kRowF16>(metric, cpl, adjc, threads, p, grid, smem, s);
+    if (rowf == kRowSQ8) return launch_team_rowf<kRowSQ8>(metric, cpl, adjc, threads, p, grid, smem, s);
+    return launch_team_rowf<kRowF32>(metric, cpl, adjc, threads, p, grid, smem, s);
 }
 
 // Where the exact visited set of a search with pop budget `ef` lives (see launch_search).
@@ -443,16 +570,23 @@ static int launch_search(zvdb_index *ix, const float *d_q, uint64_t nq, uint32_t
     const HostGraph &g = ix->g;
     if (nq == 0) return ZVDB_OK;
     if (nq > 0x7FFFFFFFull) return fail(ZVDB_ERR_UNSUPPORTED, "nq exceeds 2^31-1 queries per launch");
-    // F16 storage: the plain search gathers the f16 copy (brought up to date here) and re-ranks on the fp32 arena
-    const bool f16 = ix->storage == ZVDB_STORAGE_F16 && g.n > 0;
-    if (f16 && (fx || n_peers)) return fail(ZVDB_ERR_UNSUPPORTED, "f16 storage: the sharded exchange forms gather fp32 rows only");
-    if (f16) {
-        int rcf = sync_f16_locked(ix);
+    // F16 / SQ8 storage: the plain search gathers the compact copy (brought up to date here) and re-ranks on the fp32
+    // arena. The row format is the storage value.
+    static_assert(ZVDB_STORAGE_F16 == kRowF16 && ZVDB_STORAGE_SQ8 == kRowSQ8, "storage values name the row formats");
+    const int rowf = g.n > 0 ? ix->storage : kRowF32;
+    if (rowf != kRowF32 && (fx || n_peers))
+        return fail(ZVDB_ERR_UNSUPPORTED, rowf == kRowF16 ? "f16 storage: the sharded exchange forms gather fp32 rows only"
+                                                          : "sq8 storage: the sharded exchange forms gather fp32 rows only");
+    if (rowf == kRowSQ8 && g.row_floats > 128u * kSq8MaxCpl)
+        return fail(ZVDB_ERR_UNSUPPORTED, "sq8 storage: built for rows of up to 768 dimensions; set ZVDB_STORAGE_F32 or ZVDB_STORAGE_F16");
+    if (rowf != kRowF32) {
+        int rcf = rowf == kRowF16 ? sync_f16_locked(ix) : sync_sq8_locked(ix);
         if (rcf) return rcf;
     }
     SearchParams p{};
     p.arena = reinterpret_cast<const float4 *>(ix->d_arena);
-    p.arena16 = f16 ? ix->d_arena16 : nullptr;
+    p.arena16 = rowf == kRowF16 ? ix->d_arena16 : nullptr;
+    p.arena8 = rowf == kRowSQ8 ? reinterpret_cast<const uint32_t *>(ix->d_sq8 + 8ull * g.row_floats) : nullptr;
     p.adj = ix->d_adj;
     p.queries = d_q;
     p.ids = d_ids; p.dist = d_dist; p.counts = d_counts; p.pops = d_pops; p.evals = d_evals;
@@ -515,14 +649,14 @@ static int launch_search(zvdb_index *ix, const float *d_q, uint64_t nq, uint32_t
             cudaError_t e;
             if (p.seeds) {                                    // K2 first (its seeds are per-handle scratch: ordered across streams)
                 ZV_CUDA(cudaStreamWaitEvent(s, ix->bitmap_ev, 0));
-                e = launch_descend(f16, g.metric, cpl, p, static_cast<unsigned>((nq + 3) / 4), s);
+                e = launch_descend(rowf, g.metric, cpl, p, static_cast<unsigned>((nq + 3) / 4), s);
                 ix->launches++;
                 ZV_CUDA(e);
             }
             p.slots = static_cast<uint32_t>(slots); p.hash_words = static_cast<uint32_t>(hash_words);
             p.cand_cap = static_cast<uint32_t>(team_cap);
             if (ix->mailbox_dev && nq == 1) { p.done_flag = ix->mailbox_dev; p.done_seq = ix->mailbox_seq; ix->mailbox_armed = true; }
-            e = launch_team(f16, g.metric, cpl, adjc, threads, p, static_cast<unsigned>(nq), static_cast<size_t>(team_smem), s);
+            e = launch_team(rowf, g.metric, cpl, adjc, threads, p, static_cast<unsigned>(nq), static_cast<size_t>(team_smem), s);
             ix->launches++;
             ZV_CUDA(e);
             if (p.seeds) ZV_CUDA(cudaEventRecord(ix->bitmap_ev, s));
@@ -625,14 +759,14 @@ static int launch_search(zvdb_index *ix, const float *d_q, uint64_t nq, uint32_t
     if (p.seeds) {                                        // K2 first: one warp per query, 4 per CTA
         // the seeds are per-handle scratch like the tables: order launches from different streams
         if (vis == kVisSmemHash) ZV_CUDA(cudaStreamWaitEvent(s, ix->bitmap_ev, 0));
-        e = launch_descend(f16, g.metric, cpl, p, static_cast<unsigned>((nq + 3) / 4), s);
+        e = launch_descend(rowf, g.metric, cpl, p, static_cast<unsigned>((nq + 3) / 4), s);
         ix->launches++;
         ZV_CUDA(e);
     }
     const bool exch = n_peers != 0 || fx != nullptr;
-    if (vis == kVisSmemHash) e = launch_search_vis<kVisSmemHash>(exch, f16, g.metric, cpl, p, grid, smem, s);
-    else if (vis == kVisGlobalBitmap) e = launch_search_vis<kVisGlobalBitmap>(exch, f16, g.metric, cpl, p, grid, smem, s);
-    else e = launch_search_vis<kVisGlobalHash>(exch, f16, g.metric, cpl, p, grid, smem, s);
+    if (vis == kVisSmemHash) e = launch_search_vis<kVisSmemHash>(exch, rowf, g.metric, cpl, p, grid, smem, s);
+    else if (vis == kVisGlobalBitmap) e = launch_search_vis<kVisGlobalBitmap>(exch, rowf, g.metric, cpl, p, grid, smem, s);
+    else e = launch_search_vis<kVisGlobalHash>(exch, rowf, g.metric, cpl, p, grid, smem, s);
     ix->launches++;
     ZV_CUDA(e);
     if (vis != kVisSmemHash || p.seeds) ZV_CUDA(cudaEventRecord(ix->bitmap_ev, s));
@@ -1042,9 +1176,9 @@ void zvdb_destroy(zvdb_index *ix) {
     for (int i = 0; i < 8; ++i) if (ix->in_ev[i]) cudaEventDestroy(ix->in_ev[i]);
     if (ix->bitmap_ev) cudaEventDestroy(ix->bitmap_ev);
     if (ix->bf_ev) cudaEventDestroy(ix->bf_ev);
-    cudaFree(ix->d_arena); cudaFree(ix->d_adj); cudaFree(ix->d_arena16);
+    cudaFree(ix->d_arena); cudaFree(ix->d_adj); cudaFree(ix->d_arena16); cudaFree(ix->d_sq8);
     if (ix->h_stage) cudaFreeHost(ix->h_stage);
-    ix->f16_bad.free_();
+    ix->f16_bad.free_(); ix->sq8_minmax.free_();
     ix->q_buf.free_(); ix->dist_buf.free_(); ix->ids_buf.free_(); ix->cnt_buf.free_();
     ix->pops_buf.free_(); ix->evals_buf.free_(); ix->scat_rows.free_(); ix->scat_ids.free_(); ix->bitmap_buf.free_(); ix->vlog_buf.free_(); ix->res_buf.free_(); ix->gtable_buf.free_();
     ix->d_level.free_(); ix->d_upper_base.free_(); ix->d_upper_adj.free_(); ix->seeds_buf.free_();
@@ -1252,7 +1386,7 @@ static int set_points_locked(zvdb_index *ix, const float *points, uint64_t n, ui
     }
     g.has_entry = n > 0; g.entry = entry; g.max_level = 0;
     g.rows_uploaded = 0; g.adj_all_dirty = true;
-    ix->n_dev = 0; ix->bf_rows = 0; ix->f16_rows = 0;
+    ix->n_dev = 0; ix->bf_rows = 0; ix->f16_rows = 0; ix->sq8_rows = 0; ix->sq8_trained = false;
     return ZVDB_OK;
 }
 
@@ -1359,7 +1493,7 @@ int zvdb_load(zvdb_index *ix, const char *path) {
         g.dim = 0; g.row_floats = 0; g.rows_per_chunk = 0;
         if (hd.dim) g.fix_dim(hd.dim);
         g.ef_construction = hd.ef_construction; g.rng = hd.rng; g.dtype = 0;
-        ix->n_dev = 0; ix->bf_rows = 0; ix->f16_rows = 0;
+        ix->n_dev = 0; ix->bf_rows = 0; ix->f16_rows = 0; ix->sq8_rows = 0; ix->sq8_trained = false;
         return ZVDB_OK;
     }
     if (hd.dim == 0 || hd.dim > 1024 || hd.row_floats != (hd.dim + 31u) / 32u * 32u || hd.n >= 0xFFFFFFFEull || hd.max_level > 31 ||
@@ -1436,7 +1570,7 @@ int zvdb_load(zvdb_index *ix, const char *path) {
     g.upper_off.swap(fresh.upper_off); g.upper.swap(fresh.upper);
     g.has_entry = fresh.has_entry; g.entry = fresh.entry; g.max_level = fresh.max_level; g.top_node = fresh.top_node; g.rng = fresh.rng;
     ++g.upper_version; g.rows_uploaded = 0; g.dirty.clear(); g.adj_all_dirty = true;
-    ix->n_dev = 0; ix->bf_rows = 0; ix->f16_rows = 0;
+    ix->n_dev = 0; ix->bf_rows = 0; ix->f16_rows = 0; ix->sq8_rows = 0; ix->sq8_trained = false;
     return ZVDB_OK;
 }
 
@@ -1449,16 +1583,36 @@ int zvdb_set_descent(zvdb_index *ix, int on) {
 
 int zvdb_set_storage(zvdb_index *ix, int storage) {
     if (!ix) return fail(ZVDB_ERR_INVALID, "null index");
-    if (storage != ZVDB_STORAGE_F32 && storage != ZVDB_STORAGE_F16) return fail(ZVDB_ERR_INVALID, "set_storage: storage must be ZVDB_STORAGE_F32 or ZVDB_STORAGE_F16");
+    if (storage != ZVDB_STORAGE_F32 && storage != ZVDB_STORAGE_F16 && storage != ZVDB_STORAGE_SQ8)
+        return fail(ZVDB_ERR_INVALID, "set_storage: storage must be ZVDB_STORAGE_F32, ZVDB_STORAGE_F16 or ZVDB_STORAGE_SQ8");
     std::lock_guard<std::mutex> lk(ix->mu);
     if (storage == ZVDB_STORAGE_F16 && ix->g.dtype != 0)
         return fail(ZVDB_ERR_UNSUPPORTED, "set_storage: f16 storage is built for f32 indexes only (this one holds f64 / i32 rows)");
+    if (storage == ZVDB_STORAGE_SQ8 && ix->g.dtype != 0)
+        return fail(ZVDB_ERR_UNSUPPORTED, "set_storage: sq8 storage is built for f32 indexes only (this one holds f64 / i32 rows)");
     ix->storage = storage;
-    if (storage == ZVDB_STORAGE_F32 && ix->d_arena16) {      // searches enqueued on caller streams may still read it
+    // The copy the new setting does not read is freed (F32 frees both); setting SQ8, even again, trains a new codebook at
+    // the next search. Searches enqueued on caller streams may still read what changes here.
+    const bool drop16 = storage != ZVDB_STORAGE_F16 && ix->d_arena16;
+    const bool drop8 = ix->d_sq8 && (storage != ZVDB_STORAGE_SQ8 || ix->sq8_trained);
+    if (drop16 || drop8) {
         ZV_CUDA(cudaSetDevice(ix->device));
         ZV_CUDA(cudaDeviceSynchronize());
-        cudaFree(ix->d_arena16); ix->d_arena16 = nullptr; ix->f16_rows = 0;
     }
+    if (drop16) { cudaFree(ix->d_arena16); ix->d_arena16 = nullptr; ix->f16_rows = 0; }
+    if (storage != ZVDB_STORAGE_SQ8) { cudaFree(ix->d_sq8); ix->d_sq8 = nullptr; }
+    ix->sq8_rows = 0; ix->sq8_trained = false;
+    ix->sq8_scale.clear(); ix->sq8_offset.clear();
+    return ZVDB_OK;
+}
+
+int zvdb_storage_codebook(const zvdb_index *ix, float *scale, float *offset, uint32_t dim) {
+    if (!ix || !scale || !offset) return fail(ZVDB_ERR_INVALID, "storage_codebook: null argument");
+    ZV_LOCKED(ix);
+    if (!ix->sq8_trained || ix->sq8_scale.empty()) return fail(ZVDB_ERR_INVALID, "storage_codebook: no SQ8 codebook is trained (it is at the first search under ZVDB_STORAGE_SQ8)");
+    if (dim != ix->g.dim) return fail(ZVDB_ERR_DIM_MISMATCH, "storage_codebook: dim differs from the index's");
+    std::memcpy(scale, ix->sq8_scale.data(), dim * sizeof(float));
+    std::memcpy(offset, ix->sq8_offset.data(), dim * sizeof(float));
     return ZVDB_OK;
 }
 
@@ -1595,7 +1749,7 @@ int zvdb_build_from_candidates(zvdb_index *ix, const float *points, uint64_t n, 
         // becomes empty (the error string of the failing step is kept).
         const std::string why = g_last_error;
         g.reset_nodes();
-        ix->n_dev = 0; ix->bf_rows = 0; ix->f16_rows = 0;
+        ix->n_dev = 0; ix->bf_rows = 0; ix->f16_rows = 0; ix->sq8_rows = 0; ix->sq8_trained = false;
         return fail(rc, why);
     }
     // the table was produced on the device and copied back: both sides are current
@@ -1996,6 +2150,7 @@ int zvdb_search_batch_exchange(zvdb_index *ix, zvdb_exchange *ex, const float *d
     if (block * ex->world > ex->cap_bytes) return fail(ZVDB_ERR_INVALID, "exchange: nq * k exceeds the capacity the exchange was created with");
     std::lock_guard<std::mutex> lk(ix->mu);
     if (ix->storage == ZVDB_STORAGE_F16) return fail(ZVDB_ERR_UNSUPPORTED, "exchange: f16 storage is not built into the sharded forms; set ZVDB_STORAGE_F32");
+    if (ix->storage == ZVDB_STORAGE_SQ8) return fail(ZVDB_ERR_UNSUPPORTED, "exchange: sq8 storage is not built into the sharded forms; set ZVDB_STORAGE_F32");
     ZV_CUDA(cudaSetDevice(ix->device));
     cudaStream_t s = static_cast<cudaStream_t>(stream);
     const uint32_t epoch = ++ex->epoch;
@@ -2058,6 +2213,7 @@ int zvdb_search_batch_exchange_host(zvdb_index *ix, zvdb_exchange *ex, const flo
     if (block * ex->world > ex->cap_bytes) return fail(ZVDB_ERR_INVALID, "exchange: nq * k exceeds the capacity the exchange was created with");
     std::lock_guard<std::mutex> lk(ix->mu);
     if (ix->storage == ZVDB_STORAGE_F16) return fail(ZVDB_ERR_UNSUPPORTED, "exchange: f16 storage is not built into the sharded forms; set ZVDB_STORAGE_F32");
+    if (ix->storage == ZVDB_STORAGE_SQ8) return fail(ZVDB_ERR_UNSUPPORTED, "exchange: sq8 storage is not built into the sharded forms; set ZVDB_STORAGE_F32");
     ZV_CUDA(cudaSetDevice(ix->device));
     const bool empty = ix->g.n == 0 || !ix->g.has_entry;
     if (!empty && dim != ix->g.dim) return fail(ZVDB_ERR_DIM_MISMATCH, "Mismatched dimensions in distance calculation");

@@ -120,6 +120,9 @@ struct SearchParams {
     // F16 row format (zvdb_set_storage): the rows the traversal gathers, [n][row_chunks] 8-byte chunks of four halves (the
     // fp32 arena rounded to nearest even); `arena` stays the fp32 rows the popped set is re-scored on.
     const uint2 *arena16;
+    // SQ8 row format: [n][row_chunks] 4-byte words of four 8-bit codes (element 4i + b in byte b), preceded in the same
+    // allocation by the per-dimension codebook (sq8_codebook).
+    const uint32_t *arena8;
 };
 
 enum : int { kMetricL2 = 0, kMetricCos = 1, kMetricDot = 2 };
@@ -129,8 +132,13 @@ constexpr uint32_t kPoolCap = 64;   // pending pool slots
 // (float4) or 8 bytes of fp16 (uint2, two __half2). fp16 -> fp32 is exact, so the FFMA2 chain and the butterfly see the
 // same operands as an fp32 row holding the rounded values: a search over f16 rows is bit for bit the oracle's search on
 // the f16-rounded rows.
-enum : int { kRowF32 = 0, kRowF16 = 1 };
-template <int ROWF> using RowChunk = std::conditional_t<ROWF == kRowF16, uint2, float4>;
+// SQ8 (one 4-byte word of four codes) decodes each element as fmaf(code, scale, offset) -- exact conversion, one
+// rounding -- so the same holds for the decoded rows.
+enum : int { kRowF32 = 0, kRowF16 = 1, kRowSQ8 = 2 };
+// SQ8 is built for rows of up to 768 floats (CPL <= 6): at 1024 the one-warp kernel does not fit its registers without spills.
+constexpr int kSq8MaxCpl = 6;
+template <int ROWF> using RowChunk =
+    std::conditional_t<ROWF == kRowF16, uint2, std::conditional_t<ROWF == kRowSQ8, uint32_t, float4>>;
 __device__ __forceinline__ float4 chunk_f32(const float4 v) { return v; }
 __device__ __forceinline__ float4 chunk_f32(const uint2 w) {
     const float2 a = __half22float2(*reinterpret_cast<const __half2 *>(&w.x));
@@ -138,11 +146,15 @@ __device__ __forceinline__ float4 chunk_f32(const uint2 w) {
     return make_float4(a.x, a.y, b.x, b.y);
 }
 template <int ROWF> __device__ __forceinline__ RowChunk<ROWF> zero_chunk() {
-    if constexpr (ROWF == kRowF16) return make_uint2(0u, 0u); else return make_float4(0.f, 0.f, 0.f, 0.f);
+    if constexpr (ROWF == kRowF16) return make_uint2(0u, 0u);
+    else if constexpr (ROWF == kRowSQ8) return 0u;
+    else return make_float4(0.f, 0.f, 0.f, 0.f);
 }
-// The rows a search gathers: the fp32 arena, or its f16 copy.
+// The rows a search gathers: the fp32 arena, its f16 copy or its SQ8 codes.
 template <int ROWF> __device__ __forceinline__ const RowChunk<ROWF> *search_rows(const SearchParams &p) {
-    if constexpr (ROWF == kRowF16) return p.arena16; else return p.arena;
+    if constexpr (ROWF == kRowF16) return p.arena16;
+    else if constexpr (ROWF == kRowSQ8) return p.arena8;
+    else return p.arena;
 }
 
 // Rows a warp fetches before it starts reducing (loads in flight per lane = U * CPL float4).
@@ -154,7 +166,8 @@ template <int ROWF> __device__ __forceinline__ const RowChunk<ROWF> *search_rows
 #endif
 template <int CPL, bool WIDE, int ROWF = kRowF32> struct Unroll {
     static constexpr int narrow = CPL <= 1 ? 8 : (CPL <= 2 ? 4 : 2);
-    static constexpr int value = (WIDE ? (CPL <= 4 ? narrow * 2 : narrow) : narrow) * (ROWF == kRowF16 ? ZVDB_F16_UNROLL : 1);
+    static constexpr int value = ROWF == kRowSQ8 && CPL == 6 ? 1     // (at U = 2 the codebook loads push 768-d SQ8 into spills)
+                               : (WIDE ? (CPL <= 4 ? narrow * 2 : narrow) : narrow) * (ROWF == kRowF16 ? ZVDB_F16_UNROLL : 1);
 };
 
 // Packed f32x2 arithmetic (Blackwell FFMA2: PTX fma.rn.f32x2, sm_100+). A 16-byte chunk (x,y,z,w)
@@ -194,6 +207,37 @@ __device__ __forceinline__ uint64_t accumulate_chunk(uint64_t acc, const Chunk2 
 __device__ __forceinline__ float lane_partial(uint64_t acc) {
     float a0, a1; unpack2(acc, a0, a1); return __fadd_rn(a0, a1);
 }
+
+// SQ8 decoder. The codebook sits in front of the codes in their allocation: [2][row_chunks] float4, the scales, then the
+// offsets (zero for padding elements). A row walk over codes finds it from the pointer and pitch it already has, so the
+// fp32 and f16 walks take no extra argument and compile as they did without SQ8 (an empty decoder object passed along
+// was enough to reorder their machine code). The decoder holds the codebook entries of N chunks, packed in pairs like
+// the query; walks load it chunk by chunk next to the row loads (1 KB per 128-d codebook: L1-resident) and drop it
+// after use, since 8 registers per chunk kept for a whole query spill the one-warp kernel.
+__device__ __forceinline__ const float4 *sq8_codebook(const uint32_t *codes, uint32_t row_chunks) {
+    return reinterpret_cast<const float4 *>(codes) - 2u * row_chunks;
+}
+template <int N> struct Sq8Decoder {
+    Chunk2 s[N], o[N];
+    // slot i <- the codebook of chunk `chunk` (elements 4 chunk .. 4 chunk + 3); zero beyond the row
+    __device__ __forceinline__ void load(const uint32_t *codes, uint32_t row_chunks, int i, uint32_t chunk) {
+        const float4 *cb = sq8_codebook(codes, row_chunks);
+        float4 a = make_float4(0.f, 0.f, 0.f, 0.f), b = a;
+        if (chunk < row_chunks) { a = __ldg(cb + chunk); b = __ldg(cb + row_chunks + chunk); }
+        s[i].xy = pack2(a.x, a.y); s[i].zw = pack2(a.z, a.w);
+        o[i].xy = pack2(b.x, b.y); o[i].zw = pack2(b.z, b.w);
+    }
+    // x = fmaf(code, scale, offset) per element: (float)code is exact, fma.rn.f32x2 rounds once per element. (Not folded
+    // into the difference q - x: fmaf(code, scale, offset - q) is another arithmetic.)
+    __device__ __forceinline__ float4 operator()(uint32_t w, int i) const {
+        const uint64_t cxy = pack2(__uint2float_rn(w & 0xFFu), __uint2float_rn((w >> 8) & 0xFFu));
+        const uint64_t czw = pack2(__uint2float_rn((w >> 16) & 0xFFu), __uint2float_rn(w >> 24));
+        float4 x;
+        unpack2(ffma2(cxy, s[i].xy, o[i].xy), x.x, x.y);
+        unpack2(ffma2(czw, s[i].zw, o[i].zw), x.z, x.w);
+        return x;
+    }
+};
 
 // One query -> registers, chunked like an arena row (lane l owns 16-byte chunks l, l+32, ...), packed in pairs
 // for the f32x2 pipe, zero padded. One 16-byte load per chunk when the row allows it: the query may live in
@@ -255,7 +299,8 @@ __device__ __forceinline__ void transposed_reduce(float (&d)[R], uint32_t lane, 
 // ids[u] for u >= nrows must still be valid row ids (callers pad with a hot row): a full-width
 // batch runs without per-row predicates. Returns, in every lane l, the distance of row l / (32/U)
 // (meaningless for rows >= nrows).
-// ROWF = kRowF16: the same with 8-byte chunks (ld.global.nc.v2), converted exactly before the FMAs.
+// ROWF = kRowF16: the same with 8-byte chunks (ld.global.nc.v2), converted exactly before the FMAs; kRowSQ8: 4-byte
+// words of codes (one 128-byte line per row and 128 elements), decoded before the FMAs.
 template <int CPL, int METRIC, int U, int ROWF = kRowF32>
 __device__ __forceinline__ float rows_distance(const RowChunk<ROWF> *__restrict__ arena, uint32_t row_chunks,
                                                const uint32_t (&ids)[U], const Chunk2 (&qv)[CPL], uint32_t lane) {
@@ -282,12 +327,28 @@ __device__ __forceinline__ float rows_distance(const RowChunk<ROWF> *__restrict_
         }
     }
     float acc[U];
+    if constexpr (ROWF == kRowSQ8) {
+        // chunk by chunk (the codebook of one chunk live at a time); each row still sums its chunks in order 0, 1, ...
+        uint64_t a2[U];
+#pragma unroll
+        for (int u = 0; u < U; ++u) a2[u] = 0;
+#pragma unroll
+        for (int c = 0; c < CPL; ++c) {
+            Sq8Decoder<1> dec;
+            dec.load(arena, row_chunks, 0, lane + 32u * c);
+#pragma unroll
+            for (int u = 0; u < U; ++u) a2[u] = accumulate_chunk<METRIC>(a2[u], qv[c], dec(v[u][c], 0));
+        }
+#pragma unroll
+        for (int u = 0; u < U; ++u) acc[u] = lane_partial(a2[u]);
+    } else {
 #pragma unroll
     for (int u = 0; u < U; ++u) {
         uint64_t a2 = 0;                                 // (+0.0f, +0.0f)
 #pragma unroll
         for (int c = 0; c < CPL; ++c) a2 = accumulate_chunk<METRIC>(a2, qv[c], chunk_f32(v[u][c]));
         acc[u] = lane_partial(a2);
+    }
     }
     transposed_reduce<U>(acc, lane, 16);
     return finish_distance<METRIC>(acc[0]);
@@ -320,7 +381,13 @@ __device__ __forceinline__ float row_distance(const RowChunk<ROWF> *__restrict__
         const uint32_t chunk = lane + 32u * c;
         RowChunk<ROWF> v = zero_chunk<ROWF>();
         if (chunk < row_chunks) v = __ldg(arena + static_cast<size_t>(id) * row_chunks + chunk);
-        a2 = accumulate_chunk<METRIC>(a2, qv[c], chunk_f32(v));
+        if constexpr (ROWF == kRowSQ8) {
+            Sq8Decoder<1> dec;
+            dec.load(arena, row_chunks, 0, chunk);
+            a2 = accumulate_chunk<METRIC>(a2, qv[c], dec(v, 0));
+        } else {
+            a2 = accumulate_chunk<METRIC>(a2, qv[c], chunk_f32(v));
+        }
     }
     float acc = lane_partial(a2);
 #pragma unroll
@@ -580,7 +647,7 @@ __device__ __noinline__ void merge_one_query(const SearchParams &p, uint32_t q, 
 // EXCH = the sharded forms of the step (peer stores, records, flags, the merge tail). The plain search is a separate
 // instantiation with none of that code in it: in round 2 every piece of exchange code added behind a run-time test still
 // cost the global-visited modes 8-10 % (the 64-register pop loop is allocated together with whatever surrounds it).
-// ROWF = the format of the rows the traversal gathers. kRowF16 (plain search only, EXCH = false) adds the exact re-rank
+// ROWF = the format of the rows the traversal gathers. kRowF16 and kRowSQ8 (plain search only, EXCH = false) add the exact re-rank
 // epilogue: the popped set is re-scored on the fp32 arena and ordered by (exact distance, id). It exists only in those
 // instantiations, for the same reason as EXCH.
 template <int CPL, int METRIC, int VIS, bool EXCH, int ROWF = kRowF32>
@@ -848,7 +915,7 @@ search_layer0_kernel(const __grid_constant__ SearchParams p) {
     __syncwarp();
     uint64_t *sorted = cand;                                     // the window is dead now
     const uint32_t p2 = next_pow2(np);
-    if constexpr (ROWF == kRowF16) {
+    if constexpr (ROWF != kRowF32) {
         // Re-rank: every popped id re-scored with the fp32 distance on the fp32 arena (the K1 / K4 distance of the pair),
         // keys (exact distance, id) sorted directly; sorted[] then holds keys, not pop indices.
         constexpr int U32 = Unroll<CPL, false>::value;
@@ -906,7 +973,7 @@ search_layer0_kernel(const __grid_constant__ SearchParams p) {
         const size_t o = static_cast<size_t>(q) * p.k + r;
         uint64_t oid = ~0ull; float od = 0.0f;
         if (r < nres) {
-            const uint64_t key = (x_world || ROWF == kRowF16) ? sorted[r] : *res_at(static_cast<uint32_t>(sorted[r]));
+            const uint64_t key = (x_world || ROWF != kRowF32) ? sorted[r] : *res_at(static_cast<uint32_t>(sorted[r]));
             oid = static_cast<uint64_t>(key_id(key)) * p.id_stride + p.id_base;
             od = key_dist(key);
         }

@@ -56,7 +56,8 @@ __host__ __device__ inline uint64_t team_smem_bytes(uint64_t cand_cap, uint64_t 
     return (b + 15) & ~15ull;
 }
 
-// Lane j of a half-warp loads chunks j and j + 16 of every 32: 16-byte chunks of an fp32 row, 8-byte chunks of an f16 row.
+// Lane j of a half-warp loads chunks j and j + 16 of every 32: 16-byte chunks of an fp32 row, 8-byte chunks of an f16 row,
+// 4-byte words of SQ8 codes.
 template <int CPL, int METRIC, int ROWF = kRowF32>
 __device__ __forceinline__ void half_row_load(RowChunk<ROWF> (&vlo)[CPL], RowChunk<ROWF> (&vhi)[CPL], const RowChunk<ROWF> *__restrict__ arena,
                                               uint32_t row_chunks, uint32_t id, uint32_t j) {
@@ -94,6 +95,25 @@ __device__ __forceinline__ float half_row_reduce(const T (&vlo)[CPL], const T (&
     for (int off = 8; off >= 1; off >>= 1) s = __fadd_rn(s, __shfl_xor_sync(kFullMask, s, off));
     return finish_distance<METRIC>(s);
 }
+// The same over SQ8 codes: lane j's codebook entries (chunks j + 32 c and j + 32 c + 16) are loaded here, while the codes
+// loaded by half_row_load may still be in flight, and decoded before the FMAs.
+template <int CPL, int METRIC>
+__device__ __forceinline__ float half_row_reduce_sq8(const uint32_t (&vlo)[CPL], const uint32_t (&vhi)[CPL], const Chunk2 (&qlo)[CPL],
+                                                     const Chunk2 (&qhi)[CPL], const uint32_t *codes, uint32_t row_chunks, uint32_t j) {
+    uint64_t alo = 0, ahi = 0;                               // the sums of half_row_reduce, on the decoded chunks
+#pragma unroll
+    for (int c = 0; c < CPL; ++c) {
+        Sq8Decoder<2> dec;
+        dec.load(codes, row_chunks, 0, j + 32u * c);
+        dec.load(codes, row_chunks, 1, j + 32u * c + 16u);
+        alo = accumulate_chunk<METRIC>(alo, qlo[c], dec(vlo[c], 0));
+        ahi = accumulate_chunk<METRIC>(ahi, qhi[c], dec(vhi[c], 1));
+    }
+    float s = __fadd_rn(lane_partial(alo), lane_partial(ahi));
+#pragma unroll
+    for (int off = 8; off >= 1; off >>= 1) s = __fadd_rn(s, __shfl_xor_sync(kFullMask, s, off));
+    return finish_distance<METRIC>(s);
+}
 
 // Minimum of one 64-bit key per lane over the warp, by two 32-bit REDUX steps (distance word, then id among its holders).
 __device__ __forceinline__ uint64_t warp_min_key(uint64_t key) {
@@ -104,7 +124,7 @@ __device__ __forceinline__ uint64_t warp_min_key(uint64_t key) {
 }
 
 // MC = m when it is known at compile time (16: BASELINE's M), 0 = read it from the parameters. ROWF = the format of the
-// rows the traversal gathers; kRowF16 adds the exact re-rank of the popped set (as in search_layer0_kernel).
+// rows the traversal gathers; kRowF16 and kRowSQ8 add the exact re-rank of the popped set (as in search_layer0_kernel).
 template <int CPL, int METRIC, bool ADJC, int MC, int T, int ROWF>
 __device__ __forceinline__ void search_team_body(const SearchParams &p) {
     constexpr uint32_t TT = T, TW = T / 32, TR = T / 16;            // threads, warps, rows (half-warps) per pass
@@ -150,7 +170,8 @@ __device__ __forceinline__ void search_team_body(const SearchParams &p) {
         if (p.seeds == nullptr) {
             RowChunk<ROWF> vlo[CPL], vhi[CPL];
             half_row_load<CPL, METRIC, ROWF>(vlo, vhi, arena, p.row_chunks, entry, j);
-            d0 = half_row_reduce<CPL, METRIC>(vlo, vhi, qlo, qhi);
+            if constexpr (ROWF == kRowSQ8) d0 = half_row_reduce_sq8<CPL, METRIC>(vlo, vhi, qlo, qhi, arena, p.row_chunks, j);
+            else d0 = half_row_reduce<CPL, METRIC>(vlo, vhi, qlo, qhi);
         } else {                                                    // K2 ran first: start where the descent landed
             const uint4 sd = __ldg(p.seeds + q);
             entry = sd.x; d0 = __uint_as_float(sd.y);
@@ -202,7 +223,9 @@ __device__ __forceinline__ void search_team_body(const SearchParams &p) {
                 if (lane == owner) { wkey[par * kTeamWarps + warp] = wk; wslot[par * kTeamWarps + warp] = best_i; }
             }
             if (!active) continue;
-            const float d = half_row_reduce<CPL, METRIC>(vlo, vhi, qlo, qhi);                 // :219
+            float d;                                                                          // :219
+            if constexpr (ROWF == kRowSQ8) d = half_row_reduce_sq8<CPL, METRIC>(vlo, vhi, qlo, qhi, arena, p.row_chunks, j);
+            else d = half_row_reduce<CPL, METRIC>(vlo, vhi, qlo, qhi);
             if (fresh) cand[slot] = pack_key(d, nb);                                          // :220 (lane 0 of the half)
             if (ADJC) asm volatile("cp.async.wait_all;" ::: "memory");
         }
@@ -228,7 +251,7 @@ __device__ __forceinline__ void search_team_body(const SearchParams &p) {
     __syncthreads();
     uint64_t *sorted = cand;                                        // the candidates are dead now
     const uint32_t p2 = next_pow2(np);
-    if constexpr (ROWF == kRowF16) {
+    if constexpr (ROWF != kRowF32) {
         // Re-rank: half-warp h re-scores popped entries h, h + T / 16, ... with the fp32 distance on the fp32 arena; sorted[]
         // then holds (exact distance, id) keys, not pop indices.
         for (uint32_t i0 = 0; i0 < np; i0 += TR) {                  // (uniform bound: the reduction shuffles take whole warps)
@@ -250,7 +273,7 @@ __device__ __forceinline__ void search_team_body(const SearchParams &p) {
         const size_t o = static_cast<size_t>(q) * p.k + r;
         uint64_t oid = ~0ull; float od = 0.0f;
         if (r < nres) {
-            const uint64_t key = ROWF == kRowF16 ? sorted[r] : res[static_cast<uint32_t>(sorted[r])];
+            const uint64_t key = ROWF != kRowF32 ? sorted[r] : res[static_cast<uint32_t>(sorted[r])];
             oid = static_cast<uint64_t>(key_id(key)) * p.id_stride + p.id_base;
             od = key_dist(key);
         }
@@ -282,6 +305,14 @@ template <int CPL, int METRIC, bool ADJC, int MC, int T>
 __global__ void __launch_bounds__(T, (T == 256 ? (CPL <= 2 ? 2 : 1) : (CPL <= 4 ? 4 : 2)))
 search_team_f16_kernel(const __grid_constant__ SearchParams p) {
     search_team_body<CPL, METRIC, ADJC, MC, T, kRowF16>(p);
+}
+
+// The same over SQ8 codes (zvdb_set_storage), likewise a kernel of its own name. Half teams at 512-d are bounded like the
+// 768-d ones: at the fp32 bound (128 registers) the dot form keeps 8 bytes of stack.
+template <int CPL, int METRIC, bool ADJC, int MC, int T>
+__global__ void __launch_bounds__(T, (T == 256 ? (CPL <= 2 ? 2 : 1) : (CPL <= 2 ? 4 : 2)))
+search_team_sq8_kernel(const __grid_constant__ SearchParams p) {
+    search_team_body<CPL, METRIC, ADJC, MC, T, kRowSQ8>(p);
 }
 
 }  // namespace zvdb

@@ -222,18 +222,29 @@ class HNSW:
         L.check(L.lib().zvdb_set_descent(self._h, 1 if on else 0))
 
     # -- vector storage of the graph search (zvdb_set_storage) --------------------------------------
-    _STORAGE = {"f32": L.STORAGE_F32, "f16": L.STORAGE_F16}
+    _STORAGE = {"f32": L.STORAGE_F32, "f16": L.STORAGE_F16, "sq8": L.STORAGE_SQ8}
 
     def set_storage(self, storage: str = "f32") -> None:
-        """"f16": the graph search gathers an fp16 copy of the rows and re-ranks the popped set exactly in fp32
-        (distances returned are the fp32 ones); "f32" (default): it gathers the fp32 rows. Takes effect at the next search."""
+        """"f16": the graph search gathers an fp16 copy of the rows; "sq8": 8-bit codes of the rows with a per-dimension
+        (scale, offset) codebook, trained at the next search (setting "sq8" again retrains it). Both re-rank the popped set
+        exactly in fp32 (distances returned are the fp32 ones). "f32" (default): the search gathers the fp32 rows. Takes
+        effect at the next search."""
         if storage not in self._STORAGE:
-            raise ValueError('storage must be "f32" or "f16"')
+            raise ValueError('storage must be "f32", "f16" or "sq8"')
         L.check(L.lib().zvdb_set_storage(self._h, self._STORAGE[storage]))
 
     @property
     def storage(self) -> str:
-        return "f16" if int(L.lib().zvdb_storage(self._h)) == L.STORAGE_F16 else "f32"
+        s = int(L.lib().zvdb_storage(self._h))
+        return {L.STORAGE_F16: "f16", L.STORAGE_SQ8: "sq8"}.get(s, "f32")
+
+    def codebook(self):
+        """(scale[dim], offset[dim]) float32 of the SQ8 codebook in use: code c of dimension d decodes to
+        fmaf(c, scale[d], offset[d]). Raises ZvdbError (ERR_INVALID) when none is trained."""
+        scale, offset = np.zeros(self.dim, np.float32), np.zeros(self.dim, np.float32)
+        L.check(L.lib().zvdb_storage_codebook(self._h, scale.ctypes.data_as(C.POINTER(C.c_float)),
+                                              offset.ctypes.data_as(C.POINTER(C.c_float)), self.dim))
+        return scale, offset
 
     @property
     def descent_start(self) -> Optional[int]:
