@@ -49,77 +49,9 @@ __global__ void scatter_adj_rows_kernel(uint32_t *__restrict__ adj, const uint32
     }
 }
 
-// F16 storage: rows [r0, r1) of the fp32 arena rounded to nearest even into the f16 copy (pitch row_floats in both). The
-// one range check of the f16 path: the first row with a coordinate that rounds to +-inf (|x| >= 65520) goes to *bad_row
-// (atomicMin; ~0 = none), and the search that triggered the conversion refuses to run.
-__global__ void arena_to_f16_kernel(uint2 *__restrict__ dst, const float4 *__restrict__ src, uint64_t r0, uint64_t r1,
-                                    uint32_t row_chunks, uint32_t *__restrict__ bad_row) {
-    const uint64_t begin = r0 * row_chunks, end = r1 * row_chunks;
-    for (uint64_t i = begin + blockIdx.x * static_cast<uint64_t>(blockDim.x) + threadIdx.x; i < end;
-         i += static_cast<uint64_t>(gridDim.x) * blockDim.x) {
-        const float4 v = src[i];
-        const __half2 a = __floats2half2_rn(v.x, v.y), b = __floats2half2_rn(v.z, v.w);
-        if (__hisinf(__low2half(a)) | __hisinf(__high2half(a)) | __hisinf(__low2half(b)) | __hisinf(__high2half(b)))
-            atomicMin(bad_row, static_cast<uint32_t>(i / row_chunks));
-        dst[i] = make_uint2(*reinterpret_cast<const uint32_t *>(&a), *reinterpret_cast<const uint32_t *>(&b));
-    }
-}
-
-// SQ8 storage, training: per-dimension min and max over rows [0, n) of the fp32 arena, as order-preserving words
-// (float_to_ordered, -0 < +0), and the first row holding a non-finite coordinate (*bad_row, atomicMin; ~0 = none). Min
-// and max do not depend on the order the rows are seen in, so the codebook is deterministic. One thread per element of
-// a row (blockDim.x = row_floats), each block a stripe of rows.
-__global__ void sq8_minmax_kernel(uint32_t *__restrict__ mn, uint32_t *__restrict__ mx, const float *__restrict__ src, uint64_t n,
-                                  uint32_t row_floats, uint32_t dim, uint32_t *__restrict__ bad_row) {
-    const uint32_t d = threadIdx.x;
-    if (d >= dim) return;
-    uint32_t lo = ~0u, hi = 0u, bad = ~0u;
-    for (uint64_t r = blockIdx.x; r < n; r += gridDim.x) {
-        const float x = src[r * row_floats + d];
-        if (!isfinite(x)) bad = min(bad, static_cast<uint32_t>(r));
-        const uint32_t o = float_to_ordered(x);
-        lo = min(lo, o); hi = max(hi, o);
-    }
-    atomicMin(mn + d, lo); atomicMax(mx + d, hi);
-    if (bad != ~0u) atomicMin(bad_row, bad);
-}
-
-// The SQ8 code of one element: clamp(rint((x - o) / s), 0, 255), 0 when s == 0 (a constant dimension, or padding).
-__device__ __forceinline__ uint32_t sq8_code(float x, float s, float o) {
-    if (s == 0.f) return 0u;
-    return static_cast<uint32_t>(fminf(fmaxf(rintf(__fdiv_rn(__fsub_rn(x, o), s)), 0.f), 255.f));
-}
-// SQ8 storage: rows [r0, r1) of the fp32 arena encoded with the codebook cb ([2][row_chunks]: scales, offsets) into the
-// code copy (one 4-byte word per 4-float chunk). The first row with a non-finite coordinate goes to *bad_row.
-__global__ void arena_to_sq8_kernel(uint32_t *__restrict__ dst, const float4 *__restrict__ src, const float4 *__restrict__ cb,
-                                    uint64_t r0, uint64_t r1, uint32_t row_chunks, uint32_t *__restrict__ bad_row) {
-    const uint64_t begin = r0 * row_chunks, end = r1 * row_chunks;
-    for (uint64_t i = begin + blockIdx.x * static_cast<uint64_t>(blockDim.x) + threadIdx.x; i < end;
-         i += static_cast<uint64_t>(gridDim.x) * blockDim.x) {
-        const uint32_t c = static_cast<uint32_t>(i % row_chunks);
-        const float4 v = src[i], sc = cb[c], of = cb[row_chunks + c];
-        if (!(isfinite(v.x) && isfinite(v.y) && isfinite(v.z) && isfinite(v.w))) atomicMin(bad_row, static_cast<uint32_t>(i / row_chunks));
-        dst[i] = sq8_code(v.x, sc.x, of.x) | (sq8_code(v.y, sc.y, of.y) << 8) | (sq8_code(v.z, sc.z, of.z) << 16) |
-                 (sq8_code(v.w, sc.w, of.w) << 24);
-    }
-}
-
-template <typename T>
-struct DevBuf {
-    T *p = nullptr;
-    size_t cap = 0;
-    cudaError_t reserve(size_t count) {
-        if (count <= cap) return cudaSuccess;
-        if (p) cudaFree(p);
-        p = nullptr; cap = 0;
-        cudaError_t e = cudaMalloc(&p, count * sizeof(T));
-        if (e == cudaSuccess) cap = count;
-        return e;
-    }
-    void free_() { if (p) cudaFree(p); p = nullptr; cap = 0; }
-};
-
 }  // namespace zvdb
+
+#include "row_copy.cuh"
 
 using namespace zvdb;
 
@@ -145,16 +77,7 @@ struct zvdb_index {
     uint64_t cap_rows = 0, n_dev = 0;
     uint32_t cap_row_floats = 0, cap_m = 0;   // row layout d_arena / d_adj were sized for (a load may change dim)
     int storage = ZVDB_STORAGE_F32; // rows the graph search gathers (zvdb_set_storage)
-    uint2 *d_arena16 = nullptr;     // ZVDB_STORAGE_F16: [cap_rows][row_floats] __half copy of d_arena, rows [0, f16_rows) current
-    uint64_t f16_rows = 0;
-    DevBuf<uint32_t> f16_bad;       // first row the conversion found out of the f16 range, or (SQ8) non-finite (~0 = none)
-    // ZVDB_STORAGE_SQ8: one allocation, the codebook [2][row_floats] fp32 (scales, then offsets) followed by the 8-bit codes
-    // of d_arena [cap_rows][row_floats], rows [0, sq8_rows) current (the kernels find the codebook in front of the codes)
-    unsigned char *d_sq8 = nullptr;
-    uint64_t sq8_rows = 0;
-    bool sq8_trained = false;       // the codebook belongs to these contents (else the next SQ8 search trains it)
-    std::vector<float> sq8_scale, sq8_offset;   // the codebook, [row_floats] each (zero for the padding elements)
-    DevBuf<uint32_t> sq8_minmax;    // training scratch, [2][row_floats] ordered min / max
+    RowCopy row_copy;               // F16 / SQ8: the compact copy of d_arena in that format (row_copy.cuh)
     DevBuf<float> q_buf, dist_buf;
     DevBuf<uint64_t> ids_buf;
     DevBuf<uint32_t> cnt_buf, pops_buf, evals_buf, scat_rows, scat_ids, bitmap_buf, vlog_buf;
@@ -187,6 +110,12 @@ struct zvdb_index {
 
 namespace zvdb {
 
+// The handle's contents were replaced: nothing on the device covers them any more (the next search uploads them).
+static void forget_device_rows(zvdb_index *ix) {
+    ix->n_dev = 0; ix->bf_rows = 0;
+    ix->row_copy.new_contents();
+}
+
 // Device arena + layer-0 table for `rows` rows of the CURRENT row layout. Capacity is (rows, row_floats, m): a handle
 // whose contents were replaced by rows of another dim (zvdb_load, zvdb_load_graph, zvdb_build_from_candidates) gets
 // fresh buffers instead of reusing ones sized for the old pitch.
@@ -197,18 +126,12 @@ static int ensure_capacity(zvdb_index *ix, uint64_t rows) {
     if (!same_layout) {                                   // nothing on the device is reusable
         ZV_CUDA(cudaDeviceSynchronize());
         cudaFree(ix->d_arena); cudaFree(ix->d_adj);
-        ix->d_arena = nullptr; ix->d_adj = nullptr; ix->cap_rows = 0; ix->n_dev = 0; ix->bf_rows = 0;
+        ix->d_arena = nullptr; ix->d_adj = nullptr; ix->cap_rows = 0;
         ix->cap_row_floats = g.row_floats; ix->cap_m = g.m;
-        ix->sq8_trained = false;                          // a new row pitch: the next SQ8 search trains a codebook for it
+        forget_device_rows(ix);                           // (a new row pitch: the next SQ8 search trains a codebook for it)
     }
-    if (ix->d_arena16) {                                  // the f16 copy is sized like the arena: the next F16 search rebuilds it
-        ZV_CUDA(cudaDeviceSynchronize());
-        cudaFree(ix->d_arena16); ix->d_arena16 = nullptr; ix->f16_rows = 0;
-    }
-    if (ix->d_sq8) {                                      // so is the code copy: re-encoded (same codebook) by the next SQ8 search
-        ZV_CUDA(cudaDeviceSynchronize());
-        cudaFree(ix->d_sq8); ix->d_sq8 = nullptr; ix->sq8_rows = 0;
-    }
+    int rc = ix->row_copy.drop();
+    if (rc) return rc;
     uint64_t nc = std::max<uint64_t>(rows, std::max<uint64_t>(ix->cap_rows * 2, 1024));
     float *na = nullptr; uint32_t *nj = nullptr;
     ZV_CUDA(cudaMalloc(&na, nc * g.row_floats * sizeof(float)));
@@ -235,8 +158,7 @@ static int sync_device_locked(zvdb_index *ix) {
     if (ix->n_dev) ZV_CUDA(cudaDeviceSynchronize());
     int rc = ensure_capacity(ix, g.n);
     if (rc) return rc;
-    ix->f16_rows = std::min<uint64_t>(ix->f16_rows, g.rows_uploaded);   // rows from rows_uploaded on are (re)written now
-    ix->sq8_rows = std::min<uint64_t>(ix->sq8_rows, g.rows_uploaded);
+    ix->row_copy.clamp(g.rows_uploaded);                 // rows from rows_uploaded on are (re)written now
     for (uint64_t r = g.rows_uploaded; r < g.n;) {
         const uint64_t chunk = r / g.rows_per_chunk;
         const uint64_t end = std::min<uint64_t>(g.n, (chunk + 1) * g.rows_per_chunk);
@@ -272,106 +194,6 @@ static int sync_device_locked(zvdb_index *ix) {
     return ZVDB_OK;
 }
 
-// ZVDB_STORAGE_F16: bring the f16 copy of the arena up to the device rows (after sync_device_locked): allocated at the
-// arena's capacity, rows [f16_rows, n_dev) converted by one kernel. A row out of the f16 range fails the search that got
-// here (and every later one under F16, since f16_rows stays behind it); zvdb_set_storage(F32) recovers the handle.
-static int sync_f16_locked(zvdb_index *ix) {
-    const HostGraph &g = ix->g;
-    if (g.dtype != 0) return fail(ZVDB_ERR_UNSUPPORTED, "f16 storage: the index holds f64 / i32 rows; set ZVDB_STORAGE_F32");
-    if (ix->f16_rows >= ix->n_dev) return ZVDB_OK;
-    if (!ix->d_arena16) {
-        ZV_CUDA(cudaMalloc(&ix->d_arena16, ix->cap_rows * g.row_floats * 2));
-        ix->f16_rows = 0;
-    }
-    ZV_CUDA(ix->f16_bad.reserve(1));
-    ZV_CUDA(cudaMemsetAsync(ix->f16_bad.p, 0xFF, sizeof(uint32_t), ix->stream));
-    const uint32_t row_chunks = g.row_floats / 4;
-    const uint64_t total = (ix->n_dev - ix->f16_rows) * row_chunks;
-    const unsigned blocks = static_cast<unsigned>(std::min<uint64_t>((total + 255) / 256, static_cast<uint64_t>(ix->num_sms) * 8));
-    arena_to_f16_kernel<<<blocks, 256, 0, ix->stream>>>(ix->d_arena16, reinterpret_cast<const float4 *>(ix->d_arena), ix->f16_rows,
-                                                        ix->n_dev, row_chunks, ix->f16_bad.p);
-    ix->launches++;
-    ZV_CUDA(cudaGetLastError());
-    uint32_t bad = ~0u;
-    ZV_CUDA(cudaMemcpyAsync(&bad, ix->f16_bad.p, sizeof bad, cudaMemcpyDeviceToHost, ix->stream));
-    ZV_CUDA(cudaStreamSynchronize(ix->stream));
-    if (bad != ~0u) {
-        char buf[200];
-        snprintf(buf, sizeof buf, "f16 storage: row %u has a coordinate that rounds to +-inf in fp16 (|x| >= 65520); set ZVDB_STORAGE_F32 to search this index", bad);
-        return fail(ZVDB_ERR_UNSUPPORTED, buf);
-    }
-    ix->f16_rows = ix->n_dev;
-    return ZVDB_OK;
-}
-
-// ZVDB_STORAGE_SQ8: bring the code copy up to the device rows (after sync_device_locked). Without a codebook for these
-// contents, one is trained first on rows [0, n_dev): o = min, s = (max - min) / 255 per dimension, each a single IEEE
-// operation on the host; then every row is (re-)encoded. Later rows [sq8_rows, n_dev) are encoded with the codebook
-// they find. A non-finite coordinate fails the search that got here and every later one under SQ8 (nothing moves past
-// the row); zvdb_set_storage(F32) recovers the handle.
-static int sync_sq8_locked(zvdb_index *ix) {
-    const HostGraph &g = ix->g;
-    if (g.dtype != 0) return fail(ZVDB_ERR_UNSUPPORTED, "sq8 storage: the index holds f64 / i32 rows; set ZVDB_STORAGE_F32");
-    if (ix->sq8_trained && ix->sq8_rows >= ix->n_dev) return ZVDB_OK;
-    const uint32_t rf = g.row_floats, row_chunks = rf / 4;
-    uint32_t bad = ~0u;
-    ZV_CUDA(ix->f16_bad.reserve(1));
-    ZV_CUDA(cudaMemsetAsync(ix->f16_bad.p, 0xFF, sizeof(uint32_t), ix->stream));
-    if (!ix->sq8_trained) {
-        ZV_CUDA(cudaDeviceSynchronize());                 // searches enqueued on caller streams may still read the codebook and codes
-        ZV_CUDA(ix->sq8_minmax.reserve(2ull * rf));
-        ZV_CUDA(cudaMemsetAsync(ix->sq8_minmax.p, 0xFF, rf * sizeof(uint32_t), ix->stream));   // min: above every word
-        ZV_CUDA(cudaMemsetAsync(ix->sq8_minmax.p + rf, 0, rf * sizeof(uint32_t), ix->stream)); // max: below every word
-        const unsigned blocks = static_cast<unsigned>(std::min<uint64_t>(ix->n_dev, static_cast<uint64_t>(ix->num_sms) * 8));
-        sq8_minmax_kernel<<<blocks, rf, 0, ix->stream>>>(ix->sq8_minmax.p, ix->sq8_minmax.p + rf, ix->d_arena, ix->n_dev, rf, g.dim,
-                                                         ix->f16_bad.p);
-        ix->launches++;
-        ZV_CUDA(cudaGetLastError());
-        std::vector<uint32_t> mm(2ull * rf);
-        ZV_CUDA(cudaMemcpyAsync(mm.data(), ix->sq8_minmax.p, mm.size() * sizeof(uint32_t), cudaMemcpyDeviceToHost, ix->stream));
-        ZV_CUDA(cudaMemcpyAsync(&bad, ix->f16_bad.p, sizeof bad, cudaMemcpyDeviceToHost, ix->stream));
-        ZV_CUDA(cudaStreamSynchronize(ix->stream));
-        if (bad == ~0u) {
-            ix->sq8_scale.assign(rf, 0.0f); ix->sq8_offset.assign(rf, 0.0f);   // padding elements (d >= dim): (s, o) = (0, 0)
-            for (uint32_t d = 0; d < g.dim; ++d) {
-                const float lo = ordered_to_float(mm[d]), hi = ordered_to_float(mm[rf + d]);
-                ix->sq8_scale[d] = (hi - lo) / 255.0f;    // (built without contraction: two IEEE operations)
-                ix->sq8_offset[d] = lo;
-            }
-            ix->sq8_trained = true; ix->sq8_rows = 0;
-            if (ix->d_sq8) {                              // a copy from an earlier codebook: every row is re-encoded below
-                ZV_CUDA(cudaMemcpyAsync(ix->d_sq8, ix->sq8_scale.data(), rf * sizeof(float), cudaMemcpyHostToDevice, ix->stream));
-                ZV_CUDA(cudaMemcpyAsync(ix->d_sq8 + rf * sizeof(float), ix->sq8_offset.data(), rf * sizeof(float), cudaMemcpyHostToDevice, ix->stream));
-            }
-        }
-    }
-    if (bad == ~0u && !ix->d_sq8) {                       // (first SQ8 search, or after capacity growth: same codebook)
-        ZV_CUDA(cudaMalloc(&ix->d_sq8, 8ull * rf + ix->cap_rows * rf));
-        ZV_CUDA(cudaMemcpyAsync(ix->d_sq8, ix->sq8_scale.data(), rf * sizeof(float), cudaMemcpyHostToDevice, ix->stream));
-        ZV_CUDA(cudaMemcpyAsync(ix->d_sq8 + rf * sizeof(float), ix->sq8_offset.data(), rf * sizeof(float), cudaMemcpyHostToDevice, ix->stream));
-        ix->sq8_rows = 0;
-    }
-    if (bad == ~0u && ix->sq8_rows < ix->n_dev) {
-        const uint64_t total = (ix->n_dev - ix->sq8_rows) * row_chunks;
-        const unsigned blocks = static_cast<unsigned>(std::min<uint64_t>((total + 255) / 256, static_cast<uint64_t>(ix->num_sms) * 8));
-        arena_to_sq8_kernel<<<blocks, 256, 0, ix->stream>>>(reinterpret_cast<uint32_t *>(ix->d_sq8 + 8ull * rf),
-                                                            reinterpret_cast<const float4 *>(ix->d_arena),
-                                                            reinterpret_cast<const float4 *>(ix->d_sq8), ix->sq8_rows, ix->n_dev,
-                                                            row_chunks, ix->f16_bad.p);
-        ix->launches++;
-        ZV_CUDA(cudaGetLastError());
-        ZV_CUDA(cudaMemcpyAsync(&bad, ix->f16_bad.p, sizeof bad, cudaMemcpyDeviceToHost, ix->stream));
-        ZV_CUDA(cudaStreamSynchronize(ix->stream));
-    }
-    if (bad != ~0u) {
-        char buf[200];
-        snprintf(buf, sizeof buf, "sq8 storage: row %u has a non-finite coordinate; set ZVDB_STORAGE_F32 to search this index", bad);
-        return fail(ZVDB_ERR_UNSUPPORTED, buf);
-    }
-    ix->sq8_rows = ix->n_dev;
-    return ZVDB_OK;
-}
-
 // Device copy of layers >= 1 for the descent (K2): levels[n], upper_base[n], upper_adj[n_lists][m].
 // Re-sent whole whenever a list above layer 0 changed (half the nodes have one; the reference links
 // one neighbour per layer and insert, hnsw.zig:106-108).
@@ -397,123 +219,110 @@ static int sync_upper_locked(zvdb_index *ix) {
     return ZVDB_OK;
 }
 
-// ---- K1 launch ------------------------------------------------------------------------------
+// ---- kernel dispatch: K1, K1L, K2, K6, K4 finalize ------------------------------------------------
 
-template <int CPL, int METRIC, int VIS, bool EXCH, int ROWF>
-static cudaError_t launch_search_inst(const SearchParams &p, unsigned grid, size_t smem, cudaStream_t s) {
-    auto kern = search_layer0_kernel<CPL, METRIC, VIS, EXCH, ROWF>;
+// Chunks per lane for rows of `row_floats`, rounded up to a compiled CPL (1, 2, 4, 6, 8; anything wider counts as 8).
+static int cpl_for(uint32_t row_floats) {
+    const uint32_t c = (row_floats / 4 + 31) / 32;
+    return c <= 1 ? 1 : c <= 2 ? 2 : c <= 4 ? 4 : c <= 6 ? 6 : 8;
+}
+
+// One kernel form: the template arguments a launch picks at run time.
+template <int METRIC, int CPL, int ROWF, bool EXCH>
+struct Form { static constexpr int metric = METRIC, cpl = CPL, rowf = ROWF; static constexpr bool exch = EXCH; };
+
+// f(Form{}) if that form is compiled (row_form_built); a form that is not is never instantiated.
+template <typename Fm, typename F>
+static cudaError_t call_form(F &f) {
+    if constexpr (row_form_built(Fm::rowf, Fm::cpl, Fm::exch)) return f(Fm{});
+    else return cudaErrorInvalidValue;
+}
+template <int ROWF, bool EXCH, typename F>
+static cudaError_t dispatch_form(int metric, int cpl, F &f) {
+    auto on_cpl = [&](auto m) -> cudaError_t {
+        constexpr int M = decltype(m)::value;
+        switch (cpl) {
+            case 1: return call_form<Form<M, 1, ROWF, EXCH>>(f);
+            case 2: return call_form<Form<M, 2, ROWF, EXCH>>(f);
+            case 4: return call_form<Form<M, 4, ROWF, EXCH>>(f);
+            case 6: return call_form<Form<M, 6, ROWF, EXCH>>(f);
+            case 8: return call_form<Form<M, 8, ROWF, EXCH>>(f);
+        }
+        return cudaErrorInvalidValue;
+    };
+    if (metric == 0) return on_cpl(std::integral_constant<int, kMetricL2>{});
+    if (metric == 1) return on_cpl(std::integral_constant<int, kMetricCos>{});
+    return on_cpl(std::integral_constant<int, kMetricDot>{});
+}
+// Runtime (metric, cpl) -> f(Form<METRIC, CPL, kRowF32, false>{}); cudaErrorInvalidValue for a cpl that is not compiled.
+template <typename F>
+static cudaError_t dispatch(int metric, int cpl, F &&f) { return dispatch_form<kRowF32, false>(metric, cpl, f); }
+// The same over the gathered rows' format and the sharded (EXCH) form, for the kernels that have them (K1, K1L, K2).
+template <typename F>
+static cudaError_t dispatch_rows(int rowf, bool exch, int metric, int cpl, F &&f) {
+    if (rowf == kRowF16) return dispatch_form<kRowF16, false>(metric, cpl, f);
+    if (rowf == kRowSQ8) return dispatch_form<kRowSQ8, false>(metric, cpl, f);
+    return exch ? dispatch_form<kRowF32, true>(metric, cpl, f) : dispatch_form<kRowF32, false>(metric, cpl, f);
+}
+
+// kern<<<grid, threads, smem, s>>>(p), raising the kernel's dynamic shared-memory limit first when it asks for more than 48 KB.
+template <typename P>
+static cudaError_t launch_kernel(void (*kern)(P), unsigned grid, unsigned threads, size_t smem, cudaStream_t s, const P &p) {
     if (smem > 48 * 1024) {
         cudaError_t e = cudaFuncSetAttribute(kern, cudaFuncAttributeMaxDynamicSharedMemorySize, static_cast<int>(smem));
         if (e != cudaSuccess) return e;
     }
-    kern<<<grid, 32, smem, s>>>(p);
+    kern<<<grid, threads, smem, s>>>(p);
     return cudaGetLastError();
 }
 
-template <int METRIC, int VIS, bool EXCH, int ROWF>
-static cudaError_t launch_search_metric(int cpl, const SearchParams &p, unsigned grid, size_t smem, cudaStream_t s) {
-    switch (cpl) {
-        case 1: return launch_search_inst<1, METRIC, VIS, EXCH, ROWF>(p, grid, smem, s);
-        case 2: return launch_search_inst<2, METRIC, VIS, EXCH, ROWF>(p, grid, smem, s);
-        case 4: return launch_search_inst<4, METRIC, VIS, EXCH, ROWF>(p, grid, smem, s);
-        case 6: return launch_search_inst<6, METRIC, VIS, EXCH, ROWF>(p, grid, smem, s);
-        case 8: if constexpr (ROWF != kRowSQ8) return launch_search_inst<8, METRIC, VIS, EXCH, ROWF>(p, grid, smem, s); break;
-    }
-    return cudaErrorInvalidValue;
-}
-
-template <int VIS, bool EXCH, int ROWF>
-static cudaError_t launch_search_vis2(int metric, int cpl, const SearchParams &p, unsigned grid, size_t smem, cudaStream_t s) {
-    switch (metric) {
-        case 0: return launch_search_metric<kMetricL2, VIS, EXCH, ROWF>(cpl, p, grid, smem, s);
-        case 1: return launch_search_metric<kMetricCos, VIS, EXCH, ROWF>(cpl, p, grid, smem, s);
-        default: return launch_search_metric<kMetricDot, VIS, EXCH, ROWF>(cpl, p, grid, smem, s);
-    }
-}
-
-// exch = any sharded form of the step (peer stores, records, flags, merge tail): its own instantiation, see the kernel.
-// rowf = the rows the search gathers: kRowF16 / kRowSQ8 = the plain search over the compact copy with the exact re-rank
-// (never together with exch: the entry points refuse it).
+// K1, one warp per query. exch = any sharded form of the step (peer stores, records, flags, merge tail): its own
+// instantiation, see the kernel. rowf = the rows the search gathers: kRowF16 / kRowSQ8 = the plain search over the
+// compact copy with the exact re-rank (never together with exch: refuse_row_form stops it first).
 template <int VIS>
-static cudaError_t launch_search_vis(bool exch, int rowf, int metric, int cpl, const SearchParams &p, unsigned grid, size_t smem, cudaStream_t s) {
-    if (rowf == kRowF16) return launch_search_vis2<VIS, false, kRowF16>(metric, cpl, p, grid, smem, s);
-    if (rowf == kRowSQ8) return launch_search_vis2<VIS, false, kRowSQ8>(metric, cpl, p, grid, smem, s);
-    return exch ? launch_search_vis2<VIS, true, kRowF32>(metric, cpl, p, grid, smem, s) : launch_search_vis2<VIS, false, kRowF32>(metric, cpl, p, grid, smem, s);
+static cudaError_t launch_k1(bool exch, int rowf, int metric, int cpl, const SearchParams &p, unsigned grid, size_t smem, cudaStream_t s) {
+    return dispatch_rows(rowf, exch, metric, cpl, [&](auto fm) {
+        using Fm = decltype(fm);
+        return launch_kernel(search_layer0_kernel<Fm::cpl, Fm::metric, VIS, Fm::exch, Fm::rowf>, grid, 32, smem, s, p);
+    });
 }
 
-template <int METRIC, int ROWF>
-static cudaError_t launch_descend_metric(int cpl, const SearchParams &p, unsigned grid, cudaStream_t s) {
-    switch (cpl) {
-        case 1: descend_kernel<1, METRIC, ROWF><<<grid, 128, 0, s>>>(p); break;
-        case 2: descend_kernel<2, METRIC, ROWF><<<grid, 128, 0, s>>>(p); break;
-        case 4: descend_kernel<4, METRIC, ROWF><<<grid, 128, 0, s>>>(p); break;
-        case 6: descend_kernel<6, METRIC, ROWF><<<grid, 128, 0, s>>>(p); break;
-        case 8: if constexpr (ROWF != kRowSQ8) { descend_kernel<8, METRIC, ROWF><<<grid, 128, 0, s>>>(p); break; } else return cudaErrorInvalidValue;
-        default: return cudaErrorInvalidValue;
-    }
-    return cudaGetLastError();
-}
-template <int ROWF>
-static cudaError_t launch_descend_rowf(int metric, int cpl, const SearchParams &p, unsigned grid, cudaStream_t s) {
-    switch (metric) {
-        case 0: return launch_descend_metric<kMetricL2, ROWF>(cpl, p, grid, s);
-        case 1: return launch_descend_metric<kMetricCos, ROWF>(cpl, p, grid, s);
-        default: return launch_descend_metric<kMetricDot, ROWF>(cpl, p, grid, s);
-    }
-}
-// rowf = the rows the descent walks: those of the layer-0 search it seeds
+// K2; rowf = the rows the descent walks: those of the layer-0 search it seeds
 static cudaError_t launch_descend(int rowf, int metric, int cpl, const SearchParams &p, unsigned grid, cudaStream_t s) {
-    if (rowf == kRowF16) return launch_descend_rowf<kRowF16>(metric, cpl, p, grid, s);
-    if (rowf == kRowSQ8) return launch_descend_rowf<kRowSQ8>(metric, cpl, p, grid, s);
-    return launch_descend_rowf<kRowF32>(metric, cpl, p, grid, s);
+    return dispatch_rows(rowf, false, metric, cpl, [&](auto fm) {
+        using Fm = decltype(fm);
+        return launch_kernel(descend_kernel<Fm::cpl, Fm::metric, Fm::rowf>, grid, 128, 0, s, p);
+    });
 }
 
-// K1L, the latency form: one CTA of 8 (or 4) warps per query (search_team_kernel.cuh)
-template <int CPL, int METRIC, bool ADJC, int MC, int T, int ROWF>
-static cudaError_t launch_team_inst3(const SearchParams &p, unsigned grid, size_t smem, cudaStream_t s) {
-    auto kern = search_team_kernel<CPL, METRIC, ADJC, MC, T>;     // (if constexpr: only the format's own kernel is instantiated)
-    if constexpr (ROWF == kRowF16) kern = search_team_f16_kernel<CPL, METRIC, ADJC, MC, T>;
-    else if constexpr (ROWF == kRowSQ8) kern = search_team_sq8_kernel<CPL, METRIC, ADJC, MC, T>;
-    if (smem > 48 * 1024) {
-        cudaError_t e = cudaFuncSetAttribute(kern, cudaFuncAttributeMaxDynamicSharedMemorySize, static_cast<int>(smem));
-        if (e != cudaSuccess) return e;
-    }
-    kern<<<grid, T, smem, s>>>(p);
-    return cudaGetLastError();
+// K1L, the latency form: one CTA of 8 (or 4) warps per query (search_team_kernel.cuh), each row format a kernel of its own name
+template <typename Fm, bool ADJC, int MC, int T>
+static auto team_kernel() {
+    auto kern = search_team_kernel<Fm::cpl, Fm::metric, ADJC, MC, T>;   // (named in every format: keeps the library's kernel order)
+    if constexpr (Fm::rowf == kRowF16) kern = search_team_f16_kernel<Fm::cpl, Fm::metric, ADJC, MC, T>;
+    else if constexpr (Fm::rowf == kRowSQ8) kern = search_team_sq8_kernel<Fm::cpl, Fm::metric, ADJC, MC, T>;
+    return kern;
 }
 // Full teams (256 threads): m = 16 (BASELINE's M) with the adjacency cache is compiled with m as a constant, everything else
 // reads m from the parameters. Half teams (128 threads) exist without the cache only: they are what a batch runs on that is too
-// large for full teams to be resident at once.
-template <int CPL, int METRIC, int ROWF>
-static cudaError_t launch_team_inst(bool adjc, unsigned threads, const SearchParams &p, unsigned grid, size_t smem, cudaStream_t s) {
-    if (threads == 128) return launch_team_inst3<CPL, METRIC, false, 0, 128, ROWF>(p, grid, smem, s);
-    if (adjc && p.m == 16) return launch_team_inst3<CPL, METRIC, true, 16, 256, ROWF>(p, grid, smem, s);
-    return adjc ? launch_team_inst3<CPL, METRIC, true, 0, 256, ROWF>(p, grid, smem, s) : launch_team_inst3<CPL, METRIC, false, 0, 256, ROWF>(p, grid, smem, s);
-}
-template <int METRIC, int ROWF>
-static cudaError_t launch_team_metric(int cpl, bool adjc, unsigned threads, const SearchParams &p, unsigned grid, size_t smem, cudaStream_t s) {
-    switch (cpl) {
-        case 1: return launch_team_inst<1, METRIC, ROWF>(adjc, threads, p, grid, smem, s);
-        case 2: return launch_team_inst<2, METRIC, ROWF>(adjc, threads, p, grid, smem, s);
-        case 4: return launch_team_inst<4, METRIC, ROWF>(adjc, threads, p, grid, smem, s);
-        case 6: return launch_team_inst<6, METRIC, ROWF>(adjc, threads, p, grid, smem, s);
-        case 8: if constexpr (ROWF != kRowSQ8) return launch_team_inst<8, METRIC, ROWF>(adjc, threads, p, grid, smem, s); break;
-    }
-    return cudaErrorInvalidValue;
-}
-template <int ROWF>
-static cudaError_t launch_team_rowf(int metric, int cpl, bool adjc, unsigned threads, const SearchParams &p, unsigned grid, size_t smem, cudaStream_t s) {
-    switch (metric) {
-        case 0: return launch_team_metric<kMetricL2, ROWF>(cpl, adjc, threads, p, grid, smem, s);
-        case 1: return launch_team_metric<kMetricCos, ROWF>(cpl, adjc, threads, p, grid, smem, s);
-        default: return launch_team_metric<kMetricDot, ROWF>(cpl, adjc, threads, p, grid, smem, s);
-    }
-}
-// adjc = every candidate's adjacency row kept in shared memory (no dependent adjacency fetch at a pop); rowf = the rows gathered
+// large for full teams to be resident at once. adjc = every candidate's adjacency row kept in shared memory (no dependent
+// adjacency fetch at a pop).
 static cudaError_t launch_team(int rowf, int metric, int cpl, bool adjc, unsigned threads, const SearchParams &p, unsigned grid, size_t smem, cudaStream_t s) {
-    if (rowf == kRowF16) return launch_team_rowf<kRowF16>(metric, cpl, adjc, threads, p, grid, smem, s);
-    if (rowf == kRowSQ8) return launch_team_rowf<kRowSQ8>(metric, cpl, adjc, threads, p, grid, smem, s);
-    return launch_team_rowf<kRowF32>(metric, cpl, adjc, threads, p, grid, smem, s);
+    return dispatch_rows(rowf, false, metric, cpl, [&](auto fm) {
+        using Fm = decltype(fm);
+        auto kern = threads == 128 ? team_kernel<Fm, false, 0, 128>() : adjc && p.m == 16 ? team_kernel<Fm, true, 16, 256>()
+                  : adjc ? team_kernel<Fm, true, 0, 256>() : team_kernel<Fm, false, 0, 256>();
+        return launch_kernel(kern, grid, threads == 128 ? 128 : 256, smem, s, p);
+    });
+}
+
+// A search form that is not compiled (row_form_built) for the handle's storage: UNSUPPORTED, naming the storage.
+static int refuse_row_form(int rowf, uint32_t row_floats, bool exch) {
+    if (row_form_built(rowf, cpl_for(row_floats), exch)) return ZVDB_OK;
+    if (exch)
+        return fail(ZVDB_ERR_UNSUPPORTED, std::string("exchange: ") + (rowf == kRowF16 ? "f16" : "sq8") +
+                                              " storage is not built into the sharded forms; set ZVDB_STORAGE_F32");
+    return fail(ZVDB_ERR_UNSUPPORTED, "sq8 storage: built for rows of up to 768 dimensions; set ZVDB_STORAGE_F32 or ZVDB_STORAGE_F16");
 }
 
 // Where the exact visited set of a search with pop budget `ef` lives (see launch_search).
@@ -574,19 +383,16 @@ static int launch_search(zvdb_index *ix, const float *d_q, uint64_t nq, uint32_t
     // arena. The row format is the storage value.
     static_assert(ZVDB_STORAGE_F16 == kRowF16 && ZVDB_STORAGE_SQ8 == kRowSQ8, "storage values name the row formats");
     const int rowf = g.n > 0 ? ix->storage : kRowF32;
-    if (rowf != kRowF32 && (fx || n_peers))
-        return fail(ZVDB_ERR_UNSUPPORTED, rowf == kRowF16 ? "f16 storage: the sharded exchange forms gather fp32 rows only"
-                                                          : "sq8 storage: the sharded exchange forms gather fp32 rows only");
-    if (rowf == kRowSQ8 && g.row_floats > 128u * kSq8MaxCpl)
-        return fail(ZVDB_ERR_UNSUPPORTED, "sq8 storage: built for rows of up to 768 dimensions; set ZVDB_STORAGE_F32 or ZVDB_STORAGE_F16");
+    const bool exch = n_peers != 0 || fx != nullptr;
+    if (int rcr = refuse_row_form(rowf, g.row_floats, exch)) return rcr;
     if (rowf != kRowF32) {
-        int rcf = rowf == kRowF16 ? sync_f16_locked(ix) : sync_sq8_locked(ix);
+        int rcf = ix->row_copy.sync(rowf, g, ix->d_arena, ix->n_dev, ix->cap_rows, ix->num_sms, ix->stream, ix->launches);
         if (rcf) return rcf;
     }
     SearchParams p{};
     p.arena = reinterpret_cast<const float4 *>(ix->d_arena);
-    p.arena16 = rowf == kRowF16 ? ix->d_arena16 : nullptr;
-    p.arena8 = rowf == kRowSQ8 ? reinterpret_cast<const uint32_t *>(ix->d_sq8 + 8ull * g.row_floats) : nullptr;
+    p.arena16 = rowf == kRowF16 ? ix->row_copy.search_rows<kRowF16>(g.row_floats) : nullptr;
+    p.arena8 = rowf == kRowSQ8 ? ix->row_copy.search_rows<kRowSQ8>(g.row_floats) : nullptr;
     p.adj = ix->d_adj;
     p.queries = d_q;
     p.ids = d_ids; p.dist = d_dist; p.counts = d_counts; p.pops = d_pops; p.evals = d_evals;
@@ -608,9 +414,8 @@ static int launch_search(zvdb_index *ix, const float *d_q, uint64_t nq, uint32_t
         }
         p.seeds = ix->seeds_buf.p;
     }
-    const uint32_t chunks_per_lane = (p.row_chunks + 31) / 32;
-    if (chunks_per_lane > 8) return fail(ZVDB_ERR_UNSUPPORTED, "dim > 1024 is not built into the search kernel");
-    const int cpl = chunks_per_lane <= 1 ? 1 : chunks_per_lane <= 2 ? 2 : chunks_per_lane <= 4 ? 4 : chunks_per_lane <= 6 ? 6 : 8;
+    if (p.row_chunks > 8 * 32) return fail(ZVDB_ERR_UNSUPPORTED, "dim > 1024 is not built into the search kernel");
+    const int cpl = cpl_for(p.row_chunks * 4);
 
     const uint64_t bound = std::max<uint64_t>(1, std::min<uint64_t>(g.n, 1ull + static_cast<uint64_t>(ef) * g.m));   // visited-set maximum
     const uint64_t slots = bound + bound / 4 + 16;
@@ -763,10 +568,9 @@ static int launch_search(zvdb_index *ix, const float *d_q, uint64_t nq, uint32_t
         ix->launches++;
         ZV_CUDA(e);
     }
-    const bool exch = n_peers != 0 || fx != nullptr;
-    if (vis == kVisSmemHash) e = launch_search_vis<kVisSmemHash>(exch, rowf, g.metric, cpl, p, grid, smem, s);
-    else if (vis == kVisGlobalBitmap) e = launch_search_vis<kVisGlobalBitmap>(exch, rowf, g.metric, cpl, p, grid, smem, s);
-    else e = launch_search_vis<kVisGlobalHash>(exch, rowf, g.metric, cpl, p, grid, smem, s);
+    if (vis == kVisSmemHash) e = launch_k1<kVisSmemHash>(exch, rowf, g.metric, cpl, p, grid, smem, s);
+    else if (vis == kVisGlobalBitmap) e = launch_k1<kVisGlobalBitmap>(exch, rowf, g.metric, cpl, p, grid, smem, s);
+    else e = launch_k1<kVisGlobalHash>(exch, rowf, g.metric, cpl, p, grid, smem, s);
     ix->launches++;
     ZV_CUDA(e);
     if (vis != kVisSmemHash || p.seeds) ZV_CUDA(cudaEventRecord(ix->bitmap_ev, s));
@@ -856,27 +660,6 @@ static int launch_merge(const uint8_t *dist_base, const uint8_t *ids_base, const
     return ZVDB_OK;
 }
 
-template <int CPL, int METRIC>
-static void launch_build_stage(int stage, const BuildParams &bp, cudaStream_t s) {
-    if (stage == 1) build_forward_kernel<CPL, METRIC><<<bp.n, 32, 0, s>>>(bp);
-    else build_final_kernel<CPL, METRIC><<<bp.n, 32, 0, s>>>(bp);
-}
-template <int METRIC>
-static void launch_build_metric(int cpl, int stage, const BuildParams &bp, cudaStream_t s) {
-    switch (cpl) {
-        case 1: launch_build_stage<1, METRIC>(stage, bp, s); break;
-        case 2: launch_build_stage<2, METRIC>(stage, bp, s); break;
-        case 4: launch_build_stage<4, METRIC>(stage, bp, s); break;
-        case 6: launch_build_stage<6, METRIC>(stage, bp, s); break;
-        default: launch_build_stage<8, METRIC>(stage, bp, s); break;
-    }
-}
-static void launch_build(int metric, int cpl, int stage, const BuildParams &bp, cudaStream_t s) {
-    if (metric == 0) launch_build_metric<kMetricL2>(cpl, stage, bp, s);
-    else if (metric == 1) launch_build_metric<kMetricCos>(cpl, stage, bp, s);
-    else launch_build_metric<kMetricDot>(cpl, stage, bp, s);
-}
-
 // ---- K4 launch: exact brute-force k-NN ----------------------------------------------------------
 
 typedef CUresult (*TensorMapEncodeFn)(CUtensorMap *, CUtensorMapDataType, cuuint32_t, void *, const cuuint64_t *,
@@ -910,23 +693,6 @@ static int make_tile_map(CUtensorMap *map, const float *base, uint64_t rows, uin
                      CU_TENSOR_MAP_FLOAT_OOB_FILL_NONE);
     if (r != CUDA_SUCCESS) return fail(ZVDB_ERR_CUDA, "cuTensorMapEncodeTiled failed (" + std::to_string(static_cast<int>(r)) + ")");
     return ZVDB_OK;
-}
-
-template <int METRIC>
-static cudaError_t launch_bf_final_metric(int cpl, const bf::BfFinalParams &fp, size_t smem, cudaStream_t s) {
-#define ZV_FIN(C)                                                                                            \
-    case C: {                                                                                                \
-        auto kern = bf::bf_finalize_kernel<C, METRIC>;                                                       \
-        if (smem > 48 * 1024) {                                                                              \
-            cudaError_t e = cudaFuncSetAttribute(kern, cudaFuncAttributeMaxDynamicSharedMemorySize, static_cast<int>(smem)); \
-            if (e != cudaSuccess) return e;                                                                  \
-        }                                                                                                    \
-        kern<<<fp.nq, 32, smem, s>>>(fp);                                                                    \
-        return cudaGetLastError();                                                                           \
-    }
-    switch (cpl) { ZV_FIN(1) ZV_FIN(2) ZV_FIN(4) ZV_FIN(6) ZV_FIN(8) }
-#undef ZV_FIN
-    return cudaErrorInvalidValue;
 }
 
 // K4 work plan. The tile space is n_qtiles x n_rtiles; a segment is (query tile, row-tile range,
@@ -1110,12 +876,11 @@ static int launch_bruteforce(zvdb_index *ix, const float *d_q, uint64_t nq, uint
     fp.id_stride = id_stride; fp.id_base = id_base;
     fp.row_chunks = pitch / 4; fp.dim = g.dim; fp.nq = p.nq; fp.k = k; fp.kp = p.kp; fp.n_splits = p.n_slots;
     fp.p2 = next_pow2(p.n_slots * p.kp); fp.kk2 = std::max<uint32_t>(2, next_pow2(p.kp));
-    const uint32_t cpl_raw = (fp.row_chunks + 31) / 32;
-    const int cpl = cpl_raw <= 1 ? 1 : cpl_raw <= 2 ? 2 : cpl_raw <= 4 ? 4 : cpl_raw <= 6 ? 6 : 8;
     const size_t fsmem = (static_cast<size_t>(fp.p2) + fp.kk2) * sizeof(uint64_t);
-    cudaError_t e = g.metric == 0 ? launch_bf_final_metric<kMetricL2>(cpl, fp, fsmem, s)
-                  : g.metric == 1 ? launch_bf_final_metric<kMetricCos>(cpl, fp, fsmem, s)
-                                  : launch_bf_final_metric<kMetricDot>(cpl, fp, fsmem, s);
+    cudaError_t e = dispatch(g.metric, cpl_for(pitch), [&](auto fm) {
+        using Fm = decltype(fm);
+        return launch_kernel(bf::bf_finalize_kernel<Fm::cpl, Fm::metric>, fp.nq, 32, fsmem, s, fp);
+    });
     ix->launches++;
     ZV_CUDA(e);
     ZV_CUDA(cudaEventRecord(ix->bf_ev, s));
@@ -1176,9 +941,9 @@ void zvdb_destroy(zvdb_index *ix) {
     for (int i = 0; i < 8; ++i) if (ix->in_ev[i]) cudaEventDestroy(ix->in_ev[i]);
     if (ix->bitmap_ev) cudaEventDestroy(ix->bitmap_ev);
     if (ix->bf_ev) cudaEventDestroy(ix->bf_ev);
-    cudaFree(ix->d_arena); cudaFree(ix->d_adj); cudaFree(ix->d_arena16); cudaFree(ix->d_sq8);
+    cudaFree(ix->d_arena); cudaFree(ix->d_adj);
     if (ix->h_stage) cudaFreeHost(ix->h_stage);
-    ix->f16_bad.free_(); ix->sq8_minmax.free_();
+    ix->row_copy.release();
     ix->q_buf.free_(); ix->dist_buf.free_(); ix->ids_buf.free_(); ix->cnt_buf.free_();
     ix->pops_buf.free_(); ix->evals_buf.free_(); ix->scat_rows.free_(); ix->scat_ids.free_(); ix->bitmap_buf.free_(); ix->vlog_buf.free_(); ix->res_buf.free_(); ix->gtable_buf.free_();
     ix->d_level.free_(); ix->d_upper_base.free_(); ix->d_upper_adj.free_(); ix->seeds_buf.free_();
@@ -1386,7 +1151,7 @@ static int set_points_locked(zvdb_index *ix, const float *points, uint64_t n, ui
     }
     g.has_entry = n > 0; g.entry = entry; g.max_level = 0;
     g.rows_uploaded = 0; g.adj_all_dirty = true;
-    ix->n_dev = 0; ix->bf_rows = 0; ix->f16_rows = 0; ix->sq8_rows = 0; ix->sq8_trained = false;
+    forget_device_rows(ix);
     return ZVDB_OK;
 }
 
@@ -1493,7 +1258,7 @@ int zvdb_load(zvdb_index *ix, const char *path) {
         g.dim = 0; g.row_floats = 0; g.rows_per_chunk = 0;
         if (hd.dim) g.fix_dim(hd.dim);
         g.ef_construction = hd.ef_construction; g.rng = hd.rng; g.dtype = 0;
-        ix->n_dev = 0; ix->bf_rows = 0; ix->f16_rows = 0; ix->sq8_rows = 0; ix->sq8_trained = false;
+        forget_device_rows(ix);
         return ZVDB_OK;
     }
     if (hd.dim == 0 || hd.dim > 1024 || hd.row_floats != (hd.dim + 31u) / 32u * 32u || hd.n >= 0xFFFFFFFEull || hd.max_level > 31 ||
@@ -1570,7 +1335,7 @@ int zvdb_load(zvdb_index *ix, const char *path) {
     g.upper_off.swap(fresh.upper_off); g.upper.swap(fresh.upper);
     g.has_entry = fresh.has_entry; g.entry = fresh.entry; g.max_level = fresh.max_level; g.top_node = fresh.top_node; g.rng = fresh.rng;
     ++g.upper_version; g.rows_uploaded = 0; g.dirty.clear(); g.adj_all_dirty = true;
-    ix->n_dev = 0; ix->bf_rows = 0; ix->f16_rows = 0; ix->sq8_rows = 0; ix->sq8_trained = false;
+    forget_device_rows(ix);
     return ZVDB_OK;
 }
 
@@ -1590,29 +1355,20 @@ int zvdb_set_storage(zvdb_index *ix, int storage) {
         return fail(ZVDB_ERR_UNSUPPORTED, "set_storage: f16 storage is built for f32 indexes only (this one holds f64 / i32 rows)");
     if (storage == ZVDB_STORAGE_SQ8 && ix->g.dtype != 0)
         return fail(ZVDB_ERR_UNSUPPORTED, "set_storage: sq8 storage is built for f32 indexes only (this one holds f64 / i32 rows)");
+    int rc = ix->row_copy.set_format(ix->storage, storage, ix->device);
+    if (rc) return rc;
     ix->storage = storage;
-    // The copy the new setting does not read is freed (F32 frees both); setting SQ8, even again, trains a new codebook at
-    // the next search. Searches enqueued on caller streams may still read what changes here.
-    const bool drop16 = storage != ZVDB_STORAGE_F16 && ix->d_arena16;
-    const bool drop8 = ix->d_sq8 && (storage != ZVDB_STORAGE_SQ8 || ix->sq8_trained);
-    if (drop16 || drop8) {
-        ZV_CUDA(cudaSetDevice(ix->device));
-        ZV_CUDA(cudaDeviceSynchronize());
-    }
-    if (drop16) { cudaFree(ix->d_arena16); ix->d_arena16 = nullptr; ix->f16_rows = 0; }
-    if (storage != ZVDB_STORAGE_SQ8) { cudaFree(ix->d_sq8); ix->d_sq8 = nullptr; }
-    ix->sq8_rows = 0; ix->sq8_trained = false;
-    ix->sq8_scale.clear(); ix->sq8_offset.clear();
     return ZVDB_OK;
 }
 
 int zvdb_storage_codebook(const zvdb_index *ix, float *scale, float *offset, uint32_t dim) {
     if (!ix || !scale || !offset) return fail(ZVDB_ERR_INVALID, "storage_codebook: null argument");
     ZV_LOCKED(ix);
-    if (!ix->sq8_trained || ix->sq8_scale.empty()) return fail(ZVDB_ERR_INVALID, "storage_codebook: no SQ8 codebook is trained (it is at the first search under ZVDB_STORAGE_SQ8)");
+    const float *cb = ix->row_copy.codebook();
+    if (!cb) return fail(ZVDB_ERR_INVALID, "storage_codebook: no SQ8 codebook is trained (it is at the first search under ZVDB_STORAGE_SQ8)");
     if (dim != ix->g.dim) return fail(ZVDB_ERR_DIM_MISMATCH, "storage_codebook: dim differs from the index's");
-    std::memcpy(scale, ix->sq8_scale.data(), dim * sizeof(float));
-    std::memcpy(offset, ix->sq8_offset.data(), dim * sizeof(float));
+    std::memcpy(scale, cb, dim * sizeof(float));
+    std::memcpy(offset, cb + ix->g.row_floats, dim * sizeof(float));
     return ZVDB_OK;
 }
 
@@ -1708,10 +1464,15 @@ static int build_from_candidates_locked(zvdb_index *ix, uint64_t n, const uint32
     bp.arena = reinterpret_cast<const float4 *>(ix->d_arena);
     bp.row_chunks = g.row_floats / 4; bp.n = static_cast<uint32_t>(n); bp.m = g.m;
     bp.cand = cand_dev; bp.K = K; bp.fw = d_fw.p; bp.adj = ix->d_adj;
-    const uint32_t cpl_raw = (bp.row_chunks + 31) / 32;
-    const int cpl = cpl_raw <= 1 ? 1 : cpl_raw <= 2 ? 2 : cpl_raw <= 4 ? 4 : cpl_raw <= 6 ? 6 : 8;
-    launch_build(g.metric, cpl, 1, bp, s); ix->launches++;
-    ZV_CUDA(cudaGetLastError());
+    auto launch_build = [&](bool forward) {               // K6: forward lists, then the final lists
+        return dispatch(g.metric, cpl_for(g.row_floats), [&](auto fm) {
+            using Fm = decltype(fm);
+            return launch_kernel(forward ? build_forward_kernel<Fm::cpl, Fm::metric> : build_final_kernel<Fm::cpl, Fm::metric>,
+                                 bp.n, 32, 0, s, bp);
+        });
+    };
+    cudaError_t e = launch_build(true); ix->launches++;
+    ZV_CUDA(e);
     const uint64_t total = n * g.m;
     const unsigned blocks = static_cast<unsigned>(std::min<uint64_t>((total + 255) / 256, 148ull * 16));
     count_reverse_kernel<<<blocks, 256, 0, s>>>(d_fw.p, total, d_indeg.p); ix->launches++;
@@ -1727,8 +1488,8 @@ static int build_from_candidates_locked(zvdb_index *ix, uint64_t n, const uint32
     ZV_CUDA(cudaMemcpyAsync(d_off.p, off.data(), (n + 1) * sizeof(uint64_t), cudaMemcpyHostToDevice, s));
     fill_reverse_kernel<<<blocks, 256, 0, s>>>(d_fw.p, total, g.m, d_off.p, d_indeg.p + n, d_rev.p); ix->launches++;
     bp.rev_off = d_off.p; bp.rev = d_rev.p;
-    launch_build(g.metric, cpl, 3, bp, s); ix->launches++;
-    ZV_CUDA(cudaGetLastError());
+    e = launch_build(false); ix->launches++;
+    ZV_CUDA(e);
     ZV_CUDA(cudaMemcpyAsync(g.adj0.data(), ix->d_adj, n * g.m * sizeof(uint32_t), cudaMemcpyDeviceToHost, s));
     ZV_CUDA(cudaStreamSynchronize(s));
     return ZVDB_OK;
@@ -1749,7 +1510,7 @@ int zvdb_build_from_candidates(zvdb_index *ix, const float *points, uint64_t n, 
         // becomes empty (the error string of the failing step is kept).
         const std::string why = g_last_error;
         g.reset_nodes();
-        ix->n_dev = 0; ix->bf_rows = 0; ix->f16_rows = 0; ix->sq8_rows = 0; ix->sq8_trained = false;
+        forget_device_rows(ix);
         return fail(rc, why);
     }
     // the table was produced on the device and copied back: both sides are current
@@ -2149,8 +1910,7 @@ int zvdb_search_batch_exchange(zvdb_index *ix, zvdb_exchange *ex, const float *d
     const uint64_t block = zvdb_shard_block_bytes(nq, k);
     if (block * ex->world > ex->cap_bytes) return fail(ZVDB_ERR_INVALID, "exchange: nq * k exceeds the capacity the exchange was created with");
     std::lock_guard<std::mutex> lk(ix->mu);
-    if (ix->storage == ZVDB_STORAGE_F16) return fail(ZVDB_ERR_UNSUPPORTED, "exchange: f16 storage is not built into the sharded forms; set ZVDB_STORAGE_F32");
-    if (ix->storage == ZVDB_STORAGE_SQ8) return fail(ZVDB_ERR_UNSUPPORTED, "exchange: sq8 storage is not built into the sharded forms; set ZVDB_STORAGE_F32");
+    if (int rc = refuse_row_form(ix->storage, ix->g.row_floats, true)) return rc;
     ZV_CUDA(cudaSetDevice(ix->device));
     cudaStream_t s = static_cast<cudaStream_t>(stream);
     const uint32_t epoch = ++ex->epoch;
@@ -2212,8 +1972,7 @@ int zvdb_search_batch_exchange_host(zvdb_index *ix, zvdb_exchange *ex, const flo
     const uint64_t block = zvdb_shard_block_bytes(nq, k);
     if (block * ex->world > ex->cap_bytes) return fail(ZVDB_ERR_INVALID, "exchange: nq * k exceeds the capacity the exchange was created with");
     std::lock_guard<std::mutex> lk(ix->mu);
-    if (ix->storage == ZVDB_STORAGE_F16) return fail(ZVDB_ERR_UNSUPPORTED, "exchange: f16 storage is not built into the sharded forms; set ZVDB_STORAGE_F32");
-    if (ix->storage == ZVDB_STORAGE_SQ8) return fail(ZVDB_ERR_UNSUPPORTED, "exchange: sq8 storage is not built into the sharded forms; set ZVDB_STORAGE_F32");
+    if (int rc = refuse_row_form(ix->storage, ix->g.row_floats, true)) return rc;
     ZV_CUDA(cudaSetDevice(ix->device));
     const bool empty = ix->g.n == 0 || !ix->g.has_entry;
     if (!empty && dim != ix->g.dim) return fail(ZVDB_ERR_DIM_MISMATCH, "Mismatched dimensions in distance calculation");

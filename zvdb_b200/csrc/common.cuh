@@ -40,6 +40,21 @@ __host__ __device__ __forceinline__ uint32_t next_pow2(uint32_t v) {
     return p;
 }
 
+template <typename T>
+struct DevBuf {
+    T *p = nullptr;
+    size_t cap = 0;
+    cudaError_t reserve(size_t count) {
+        if (count <= cap) return cudaSuccess;
+        if (p) cudaFree(p);
+        p = nullptr; cap = 0;
+        cudaError_t e = cudaMalloc(&p, count * sizeof(T));
+        if (e == cudaSuccess) cap = count;
+        return e;
+    }
+    void free_() { if (p) cudaFree(p); p = nullptr; cap = 0; }
+};
+
 #ifdef __CUDACC__
 // Barrier for a query team: a team is the whole CTA; a one-warp CTA only needs a warp barrier.
 __device__ __forceinline__ void team_sync() {

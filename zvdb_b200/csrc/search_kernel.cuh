@@ -137,6 +137,11 @@ constexpr uint32_t kPoolCap = 64;   // pending pool slots
 enum : int { kRowF32 = 0, kRowF16 = 1, kRowSQ8 = 2 };
 // SQ8 is built for rows of up to 768 floats (CPL <= 6): at 1024 the one-warp kernel does not fit its registers without spills.
 constexpr int kSq8MaxCpl = 6;
+// The (row format, CPL, sharded step) forms K1, K1L and K2 are compiled for: fp32 everywhere; the compact formats in the plain
+// search only (the sharded forms gather fp32 rows); SQ8 up to kSq8MaxCpl. Host side: what is instantiated and what is refused.
+constexpr bool row_form_built(int rowf, int cpl, bool exch) {
+    return rowf == kRowF32 || (!exch && (rowf != kRowSQ8 || cpl <= kSq8MaxCpl));
+}
 template <int ROWF> using RowChunk =
     std::conditional_t<ROWF == kRowF16, uint2, std::conditional_t<ROWF == kRowSQ8, uint32_t, float4>>;
 __device__ __forceinline__ float4 chunk_f32(const float4 v) { return v; }
