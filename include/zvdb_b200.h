@@ -135,6 +135,26 @@ ZVDB_API int zvdb_load_graph(zvdb_index *ix, const float *points, uint64_t n, ui
 ZVDB_API int zvdb_build_from_candidates(zvdb_index *ix, const float *points, uint64_t n, uint32_t dim,
                                         const uint32_t *cand, uint32_t K, int cand_on_device);
 
+/* Append n rows points[n x dim] to a non-empty index and link them ON THE GPU without a rebuild (K7,
+ * zvdb_b200/csrc/append.cuh). The rows become nodes n0 .. n0+n-1 (n0 = the count before the call) at
+ * level 0. Every distance is in the kernels' summation order, every ordering by (distance, id):
+ *   1. C_i = the first K ids zvdb_search_batch_device(x_i, k = K, ef) returns on the graph as it was
+ *      before the call (the handle's storage, descent and variant settings apply; x_i = the stored row,
+ *      normalised under cosine). Rows of one call cannot find each other.
+ *   2. fw[i] = the builder's relative-neighbourhood selection over C_i, stopping at m.
+ *   3. R_j = { i in the batch : j in fw[i] } for every node j.
+ *   4. The builder's final rule -- the union cut to its nearest 96 members, the relative-neighbourhood
+ *      selection, a top-up with the nearest rejected members -- over fw[i] + R_i for a new row, and over
+ *      its current layer-0 list + R_j for an old row with a non-empty R_j. Every other row keeps its list.
+ * Upper layers, max_level, the entry point and the descent start do not change. ef = 0 means 4 * K.
+ * On success host and device copies are both current. On failure the index is as before the call.
+ * n = 0 is a no-op. Errors: ZVDB_ERR_INVALID (empty index: build it with zvdb_build_from_candidates or
+ * zvdb_insert first; ef < K; NULL points), ZVDB_ERR_DIM_MISMATCH, ZVDB_ERR_UNSUPPORTED (f64 / i32
+ * index, m > 64, K outside 1..128, more than 2^32-2 nodes). SQ8 does not retrain: an append counts as
+ * an insert. */
+ZVDB_API int zvdb_append_batch(zvdb_index *ix, const float *points, uint64_t n, uint32_t dim, uint32_t K,
+                               uint32_t ef);
+
 /* ---- upper layers and the descent (north_star subsystem 2, SURVEY 8f rank 2) ----------------------
  * The reference BUILDS layers >= 1 (hnsw.zig:88-108) but its search never reads them (hnsw.zig:216).
  * With the descent switched on, a search first walks layers max_level..1 greedily from the node that

@@ -29,6 +29,7 @@ extern fn zvdb_search_typed(ix: *zvdb_index, query: *const anyopaque, dim: u32, 
 extern fn zvdb_search_batch_typed(ix: *zvdb_index, queries: *const anyopaque, nq: u64, dim: u32, dtype: c_int, k: u32, ef: u32, ids: [*]u64, dist: [*]f32, counts: [*]u32) c_int;
 extern fn zvdb_get_point_typed(ix: *const zvdb_index, id: u64) ?*const anyopaque;
 extern fn zvdb_set_descent(ix: *zvdb_index, on: c_int) c_int;
+extern fn zvdb_append_batch(ix: *zvdb_index, points: [*]const f32, n: u64, dim: u32, K: u32, ef: u32) c_int;
 extern fn zvdb_set_storage(ix: *zvdb_index, storage: c_int) c_int;
 extern fn zvdb_storage(ix: *const zvdb_index) c_int;
 extern fn zvdb_save(ix: *const zvdb_index, path: [*:0]const u8) c_int;
@@ -134,6 +135,16 @@ pub fn HNSW(comptime T: type) type {
             const h = self.handle orelse return error.CudaError;
             const dim = queries.len / nq;
             try check(zvdb_search_batch_typed(h, @ptrCast(queries.ptr), nq, @intCast(dim), dtype, @intCast(k), @intCast(ef), ids.ptr, dist.ptr, counts.ptr));
+        }
+
+        /// Extension: append n rows (points = n x dim, f32 indexes only) to a built index and link them on the GPU
+        /// (zvdb_append_batch, K7): each row is searched on the graph as it was (K candidates, ef pops; 0 = 4 * K) and
+        /// linked by the builder's rules; the old rows it links to gain it. Rows of one call cannot find each other:
+        /// append a large batch in parts of a few percent of count().
+        pub fn appendBatch(self: *Self, points: []const f32, n: usize, K: usize, ef: usize) !void {
+            const h = self.handle orelse return error.CudaError;
+            if (n == 0) return;
+            try check(zvdb_append_batch(h, points.ptr, n, @intCast(points.len / n), @intCast(K), @intCast(ef)));
         }
 
         /// Extension: walk layers max_level..1 greedily (the walk of insert, hnsw.zig:89-104) before the

@@ -43,6 +43,7 @@ SIGNATURES = {
     "zvdb_export_layer": (_i32, [_vp, _u32, _pu32, _pu32]),
     "zvdb_load_graph": (_i32, [_vp, _pf, _u64, _u32, _pu64, _pu32, _u64]),
     "zvdb_build_from_candidates": (_i32, [_vp, _pf, _u64, _u32, _vp, _u32, _i32]),
+    "zvdb_append_batch": (_i32, [_vp, _pf, _u64, _u32, _u32, _u32]),
     "zvdb_set_descent": (_i32, [_vp, _i32]),
     "zvdb_descent_start": (_i64, [_vp]),
     "zvdb_set_storage": (_i32, [_vp, _i32]),

@@ -15,7 +15,12 @@
 #include "search_kernel.cuh"
 #include "search_team_kernel.cuh"
 #include "builder.cuh"
+#include "append.cuh"
 #include "bruteforce.cuh"
+#include <cub/device/device_scan.cuh>
+#include <cub/device/device_select.cuh>
+#include <thrust/iterator/counting_iterator.h>
+#include <thrust/iterator/transform_iterator.h>
 
 namespace zvdb {
 
@@ -1136,19 +1141,7 @@ static int set_points_locked(zvdb_index *ix, const float *points, uint64_t n, ui
         g.chunks.push_back(p);
     }
     g.n = n;
-    for (uint64_t i = 0; i < n; ++i) {
-        float *row = g.point_mut(i);
-        std::memcpy(row, points + i * dim, dim * sizeof(float));
-        if (g.metric == 1) {
-            double s = 0.0;
-            for (uint32_t t = 0; t < dim; ++t) s += static_cast<double>(row[t]) * static_cast<double>(row[t]);
-            if (s > 0.0) {
-                const double inv = 1.0 / std::sqrt(s);
-                for (uint32_t t = 0; t < dim; ++t) row[t] = static_cast<float>(static_cast<double>(row[t]) * inv);
-            }
-        }
-        for (uint32_t t = dim; t < g.row_floats; ++t) row[t] = 0.0f;
-    }
+    for (uint64_t i = 0; i < n; ++i) g.store_row(g.point_mut(i), points + i * dim);
     g.has_entry = n > 0; g.entry = entry; g.max_level = 0;
     g.rows_uploaded = 0; g.adj_all_dirty = true;
     forget_device_rows(ix);
@@ -1516,6 +1509,151 @@ int zvdb_build_from_candidates(zvdb_index *ix, const float *points, uint64_t n, 
     // the table was produced on the device and copied back: both sides are current
     g.rows_uploaded = n; g.dirty.clear(); g.adj_all_dirty = false;
     ix->n_dev = n;
+    return ZVDB_OK;
+}
+
+// K7 on rows [n0, g.n) of the host graph (append_rows done, device current up to n0): upload, steps 1-4 of append.cuh,
+// the touched rows back into g.adj0. touched_host holds the touched ids before the final pass starts (final_started),
+// so that a failure after that can mark them for re-sending.
+static int append_locked(zvdb_index *ix, uint64_t n0, uint32_t K, uint32_t ef, std::vector<uint32_t> &touched_host,
+                         bool &final_started) {
+    HostGraph &g = ix->g;
+    const uint64_t n = g.n, nb = n - n0;
+    int rc = ensure_capacity(ix, n);
+    if (rc) return rc;
+    cudaStream_t s = ix->stream;
+    for (uint64_t r = n0; r < n;) {                      // the batch's arena rows up (no links yet: nothing reaches them)
+        const uint64_t chunk = r / g.rows_per_chunk;
+        const uint64_t end = std::min<uint64_t>(n, (chunk + 1) * g.rows_per_chunk);
+        ZV_CUDA(cudaMemcpyAsync(ix->d_arena + r * g.row_floats, g.point(r), (end - r) * g.row_floats * sizeof(float), cudaMemcpyHostToDevice, s));
+        r = end;
+    }
+    DevBuf<float> d_q, d_dist;
+    DevBuf<uint64_t> d_ids, d_off;
+    DevBuf<uint32_t> d_cnt, d_fw, d_indeg, d_rev, d_touched, d_rows;
+    DevBuf<uint8_t> d_tmp;
+    struct Cleanup {                                     // every exit frees the append scratch
+        DevBuf<float> &a, &b; DevBuf<uint64_t> &c, &d; DevBuf<uint32_t> &e, &f, &g, &h, &i, &j; DevBuf<uint8_t> &k;
+        ~Cleanup() { a.free_(); b.free_(); c.free_(); d.free_(); e.free_(); f.free_(); g.free_(); h.free_(); i.free_(); j.free_(); k.free_(); }
+    } cleanup{d_q, d_dist, d_ids, d_off, d_cnt, d_fw, d_indeg, d_rev, d_touched, d_rows, d_tmp};
+    // 1. search: the batch's stored rows as queries (dim floats each), on the graph as it was
+    ZV_CUDA(d_q.reserve(nb * g.dim));
+    ZV_CUDA(cudaMemcpy2DAsync(d_q.p, g.dim * sizeof(float), ix->d_arena + n0 * g.row_floats, g.row_floats * sizeof(float),
+                              g.dim * sizeof(float), nb, cudaMemcpyDeviceToDevice, s));
+    ZV_CUDA(d_ids.reserve(nb * K));
+    ZV_CUDA(d_dist.reserve(nb * K));
+    ZV_CUDA(d_cnt.reserve(nb));
+    for (uint64_t q0 = 0; q0 < nb; q0 += 0x7FFFFFFFull) {   // launch_search's per-launch query limit
+        const uint64_t cnt = std::min<uint64_t>(nb - q0, 0x7FFFFFFFull);
+        rc = launch_search(ix, d_q.p + q0 * g.dim, cnt, K, ef, d_ids.p + q0 * K, d_dist.p + q0 * K, d_cnt.p + q0, nullptr, nullptr,
+                           1, 0, s);
+        if (rc) return rc;
+    }
+    // 2. forward lists of the batch
+    ZV_CUDA(d_fw.reserve(nb * g.m));
+    AppendParams ap{};
+    ap.arena = reinterpret_cast<const float4 *>(ix->d_arena);
+    ap.row_chunks = g.row_floats / 4; ap.n = static_cast<uint32_t>(n); ap.n0 = static_cast<uint32_t>(n0); ap.m = g.m;
+    ap.cand = d_ids.p; ap.K = K; ap.fw = d_fw.p; ap.adj = ix->d_adj;
+    const int cpl = cpl_for(g.row_floats);
+    cudaError_t e = dispatch(g.metric, cpl, [&](auto fm) {
+        using Fm = decltype(fm);
+        return launch_kernel(append_forward_kernel<Fm::cpl, Fm::metric>, static_cast<unsigned>(nb), 32, 0, s, ap);
+    });
+    ix->launches++;
+    ZV_CUDA(e);
+    // 3. reverse rows: per-node counts (K6's kernels), offsets by a scan over the counts, the touched rows by a select
+    ZV_CUDA(d_indeg.reserve(2 * n));
+    ZV_CUDA(d_off.reserve(n));
+    ZV_CUDA(cudaMemsetAsync(d_indeg.p, 0, 2 * n * sizeof(uint32_t), s));
+    const uint64_t total = nb * g.m;
+    const unsigned blocks = static_cast<unsigned>(std::min<uint64_t>((total + 255) / 256, 148ull * 16));
+    count_reverse_kernel<<<blocks, 256, 0, s>>>(d_fw.p, total, d_indeg.p); ix->launches++;
+    ZV_CUDA(cudaGetLastError());
+    const uint64_t touched_cap = std::min<uint64_t>(n, nb + total);
+    ZV_CUDA(d_touched.reserve(touched_cap + 1));          // + the select's count word
+    uint32_t *d_nsel = d_touched.p + touched_cap;
+    auto widened = thrust::make_transform_iterator(d_indeg.p, WidenU32{});
+    const thrust::counting_iterator<uint32_t> node_ids(0);
+    const TouchedRow pick{d_indeg.p, static_cast<uint32_t>(n0)};
+    size_t scan_bytes = 0, select_bytes = 0;
+    ZV_CUDA(cub::DeviceScan::ExclusiveSum(nullptr, scan_bytes, widened, d_off.p, static_cast<int64_t>(n), s));
+    ZV_CUDA(cub::DeviceSelect::If(nullptr, select_bytes, node_ids, d_touched.p, d_nsel, static_cast<int64_t>(n), pick, s));
+    ZV_CUDA(d_tmp.reserve(std::max<size_t>(std::max(scan_bytes, select_bytes), 1)));
+    ZV_CUDA(cub::DeviceScan::ExclusiveSum(d_tmp.p, scan_bytes, widened, d_off.p, static_cast<int64_t>(n), s));
+    ix->launches++;
+    ZV_CUDA(d_rev.reserve(std::max<uint64_t>(total, 1)));
+    fill_reverse_kernel<<<blocks, 256, 0, s>>>(d_fw.p, total, g.m, d_off.p, d_indeg.p + n, d_rev.p); ix->launches++;
+    ZV_CUDA(cudaGetLastError());
+    ZV_CUDA(cub::DeviceSelect::If(d_tmp.p, select_bytes, node_ids, d_touched.p, d_nsel, static_cast<int64_t>(n), pick, s));
+    ix->launches++;
+    uint32_t nt = 0;
+    ZV_CUDA(cudaMemcpyAsync(&nt, d_nsel, sizeof nt, cudaMemcpyDeviceToHost, s));
+    ZV_CUDA(cudaStreamSynchronize(s));
+    try { touched_host.resize(nt); } catch (const std::bad_alloc &) { return fail(ZVDB_ERR_OUT_OF_MEMORY, "append: out of memory"); }
+    ZV_CUDA(cudaMemcpyAsync(touched_host.data(), d_touched.p, nt * sizeof(uint32_t), cudaMemcpyDeviceToHost, s));
+    ZV_CUDA(cudaStreamSynchronize(s));
+    // 4. final lists of the touched rows, in place
+    ap.touched = d_touched.p; ap.rev_off = d_off.p; ap.rev_cnt = d_indeg.p; ap.rev = d_rev.p;
+    final_started = true;
+    e = dispatch(g.metric, cpl, [&](auto fm) {
+        using Fm = decltype(fm);
+        return launch_kernel(append_final_kernel<Fm::cpl, Fm::metric>, nt, 32, 0, s, ap);
+    });
+    ix->launches++;
+    ZV_CUDA(e);
+    // the touched rows back: gather on the device, one copy, scatter into the host table
+    std::vector<uint32_t> rows;
+    try { rows.resize(static_cast<size_t>(nt) * g.m); } catch (const std::bad_alloc &) { return fail(ZVDB_ERR_OUT_OF_MEMORY, "append: out of memory"); }
+    ZV_CUDA(d_rows.reserve(std::max<size_t>(rows.size(), 1)));
+    const unsigned gblocks = static_cast<unsigned>(std::min<uint64_t>((rows.size() + 255) / 256 + 1, 148ull * 8));
+    gather_adj_rows_kernel<<<gblocks, 256, 0, s>>>(d_rows.p, ix->d_adj, d_touched.p, nt, g.m); ix->launches++;
+    ZV_CUDA(cudaGetLastError());
+    ZV_CUDA(cudaMemcpyAsync(rows.data(), d_rows.p, rows.size() * sizeof(uint32_t), cudaMemcpyDeviceToHost, s));
+    ZV_CUDA(cudaStreamSynchronize(s));
+    for (uint32_t t = 0; t < nt; ++t)
+        std::memcpy(g.adj0.data() + static_cast<size_t>(touched_host[t]) * g.m, rows.data() + static_cast<size_t>(t) * g.m, g.m * sizeof(uint32_t));
+    return ZVDB_OK;
+}
+
+int zvdb_append_batch(zvdb_index *ix, const float *points, uint64_t n, uint32_t dim, uint32_t K, uint32_t ef) {
+    if (!ix) return fail(ZVDB_ERR_INVALID, "null index");
+    if (n == 0) return ZVDB_OK;
+    if (!points) return fail(ZVDB_ERR_INVALID, "append: null points");
+    if (K == 0 || K > kBuildBuf) return fail(ZVDB_ERR_UNSUPPORTED, "append: K must be in 1..128");
+    if (ef == 0) ef = 4 * K;                              // the incremental builder's default
+    if (ef < K) return fail(ZVDB_ERR_INVALID, "append: ef must be >= K (0 = 4 * K)");
+    std::lock_guard<std::mutex> lk(ix->mu);
+    HostGraph &g = ix->g;
+    if (g.n == 0 || !g.has_entry)
+        return fail(ZVDB_ERR_INVALID, "append: the index is empty; build it with zvdb_build_from_candidates or zvdb_insert first");
+    if (g.dtype != 0) return fail(ZVDB_ERR_UNSUPPORTED, "append: f64 / i32 indexes are not supported; use zvdb_insert_typed");
+    if (g.m > 64) return fail(ZVDB_ERR_UNSUPPORTED, "append: m must be <= 64");
+    if (dim != g.dim) return fail(ZVDB_ERR_DIM_MISMATCH, "Mismatched dimensions in distance calculation");
+    if (n >= 0xFFFFFFFEull - g.n) return fail(ZVDB_ERR_UNSUPPORTED, "append: more than 2^32-2 nodes in one shard");
+    ZV_CUDA(cudaSetDevice(ix->device));
+    int rc = sync_device_locked(ix);                      // the device holds the graph before the call
+    if (rc) return rc;
+    ZV_CUDA(cudaDeviceSynchronize());                     // searches enqueued on caller streams may still read the tables
+    const uint64_t n0 = g.n;
+    if (g.append_rows(points, n)) return fail(ZVDB_ERR_OUT_OF_MEMORY, "append: out of memory");
+    std::vector<uint32_t> touched;
+    bool final_started = false;
+    rc = append_locked(ix, n0, K, ef, touched, final_started);
+    if (rc) {
+        // the pre-call index: the batch's rows are dropped; once the final pass has started the device table may hold
+        // rewritten rows, which the next sync re-sends from the host
+        const std::string why = g_last_error;
+        cudaDeviceSynchronize();
+        cudaGetLastError();
+        g.truncate(n0);
+        if (final_started)
+            for (uint32_t j : touched) if (j < n0) g.mark_dirty(j);
+        return fail(rc, why);
+    }
+    // the table was linked on the device and the touched rows copied back: both sides are current
+    g.rows_uploaded = g.n;
+    ix->n_dev = g.n; ix->bf_rows = 0;
     return ZVDB_OK;
 }
 

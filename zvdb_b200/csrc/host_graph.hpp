@@ -182,6 +182,20 @@ struct HostGraph {
         if (dirty.size() > n / 4 + 4096) { adj_all_dirty = true; dirty.clear(); dirty.shrink_to_fit(); }
     }
 
+    // A caller's row as the arena holds it: dim floats, normalised once under cosine, zero padded to the row pitch.
+    void store_row(float *row, const float *src) const {
+        std::memcpy(row, src, dim * sizeof(float));
+        if (metric == 1) {
+            double s = 0.0;
+            for (uint32_t i = 0; i < dim; ++i) s += static_cast<double>(row[i]) * static_cast<double>(row[i]);
+            if (s > 0.0) {
+                const double inv = 1.0 / std::sqrt(s);
+                for (uint32_t i = 0; i < dim; ++i) row[i] = static_cast<float>(static_cast<double>(row[i]) * inv);
+            }
+        }
+        for (uint32_t i = dim; i < row_floats; ++i) row[i] = 0.0f;
+    }
+
     // insert, hnsw.zig:73-117. forced_level < 0 draws the level. `typed` (f64 / i32 indexes) is the caller's row in
     // its own element type; `pt` its f32 conversion.
     int insert(const float *pt, int forced_level, const void *typed = nullptr) {
@@ -220,18 +234,8 @@ struct HostGraph {
             adj0.resize(id * m); level.resize(id); upper_off.resize(id); upper.resize(upper_before);
             return 1;
         }
-        float *row = point_mut(id);
-        std::memcpy(row, pt, dim * sizeof(float));                               // owned copy, :24-26
-        if (metric == 1) {                                                       // cosine: normalise once
-            double s = 0.0;
-            for (uint32_t i = 0; i < dim; ++i) s += static_cast<double>(row[i]) * static_cast<double>(row[i]);
-            if (s > 0.0) {
-                const double inv = 1.0 / std::sqrt(s);
-                for (uint32_t i = 0; i < dim; ++i) row[i] = static_cast<float>(static_cast<double>(row[i]) * inv);
-            }
-        }
-        for (uint32_t i = dim; i < row_floats; ++i) row[i] = 0.0f;
-        n = id + 1;                                                              // :82
+        store_row(point_mut(id), pt);                                            // owned copy, :24-26
+        n = id + 1;                                                            // :82
         mark_dirty(id);
 
         static thread_local std::vector<uint32_t> tmp;
@@ -266,6 +270,34 @@ struct HostGraph {
         }
         if (lv > max_level) { max_level = lv; top_node = id; }                   // after the loop, :114-116
         return 0;
+    }
+
+    // The host half of zvdb_append_batch (K7, append.cuh): `count` rows become nodes n .. n+count-1 at level 0 with
+    // empty lists, stored like insert stores them (cosine: normalised once; zero padded to the row pitch). Links,
+    // entry point and upper layers are left alone: the device links the rows, and truncate(n) undoes this call.
+    int append_rows(const float *pts, uint64_t count) {
+        const uint64_t n0 = n;
+        try {
+            adj0.resize((n0 + count) * m, kInvalidId);
+            level.resize(n0 + count, 0);
+            upper_off.resize(n0 + count, ~0ull);
+        } catch (const std::bad_alloc &) { truncate(n0); return 1; }
+        const uint64_t need = (n0 + count + rows_per_chunk - 1) / rows_per_chunk;
+        while (chunks.size() < need) {
+            float *c = nullptr;
+            if (cudaHostAlloc(&c, static_cast<size_t>(rows_per_chunk) * row_floats * sizeof(float),
+                              cudaHostAllocDefault) != cudaSuccess) { cudaGetLastError(); truncate(n0); return 1; }
+            chunks.push_back(c);
+        }
+        for (uint64_t r = 0; r < count; ++r) store_row(point_mut(n0 + r), pts + r * dim);
+        n = n0 + count;
+        return 0;
+    }
+    // Back to the first n0 nodes after an append that did not complete (shrinking never throws; pinned chunks stay for
+    // the next insert).
+    void truncate(uint64_t n0) {
+        adj0.resize(n0 * m); level.resize(n0); upper_off.resize(n0);
+        n = n0;
     }
 
     // Layers >= 1 in the flat form the device (and zvdb_export_upper_layers) uses: node i has level[i]

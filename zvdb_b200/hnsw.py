@@ -216,6 +216,24 @@ class HNSW:
             L.check(L.lib().zvdb_build_from_candidates(self._h, p.ctypes.data_as(C.POINTER(C.c_float)), p.shape[0],
                                                        p.shape[1], c.ctypes.data, c.shape[1], 0))
 
+    def append_batch(self, points, K: int = 64, ef: int = 0, growth: float = 2.0) -> None:
+        """Append rows to a built index and link them on the GPU (zvdb_append_batch, K7): each row is searched on the
+        graph (K candidates, ef pops; 0 = 4 * K), linked by the builder's rules, and the old rows it links to gain it.
+        Rows of one call cannot find each other, so a large batch goes in calls of at most count * (growth - 1) rows,
+        the prefixes of the incremental builder."""
+        self._require_f32("append_batch")
+        p = np.ascontiguousarray(points, np.float32)
+        if p.ndim != 2:
+            raise ValueError("points must be [n, dim]")
+        if growth <= 1.0:
+            raise ValueError("growth must be > 1")
+        s = 0
+        while s < len(p):
+            step = max(1, int(self.count() * (growth - 1.0)))
+            e = min(len(p), s + step)
+            L.check(L.lib().zvdb_append_batch(self._h, p[s:e].ctypes.data_as(C.POINTER(C.c_float)), e - s, p.shape[1], K, ef))
+            s = e
+
     # -- upper layers and the descent (K2; extension, off = the reference's search) ----------------
     def set_descent(self, on: bool = True) -> None:
         """Walk layers max_level..1 greedily before the layer-0 search (zvdb_set_descent)."""
