@@ -155,6 +155,52 @@ ZVDB_API int zvdb_build_from_candidates(zvdb_index *ix, const float *points, uin
 ZVDB_API int zvdb_append_batch(zvdb_index *ix, const float *points, uint64_t n, uint32_t dim, uint32_t K,
                                uint32_t ef);
 
+/* ---- reachability of layer 0 (K8, zvdb_b200/csrc/connect.cuh) ----------------------------------------
+ * A search starts at the entry point and follows layer-0 edges: a row no such path reaches is never
+ * returned, not even to a query equal to it. */
+
+/* Layer-0 rows reachable from the entry point, by a breadth-first search on the device over the device
+ * table (brought up to date first). *count = how many; mask[n] (may be NULL) = 1 for a reached row, 0
+ * otherwise. Only the mask crosses PCIe. Any index type; an empty index gives *count = 0. Errors:
+ * ZVDB_ERR_INVALID (NULL ix or count). */
+ZVDB_API int zvdb_reachable(zvdb_index *ix, uint8_t *mask, uint64_t *count);
+
+typedef struct zvdb_connect_stats {
+    uint64_t reachable_before, reachable_after; /* rows reachable from the entry point before / after */
+    uint64_t attached;                          /* links added (one per attached row and round) */
+    uint64_t rows_rewritten;                    /* rows whose layer-0 list changed */
+    uint32_t rounds;                            /* rounds run (a round that attaches nothing ends the call) */
+    uint32_t searched;                          /* rows searched: those unreached before the call */
+} zvdb_connect_stats;
+
+/* Link the unreached rows of layer 0 into the graph ON THE GPU (K8), without dropping any edge of the
+ * breadth-first tree. Every distance is in the kernels' summation order, every ordering by (distance, id):
+ *   BFS. From the entry point, level by level. parent(w) = the smallest id among the nodes one level
+ *        closer that link to w. R = the reached rows.
+ *   0. U = the rows not in R (none: the call returns). Each u in U is searched once, on the graph before
+ *      the call, with the stored row (normalised under cosine), k = K and ef, as zvdb_search_batch_device
+ *      does (the handle's storage, descent and variant settings apply). C_u = the returned ids in order,
+ *      each with its returned distance.
+ *   1. A round: the BFS again; U' = the rows of U still unreached (none: stop). v is eligible when v is
+ *      in R, has accepted fewer than max_new rows in this call and none in this round, and has a free
+ *      slot or a non-tree edge v->w (parent(w) != v).
+ *   2. Matching, in passes until no proposal is made: each unmatched u of U' proposes to the first eligible
+ *      v of C_u (a candidate outside R never is) with the key (d(u,v), u); v keeps the smallest key it
+ *      receives and that u is matched to it; the others try again in the next pass.
+ *   3. Apply: u takes the first free slot of v, else the slot of the non-tree edge v->w with the largest
+ *      (d(v,w), w). No other slot moves.
+ *   4. Stop when U' is empty, when a round attaches nothing, or after max_rounds rounds. Returning early
+ *      is not an error; stats (may be NULL) say what was reached.
+ * No tree edge is ever dropped, so every row reached at the start of a round is reached at its end and
+ * the reached count grows in every round that attaches a row. Upper layers, max_level, the entry point,
+ * the descent start, the lists of the attached rows and of every row that accepted nothing do not change.
+ * ef = 0 means 4 * K, max_new = 0 means ceil(m / 4), max_rounds = 0 means 64. On success host and device
+ * copies are both current. On failure the host table is as before the call and the next search re-sends
+ * it. An empty index is a no-op. Errors: ZVDB_ERR_INVALID (ef < K), ZVDB_ERR_UNSUPPORTED (f64 / i32 index,
+ * m > 64, K outside 1..128); a refused call changes nothing. */
+ZVDB_API int zvdb_connect(zvdb_index *ix, uint32_t K, uint32_t ef, uint32_t max_new, uint32_t max_rounds,
+                          zvdb_connect_stats *stats);
+
 /* ---- upper layers and the descent (north_star subsystem 2, SURVEY 8f rank 2) ----------------------
  * The reference BUILDS layers >= 1 (hnsw.zig:88-108) but its search never reads them (hnsw.zig:216).
  * With the descent switched on, a search first walks layers max_level..1 greedily from the node that

@@ -30,6 +30,16 @@ extern fn zvdb_search_batch_typed(ix: *zvdb_index, queries: *const anyopaque, nq
 extern fn zvdb_get_point_typed(ix: *const zvdb_index, id: u64) ?*const anyopaque;
 extern fn zvdb_set_descent(ix: *zvdb_index, on: c_int) c_int;
 extern fn zvdb_append_batch(ix: *zvdb_index, points: [*]const f32, n: u64, dim: u32, K: u32, ef: u32) c_int;
+extern fn zvdb_reachable(ix: *zvdb_index, mask: ?[*]u8, count: *u64) c_int;
+pub const ConnectStats = extern struct {
+    reachable_before: u64 = 0,
+    reachable_after: u64 = 0,
+    attached: u64 = 0,
+    rows_rewritten: u64 = 0,
+    rounds: u32 = 0,
+    searched: u32 = 0,
+};
+extern fn zvdb_connect(ix: *zvdb_index, K: u32, ef: u32, max_new: u32, max_rounds: u32, stats: ?*ConnectStats) c_int;
 extern fn zvdb_set_storage(ix: *zvdb_index, storage: c_int) c_int;
 extern fn zvdb_storage(ix: *const zvdb_index) c_int;
 extern fn zvdb_save(ix: *const zvdb_index, path: [*:0]const u8) c_int;
@@ -145,6 +155,26 @@ pub fn HNSW(comptime T: type) type {
             const h = self.handle orelse return error.CudaError;
             if (n == 0) return;
             try check(zvdb_append_batch(h, points.ptr, n, @intCast(points.len / n), @intCast(K), @intCast(ef)));
+        }
+
+        /// Extension: how many layer-0 rows a search from the entry point can reach (zvdb_reachable, a BFS on the GPU);
+        /// mask (count() bytes, or null) gets 1 for each reached row. A row nobody reaches is never returned.
+        pub fn reachable(self: *Self, mask: ?[]u8) !usize {
+            const h = self.handle orelse return error.CudaError;
+            var count: u64 = 0;
+            try check(zvdb_reachable(h, if (mask) |m| m.ptr else null, &count));
+            return @intCast(count);
+        }
+
+        /// Extension: link the unreached layer-0 rows into the graph on the GPU (zvdb_connect, K8) without dropping
+        /// an edge of the BFS tree: each is searched once (K candidates, ef pops; 0 = 4 * K) and attached, round by
+        /// round, to its nearest reached candidate with a free slot or a non-tree edge. 0 = the defaults for
+        /// max_new (ceil(m / 4)) and max_rounds (64). f32 indexes only.
+        pub fn connect(self: *Self, K: usize, ef: usize, max_new: usize, max_rounds: usize) !ConnectStats {
+            const h = self.handle orelse return error.CudaError;
+            var st = ConnectStats{};
+            try check(zvdb_connect(h, @intCast(K), @intCast(ef), @intCast(max_new), @intCast(max_rounds), &st));
+            return st;
         }
 
         /// Extension: walk layers max_level..1 greedily (the walk of insert, hnsw.zig:89-104) before the

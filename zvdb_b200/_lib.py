@@ -44,6 +44,8 @@ SIGNATURES = {
     "zvdb_load_graph": (_i32, [_vp, _pf, _u64, _u32, _pu64, _pu32, _u64]),
     "zvdb_build_from_candidates": (_i32, [_vp, _pf, _u64, _u32, _vp, _u32, _i32]),
     "zvdb_append_batch": (_i32, [_vp, _pf, _u64, _u32, _u32, _u32]),
+    "zvdb_reachable": (_i32, [_vp, _vp, _pu64]),
+    "zvdb_connect": (_i32, [_vp, _u32, _u32, _u32, _u32, _vp]),
     "zvdb_set_descent": (_i32, [_vp, _i32]),
     "zvdb_descent_start": (_i64, [_vp]),
     "zvdb_set_storage": (_i32, [_vp, _i32]),
@@ -77,6 +79,12 @@ SIGNATURES = {
     "zvdb_last_error": (C.c_char_p, []),
     "zvdb_version": (C.c_char_p, []),
 }
+
+
+class ConnectStats(C.Structure):
+    """zvdb_connect_stats"""
+    _fields_ = [("reachable_before", C.c_uint64), ("reachable_after", C.c_uint64), ("attached", C.c_uint64),
+                ("rows_rewritten", C.c_uint64), ("rounds", C.c_uint32), ("searched", C.c_uint32)]
 
 
 class ZvdbError(RuntimeError):

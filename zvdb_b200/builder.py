@@ -62,9 +62,11 @@ def knn_candidates_k4(X: np.ndarray, K: int, device, metric: int = 0, chunk: int
     return out
 
 
-def build_quality_graph(h, X: np.ndarray, m: int, K: int = 64, device=None, chunk: int = 8192, source: str = "k4"):
+def build_quality_graph(h, X: np.ndarray, m: int, K: int = 64, device=None, chunk: int = 8192, source: str = "k4",
+                        connect: bool = False):
     """Fill index `h` with a graph built on the GPU from K candidates per node. source = "k4": exact candidates from the
-    repo's own brute-force kernel; "torch": round 1's bf16 library GEMM + top-k (kept for A/B)."""
+    repo's own brute-force kernel; "torch": round 1's bf16 library GEMM + top-k (kept for A/B). connect = True then
+    links the rows the entry point does not reach (h.connect(), K8) and returns its statistics."""
     import torch
     device = device or torch.device("cuda", h.device)
     K = min(K, 128, max(1, len(X)))
@@ -76,6 +78,7 @@ def build_quality_graph(h, X: np.ndarray, m: int, K: int = 64, device=None, chun
     h.build_from_candidates(X, K=K, cand_device_ptr=cand.data_ptr())
     del cand
     torch.cuda.empty_cache()
+    return h.connect() if connect else None
 
 
 def draw_levels(n: int, seed: int = 0, p: float = 0.5, cap: int = 31) -> np.ndarray:
@@ -118,7 +121,7 @@ def build_hierarchy(h, X: np.ndarray, m: int, levels=None, seed: int = 0, K: int
 
 def build_quality_graph_incremental(h, X: np.ndarray, m: int, K: int = 64, seed_rows: int = 131072, ef: int = 0,
                                     growth: float = 2.0, refine_rounds: int = 2, join: int = 0, query_chunk: int = 1 << 20,
-                                    device=None, log=None):
+                                    device=None, log=None, connect: bool = False):
     """Fill index `h` with a graph over all rows of X, built prefix by prefix: the first `seed_rows` rows from GEMM
     candidates, then each new block of rows (the prefix grows by `growth`) is SEARCHED on the current graph
     (K1, ef = K pops: the popped set is the candidate list, nearest first) and the builder kernels re-link the whole
@@ -128,6 +131,8 @@ def build_quality_graph_incremental(h, X: np.ndarray, m: int, K: int = 64, seed_
     candidates (one batched search of n queries + one builder pass per round). With `join` = J > 0 a refinement round
     also offers every row the neighbour lists of its first J neighbours (the local join of NN-descent), J * m extra
     candidates per row (K + m + J * m <= 128).
+    With `connect` the rows the entry point does not reach are then linked in (h.connect(), K8); its statistics are
+    returned under "connect".
     Cost: O(n log n) row evaluations in searches + (2 + refine_rounds) builder passes over n. Returns build statistics."""
     import time
     import torch
@@ -196,4 +201,5 @@ def build_quality_graph_incremental(h, X: np.ndarray, m: int, K: int = 64, seed_
             log(f"[builder] refinement round {r + 1} / {refine_rounds} ({time.time() - t0:.1f}s)")
     del cand
     torch.cuda.empty_cache()
-    return {"phases": phases, "refine_rounds": refine_rounds, "rows_searched": searched[0], "seconds": time.time() - t0, "K": K, "ef": ef, "join": join, "growth": growth}
+    stats = {"connect": h.connect()} if connect else {}
+    return {**stats, "phases": phases, "refine_rounds": refine_rounds, "rows_searched": searched[0], "seconds": time.time() - t0, "K": K, "ef": ef, "join": join, "growth": growth}

@@ -16,6 +16,7 @@
 #include "search_team_kernel.cuh"
 #include "builder.cuh"
 #include "append.cuh"
+#include "connect.cuh"
 #include "bruteforce.cuh"
 #include <cub/device/device_scan.cuh>
 #include <cub/device/device_select.cuh>
@@ -892,6 +893,185 @@ static int launch_bruteforce(zvdb_index *ix, const float *d_q, uint64_t nq, uint
     return ZVDB_OK;
 }
 
+// ---- K8: reachability report and repair (connect.cuh) -------------------------------------------------
+
+// BFS scratch of zvdb_reachable and K8 (connect.cuh): depth and parent per node, two frontier queues, the next
+// frontier's length. 16 bytes per node and 4.
+struct ReachScratch {
+    DevBuf<uint32_t> depth, parent, q0, q1, count;
+    ~ReachScratch() { depth.free_(); parent.free_(); q0.free_(); q1.free_(); count.free_(); }
+};
+
+// Level-synchronous BFS over the device table from the entry point (device current, n > 0): depth, parent, and the
+// reached count. One launch and one 4-byte copy back per level.
+static int reach_locked(zvdb_index *ix, ReachScratch &r, uint64_t &reached) {
+    const HostGraph &g = ix->g;
+    const uint32_t n = static_cast<uint32_t>(g.n);
+    cudaStream_t s = ix->stream;
+    ZV_CUDA(r.depth.reserve(n));
+    ZV_CUDA(r.parent.reserve(n));
+    ZV_CUDA(r.q0.reserve(n));
+    ZV_CUDA(r.q1.reserve(n));
+    ZV_CUDA(r.count.reserve(1));
+    ZV_CUDA(cudaMemsetAsync(r.depth.p, 0xFF, static_cast<size_t>(n) * sizeof(uint32_t), s));
+    ZV_CUDA(cudaMemsetAsync(r.parent.p, 0xFF, static_cast<size_t>(n) * sizeof(uint32_t), s));
+    bfs_seed_kernel<<<1, 1, 0, s>>>(r.depth.p, r.q0.p, static_cast<uint32_t>(g.entry)); ix->launches++;
+    ZV_CUDA(cudaGetLastError());
+    uint32_t *cur = r.q0.p, *next = r.q1.p;
+    uint32_t count = 1;
+    reached = 1;
+    for (uint32_t level = 0; count != 0; ++level) {
+        ZV_CUDA(cudaMemsetAsync(r.count.p, 0, sizeof(uint32_t), s));
+        const uint64_t total = static_cast<uint64_t>(count) * g.m;
+        const unsigned blocks = static_cast<unsigned>(std::min<uint64_t>((total + 255) / 256, 148ull * 16));
+        bfs_level_kernel<<<blocks, 256, 0, s>>>(ix->d_adj, g.m, n, cur, count, level, r.depth.p, r.parent.p, next, r.count.p);
+        ix->launches++;
+        ZV_CUDA(cudaGetLastError());
+        ZV_CUDA(cudaMemcpyAsync(&count, r.count.p, sizeof count, cudaMemcpyDeviceToHost, s));
+        ZV_CUDA(cudaStreamSynchronize(s));
+        reached += count;
+        std::swap(cur, next);
+    }
+    return ZVDB_OK;
+}
+
+// K8 scratch beyond the BFS: U and its search, the per-node matching state, the per-row-of-U cursors.
+struct ConnectScratch {
+    DevBuf<float> q, dist;
+    DevBuf<uint64_t> ids, best;
+    DevBuf<uint32_t> unreached, cnt, accepted, cursor, target, won, counters, rows, touched;
+    DevBuf<uint8_t> eligible, tmp;
+    ~ConnectScratch() {
+        q.free_(); dist.free_(); ids.free_(); best.free_(); unreached.free_(); cnt.free_(); accepted.free_(); cursor.free_();
+        target.free_(); won.free_(); counters.free_(); rows.free_(); touched.free_(); eligible.free_(); tmp.free_();
+    }
+};
+
+// rows[0..count) = the ids v < n with pred(v), ascending (CUB select over the node ids); returns count.
+template <typename Pred>
+static int select_rows(uint32_t n, Pred pred, DevBuf<uint32_t> &out, DevBuf<uint8_t> &tmp, uint32_t &count, zvdb_index *ix) {
+    cudaStream_t s = ix->stream;
+    ZV_CUDA(out.reserve(static_cast<size_t>(n) + 1));      // + the select's count word
+    uint32_t *d_nsel = out.p + n;
+    const thrust::counting_iterator<uint32_t> node_ids(0);
+    size_t bytes = 0;
+    ZV_CUDA(cub::DeviceSelect::If(nullptr, bytes, node_ids, out.p, d_nsel, static_cast<int64_t>(n), pred, s));
+    ZV_CUDA(tmp.reserve(std::max<size_t>(bytes, 1)));
+    ZV_CUDA(cub::DeviceSelect::If(tmp.p, bytes, node_ids, out.p, d_nsel, static_cast<int64_t>(n), pred, s));
+    ix->launches++;
+    ZV_CUDA(cudaMemcpyAsync(&count, d_nsel, sizeof count, cudaMemcpyDeviceToHost, s));
+    ZV_CUDA(cudaStreamSynchronize(s));
+    return ZVDB_OK;
+}
+
+// K8 on a non-empty f32 index whose device copy is current (connect.cuh). applied is set once the first apply kernel
+// is enqueued: from then on the device table may differ from the host's.
+static int connect_locked(zvdb_index *ix, uint32_t K, uint32_t ef, uint32_t max_new, uint32_t max_rounds,
+                          zvdb_connect_stats &st, bool &applied) {
+    HostGraph &g = ix->g;
+    const uint32_t n = static_cast<uint32_t>(g.n);
+    cudaStream_t s = ix->stream;
+    ReachScratch r;
+    ConnectScratch c;
+    uint64_t reached = 0;
+    int rc = reach_locked(ix, r, reached);
+    if (rc) return rc;
+    st.reachable_before = st.reachable_after = reached;
+    if (reached == n) return ZVDB_OK;
+    // 0. U and one search of each of its rows on the graph before the call
+    uint32_t nu = 0;
+    rc = select_rows(n, UnreachedRow{r.depth.p}, c.unreached, c.tmp, nu, ix);
+    if (rc) return rc;
+    st.searched = nu;
+    ZV_CUDA(c.q.reserve(static_cast<size_t>(nu) * g.dim));
+    const unsigned qblocks = static_cast<unsigned>(std::min<uint64_t>((static_cast<uint64_t>(nu) * g.dim + 255) / 256, 148ull * 8));
+    gather_query_rows_kernel<<<qblocks, 256, 0, s>>>(c.q.p, ix->d_arena, g.row_floats, c.unreached.p, nu, g.dim); ix->launches++;
+    ZV_CUDA(cudaGetLastError());
+    ZV_CUDA(c.ids.reserve(static_cast<size_t>(nu) * K));
+    ZV_CUDA(c.dist.reserve(static_cast<size_t>(nu) * K));
+    ZV_CUDA(c.cnt.reserve(nu));
+    for (uint64_t q0 = 0; q0 < nu; q0 += 0x7FFFFFFFull) {   // launch_search's per-launch query limit
+        const uint64_t cnt = std::min<uint64_t>(nu - q0, 0x7FFFFFFFull);
+        rc = launch_search(ix, c.q.p + q0 * g.dim, cnt, K, ef, c.ids.p + q0 * K, c.dist.p + q0 * K, c.cnt.p + q0, nullptr, nullptr,
+                           1, 0, s);
+        if (rc) return rc;
+    }
+    c.q.free_();
+    // the matching state
+    ZV_CUDA(c.accepted.reserve(n));
+    ZV_CUDA(c.eligible.reserve(n));
+    ZV_CUDA(c.best.reserve(n));
+    ZV_CUDA(c.cursor.reserve(nu));
+    ZV_CUDA(c.target.reserve(nu));
+    ZV_CUDA(c.won.reserve(nu));
+    ZV_CUDA(c.counters.reserve(2));
+    ZV_CUDA(cudaMemsetAsync(c.accepted.p, 0, static_cast<size_t>(n) * sizeof(uint32_t), s));
+    ConnectParams cp{};
+    cp.arena = reinterpret_cast<const float4 *>(ix->d_arena);
+    cp.row_chunks = g.row_floats / 4; cp.n = n; cp.m = g.m; cp.adj = ix->d_adj;
+    cp.depth = r.depth.p; cp.parent = r.parent.p; cp.unreached = c.unreached.p; cp.nu = nu;
+    cp.cand = c.ids.p; cp.cand_dist = c.dist.p; cp.K = K; cp.max_new = max_new;
+    cp.accepted = c.accepted.p; cp.eligible = c.eligible.p; cp.best = c.best.p; cp.cursor = c.cursor.p; cp.target = c.target.p;
+    cp.won = c.won.p; cp.counters = c.counters.p;
+    const unsigned nblocks = static_cast<unsigned>(std::min<uint64_t>((n + 255) / 256, 148ull * 16));
+    const unsigned ublocks = static_cast<unsigned>(std::min<uint64_t>((nu + 255) / 256, 148ull * 16));
+    const int cpl = cpl_for(g.row_floats);
+    // rounds; the BFS of the first round is the one above (nothing has changed since)
+    while (st.rounds < max_rounds && reached < n) {
+        ++st.rounds;
+        ZV_CUDA(cudaMemsetAsync(c.counters.p + 1, 0, sizeof(uint32_t), s));
+        connect_eligible_kernel<<<nblocks, 256, 0, s>>>(cp); ix->launches++;
+        ZV_CUDA(cudaGetLastError());
+        connect_open_kernel<<<ublocks, 256, 0, s>>>(cp); ix->launches++;
+        ZV_CUDA(cudaGetLastError());
+        for (;;) {                                           // matching passes until nobody proposes
+            uint32_t proposals = 0;
+            ZV_CUDA(cudaMemsetAsync(c.counters.p, 0, sizeof(uint32_t), s));
+            connect_propose_kernel<<<ublocks, 256, 0, s>>>(cp); ix->launches++;
+            ZV_CUDA(cudaGetLastError());
+            ZV_CUDA(cudaMemcpyAsync(&proposals, c.counters.p, sizeof proposals, cudaMemcpyDeviceToHost, s));
+            ZV_CUDA(cudaStreamSynchronize(s));
+            if (proposals == 0) break;
+            connect_resolve_kernel<<<ublocks, 256, 0, s>>>(cp); ix->launches++;
+            ZV_CUDA(cudaGetLastError());
+        }
+        uint32_t nw = 0;
+        ZV_CUDA(cudaMemcpyAsync(&nw, c.counters.p + 1, sizeof nw, cudaMemcpyDeviceToHost, s));
+        ZV_CUDA(cudaStreamSynchronize(s));
+        if (nw == 0) break;                                  // nothing attached: no later round would differ
+        applied = true;
+        cudaError_t e = dispatch(g.metric, cpl, [&](auto fm) {
+            using Fm = decltype(fm);
+            return launch_kernel(connect_apply_kernel<Fm::cpl, Fm::metric>, nw, 32, 0, s, cp);
+        });
+        ix->launches++;
+        ZV_CUDA(e);
+        st.attached += nw;
+        rc = reach_locked(ix, r, reached);
+        if (rc) return rc;
+        st.reachable_after = reached;
+    }
+    if (!applied) return ZVDB_OK;
+    // the rewritten rows back: select, gather on the device, one copy, scatter into the host table
+    uint32_t nt = 0;
+    rc = select_rows(n, AcceptedRow{c.accepted.p}, c.touched, c.tmp, nt, ix);
+    if (rc) return rc;
+    st.rows_rewritten = nt;
+    std::vector<uint32_t> touched, rows;
+    try { touched.resize(nt); rows.resize(static_cast<size_t>(nt) * g.m); }
+    catch (const std::bad_alloc &) { return fail(ZVDB_ERR_OUT_OF_MEMORY, "connect: out of memory"); }
+    ZV_CUDA(c.rows.reserve(std::max<size_t>(rows.size(), 1)));
+    const unsigned gblocks = static_cast<unsigned>(std::min<uint64_t>((rows.size() + 255) / 256 + 1, 148ull * 8));
+    gather_adj_rows_kernel<<<gblocks, 256, 0, s>>>(c.rows.p, ix->d_adj, c.touched.p, nt, g.m); ix->launches++;
+    ZV_CUDA(cudaGetLastError());
+    ZV_CUDA(cudaMemcpyAsync(touched.data(), c.touched.p, nt * sizeof(uint32_t), cudaMemcpyDeviceToHost, s));
+    ZV_CUDA(cudaMemcpyAsync(rows.data(), c.rows.p, rows.size() * sizeof(uint32_t), cudaMemcpyDeviceToHost, s));
+    ZV_CUDA(cudaStreamSynchronize(s));
+    for (uint32_t t = 0; t < nt; ++t)
+        std::memcpy(g.adj0.data() + static_cast<size_t>(touched[t]) * g.m, rows.data() + static_cast<size_t>(t) * g.m, g.m * sizeof(uint32_t));
+    return ZVDB_OK;
+}
+
 }  // namespace zvdb
 
 // ================================ exported C ABI ================================================
@@ -1654,6 +1834,65 @@ int zvdb_append_batch(zvdb_index *ix, const float *points, uint64_t n, uint32_t 
     // the table was linked on the device and the touched rows copied back: both sides are current
     g.rows_uploaded = g.n;
     ix->n_dev = g.n; ix->bf_rows = 0;
+    return ZVDB_OK;
+}
+
+int zvdb_reachable(zvdb_index *ix, uint8_t *mask, uint64_t *count) {
+    if (!ix || !count) return fail(ZVDB_ERR_INVALID, "null argument");
+    std::lock_guard<std::mutex> lk(ix->mu);
+    const HostGraph &g = ix->g;
+    *count = 0;
+    if (g.n == 0 || !g.has_entry) return ZVDB_OK;
+    ZV_CUDA(cudaSetDevice(ix->device));
+    int rc = sync_device_locked(ix);
+    if (rc) return rc;
+    ReachScratch r;
+    uint64_t reached = 0;
+    rc = reach_locked(ix, r, reached);
+    if (rc) return rc;
+    if (mask) {
+        DevBuf<uint8_t> d_mask;
+        struct Cleanup { DevBuf<uint8_t> &m; ~Cleanup() { m.free_(); } } cleanup{d_mask};
+        ZV_CUDA(d_mask.reserve(g.n));
+        const unsigned blocks = static_cast<unsigned>(std::min<uint64_t>((g.n + 255) / 256, 148ull * 16));
+        reach_mask_kernel<<<blocks, 256, 0, ix->stream>>>(r.depth.p, g.n, d_mask.p); ix->launches++;
+        ZV_CUDA(cudaGetLastError());
+        ZV_CUDA(cudaMemcpyAsync(mask, d_mask.p, g.n, cudaMemcpyDeviceToHost, ix->stream));
+        ZV_CUDA(cudaStreamSynchronize(ix->stream));
+    }
+    *count = reached;
+    return ZVDB_OK;
+}
+
+int zvdb_connect(zvdb_index *ix, uint32_t K, uint32_t ef, uint32_t max_new, uint32_t max_rounds, zvdb_connect_stats *stats) {
+    if (!ix) return fail(ZVDB_ERR_INVALID, "null index");
+    if (K == 0 || K > kBuildBuf) return fail(ZVDB_ERR_UNSUPPORTED, "connect: K must be in 1..128");
+    if (ef == 0) ef = 4 * K;
+    if (ef < K) return fail(ZVDB_ERR_INVALID, "connect: ef must be >= K (0 = 4 * K)");
+    std::lock_guard<std::mutex> lk(ix->mu);
+    HostGraph &g = ix->g;
+    if (g.dtype != 0) return fail(ZVDB_ERR_UNSUPPORTED, "connect: f64 / i32 indexes are not supported");
+    if (g.m > 64) return fail(ZVDB_ERR_UNSUPPORTED, "connect: m must be <= 64");
+    zvdb_connect_stats st{};
+    if (max_new == 0) max_new = (g.m + 3) / 4;
+    if (max_rounds == 0) max_rounds = 64;
+    if (g.n > 0 && g.has_entry) {
+        ZV_CUDA(cudaSetDevice(ix->device));
+        int rc = sync_device_locked(ix);                  // the device holds the graph before the call
+        if (rc) return rc;
+        ZV_CUDA(cudaDeviceSynchronize());                 // searches enqueued on caller streams may still read the table
+        bool applied = false;
+        rc = connect_locked(ix, K, ef, max_new, max_rounds, st, applied);
+        if (rc) {
+            // the host table is the pre-call one; once a row was rewritten on the device the next sync re-sends the table
+            const std::string why = g_last_error;
+            cudaDeviceSynchronize();
+            cudaGetLastError();
+            if (applied) g.adj_all_dirty = true;
+            return fail(rc, why);
+        }
+    }
+    if (stats) *stats = st;
     return ZVDB_OK;
 }
 

@@ -234,6 +234,24 @@ class HNSW:
             L.check(L.lib().zvdb_append_batch(self._h, p[s:e].ctypes.data_as(C.POINTER(C.c_float)), e - s, p.shape[1], K, ef))
             s = e
 
+    # -- reachability of layer 0 (K8) -------------------------------------------------------------
+    def reachable(self):
+        """(mask, count): mask[i] = True when layer-0 row i is reachable from the entry point, so that a search can
+        return it; count = mask.sum() (zvdb_reachable, a BFS on the device)."""
+        mask = np.zeros(self.count(), np.uint8)
+        cnt = C.c_uint64(0)
+        L.check(L.lib().zvdb_reachable(self._h, mask.ctypes.data if len(mask) else None, C.byref(cnt)))
+        return mask.astype(bool), int(cnt.value)
+
+    def connect(self, K: int = 64, ef: int = 0, max_new: int = 0, max_rounds: int = 0) -> dict:
+        """Link the rows the entry point does not reach into layer 0 on the GPU (zvdb_connect, K8): each is searched
+        once (K candidates, ef pops; 0 = 4 * K) and attached, round by round, to its nearest reached candidate that
+        has a free slot or an edge outside the BFS tree; no tree edge is dropped. max_new (0 = ceil(m / 4)) caps the
+        rows one node accepts, max_rounds (0 = 64) the rounds. Returns the call's statistics."""
+        st = L.ConnectStats()
+        L.check(L.lib().zvdb_connect(self._h, K, ef, max_new, max_rounds, C.byref(st)))
+        return {name: int(getattr(st, name)) for name, _ in L.ConnectStats._fields_}
+
     # -- upper layers and the descent (K2; extension, off = the reference's search) ----------------
     def set_descent(self, on: bool = True) -> None:
         """Walk layers max_level..1 greedily before the layer-0 search (zvdb_set_descent)."""
