@@ -78,8 +78,8 @@ struct zvdb_index {
     uint32_t *mailbox_dev = nullptr; // set around the single-query launch: device address of the staging block's completion word ...
     uint32_t mailbox_seq = 0;        // ... the value the kernel writes there ...
     bool mailbox_armed = false;      // ... and whether the launch took it (only the one-CTA-per-query kernel does)
-    float *d_arena = nullptr;       // [cap_rows][row_floats]
-    uint32_t *d_adj = nullptr;      // [cap_rows][m]
+    DevBuf<float> d_arena;          // [cap_rows][row_floats]
+    DevBuf<uint32_t> d_adj;         // [cap_rows][m]
     uint64_t cap_rows = 0, n_dev = 0;
     uint32_t cap_row_floats = 0, cap_m = 0;   // row layout d_arena / d_adj were sized for (a load may change dim)
     int storage = ZVDB_STORAGE_F32; // rows the graph search gathers (zvdb_set_storage)
@@ -131,26 +131,34 @@ static int ensure_capacity(zvdb_index *ix, uint64_t rows) {
     if (same_layout && rows <= ix->cap_rows) return ZVDB_OK;
     if (!same_layout) {                                   // nothing on the device is reusable
         ZV_CUDA(cudaDeviceSynchronize());
-        cudaFree(ix->d_arena); cudaFree(ix->d_adj);
-        ix->d_arena = nullptr; ix->d_adj = nullptr; ix->cap_rows = 0;
+        ix->d_arena.free_(); ix->d_adj.free_(); ix->cap_rows = 0;
         ix->cap_row_floats = g.row_floats; ix->cap_m = g.m;
         forget_device_rows(ix);                           // (a new row pitch: the next SQ8 search trains a codebook for it)
     }
     int rc = ix->row_copy.drop();
     if (rc) return rc;
     uint64_t nc = std::max<uint64_t>(rows, std::max<uint64_t>(ix->cap_rows * 2, 1024));
-    float *na = nullptr; uint32_t *nj = nullptr;
-    ZV_CUDA(cudaMalloc(&na, nc * g.row_floats * sizeof(float)));
-    cudaError_t e = cudaMalloc(&nj, nc * g.m * sizeof(uint32_t));
-    if (e != cudaSuccess) { cudaFree(na); ZV_CUDA(e); }
+    DevBuf<float> na;
+    DevBuf<uint32_t> nj;
+    ZV_CUDA(na.reserve(nc * g.row_floats));
+    ZV_CUDA(nj.reserve(nc * g.m));
     if (ix->n_dev) {
-        ZV_CUDA(cudaMemcpyAsync(na, ix->d_arena, ix->n_dev * g.row_floats * sizeof(float), cudaMemcpyDeviceToDevice, ix->stream));
-        ZV_CUDA(cudaMemcpyAsync(nj, ix->d_adj, ix->n_dev * g.m * sizeof(uint32_t), cudaMemcpyDeviceToDevice, ix->stream));
+        ZV_CUDA(cudaMemcpyAsync(na.p, ix->d_arena.p, ix->n_dev * g.row_floats * sizeof(float), cudaMemcpyDeviceToDevice, ix->stream));
+        ZV_CUDA(cudaMemcpyAsync(nj.p, ix->d_adj.p, ix->n_dev * g.m * sizeof(uint32_t), cudaMemcpyDeviceToDevice, ix->stream));
         ZV_CUDA(cudaStreamSynchronize(ix->stream));
     }
-    cudaFree(ix->d_arena); cudaFree(ix->d_adj);
-    ix->d_arena = na; ix->d_adj = nj; ix->cap_rows = nc;
+    ix->d_arena = std::move(na); ix->d_adj = std::move(nj); ix->cap_rows = nc;
     return ZVDB_OK;
+}
+
+// Arena rows [r0, r1) of the host graph to the device (ensure_capacity done), enqueued on the handle's stream.
+static int upload_rows(zvdb_index *ix, uint64_t r0, uint64_t r1) {
+    const HostGraph &g = ix->g;
+    return g.for_each_span(r0, r1, [&](uint64_t r, uint64_t end) -> int {
+        ZV_CUDA(cudaMemcpyAsync(ix->d_arena.p + r * g.row_floats, g.point(r), (end - r) * g.row_floats * sizeof(float),
+                                cudaMemcpyHostToDevice, ix->stream));
+        return ZVDB_OK;
+    });
 }
 
 // Bring the device copy up to date with the host graph: new arena rows are appended, layer-0 rows
@@ -165,15 +173,10 @@ static int sync_device_locked(zvdb_index *ix) {
     int rc = ensure_capacity(ix, g.n);
     if (rc) return rc;
     ix->row_copy.clamp(g.rows_uploaded);                 // rows from rows_uploaded on are (re)written now
-    for (uint64_t r = g.rows_uploaded; r < g.n;) {
-        const uint64_t chunk = r / g.rows_per_chunk;
-        const uint64_t end = std::min<uint64_t>(g.n, (chunk + 1) * g.rows_per_chunk);
-        ZV_CUDA(cudaMemcpyAsync(ix->d_arena + r * g.row_floats, g.point(r), (end - r) * g.row_floats * sizeof(float),
-                                cudaMemcpyHostToDevice, ix->stream));
-        r = end;
-    }
+    rc = upload_rows(ix, g.rows_uploaded, g.n);
+    if (rc) return rc;
     if (g.adj_all_dirty || g.dirty.size() * 8 > g.n) {
-        ZV_CUDA(cudaMemcpyAsync(ix->d_adj, g.adj0.data(), g.n * g.m * sizeof(uint32_t), cudaMemcpyHostToDevice, ix->stream));
+        ZV_CUDA(cudaMemcpyAsync(ix->d_adj.p, g.adj0.data(), g.n * g.m * sizeof(uint32_t), cudaMemcpyHostToDevice, ix->stream));
     } else if (!g.dirty.empty()) {
         std::sort(g.dirty.begin(), g.dirty.end());
         g.dirty.erase(std::unique(g.dirty.begin(), g.dirty.end()), g.dirty.end());
@@ -187,7 +190,7 @@ static int sync_device_locked(zvdb_index *ix) {
         ZV_CUDA(cudaMemcpyAsync(ix->scat_ids.p, g.dirty.data(), cnt * sizeof(uint32_t), cudaMemcpyHostToDevice, ix->stream));
         const uint64_t total = cnt * g.m;
         const unsigned blocks = static_cast<unsigned>(std::min<uint64_t>((total + 255) / 256, 148ull * 8));
-        scatter_adj_rows_kernel<<<blocks, 256, 0, ix->stream>>>(ix->d_adj, ix->scat_rows.p, ix->scat_ids.p,
+        scatter_adj_rows_kernel<<<blocks, 256, 0, ix->stream>>>(ix->d_adj.p, ix->scat_rows.p, ix->scat_ids.p,
                                                                 static_cast<uint32_t>(cnt), g.m);
         ix->launches++;
         ZV_CUDA(cudaGetLastError());
@@ -331,15 +334,26 @@ static int refuse_row_form(int rowf, uint32_t row_floats, bool exch) {
     return fail(ZVDB_ERR_UNSUPPORTED, "sq8 storage: built for rows of up to 768 dimensions; set ZVDB_STORAGE_F32 or ZVDB_STORAGE_F16");
 }
 
-// Where the exact visited set of a search with pop budget `ef` lives (see launch_search).
-static int plan_visited(const zvdb_index *ix, uint32_t ef) {
+// One-warp CTAs of `smem` bytes of shared memory resident per SM, at most 32.
+static uint64_t ctas_for(uint64_t smem) { return std::min<uint64_t>(32, (227ull * 1024) / (smem + 1024)); }
+
+// The exact visited set of a search with pop budget `ef`: its sizes, and where it lives (see launch_search).
+struct VisitedPlan {
+    uint64_t bound;        // visited-set maximum
+    uint64_t slots, hash_words;
+    uint64_t cand_cap;     // >= ef, even (alignment), reused by the final sort
+    uint64_t smem_lists, smem_hash;
+    int vis;
+};
+static VisitedPlan plan_visited(const zvdb_index *ix, uint32_t ef) {
     const HostGraph &g = ix->g;
-    const uint64_t bound = std::min<uint64_t>(g.n, 1ull + static_cast<uint64_t>(ef) * g.m);
-    const uint64_t slots = bound + bound / 4 + 16;
-    const uint64_t cand_cap = std::max<uint64_t>(2, next_pow2(ef));
-    const uint64_t smem_lists = (((static_cast<uint64_t>(ef) + 1) & ~1ull) + cand_cap) * 8 + kPoolCap * 8 + 32 * 4 + kPoolCap * 4 + 16;
-    const uint64_t smem_hash = smem_lists + slots * 4;
-    const uint64_t ctas = std::min<uint64_t>(32, (227ull * 1024) / (smem_hash + 1024));
+    VisitedPlan v;
+    v.bound = std::max<uint64_t>(1, std::min<uint64_t>(g.n, 1ull + static_cast<uint64_t>(ef) * g.m));
+    v.slots = v.bound + v.bound / 4 + 16;
+    v.hash_words = (v.slots + 3) & ~3ull;                 // tables are wiped 16 bytes at a time
+    v.cand_cap = std::max<uint64_t>(2, next_pow2(ef));
+    v.smem_lists = (((static_cast<uint64_t>(ef) + 1) & ~1ull) + v.cand_cap) * 8 + kPoolCap * 8 + 32 * 4 + kPoolCap * 4 + 16;
+    v.smem_hash = v.smem_lists + v.slots * 4;
     // On chip while that still leaves >= 20 queries per SM. Beyond that, in global memory, per resident CTA: the n-bit
     // bitmap (one atomicOr per neighbour, never a second probe: the fastest form measured, profiles/r02_k1_visited_ab.jsonl)
     // while the bitmaps of all resident CTAs fit a 32 GiB scratch budget (n <= 58 M rows at full residency: 7.4 GB next to
@@ -348,40 +362,20 @@ static int plan_visited(const zvdb_index *ix, uint32_t ef) {
     // ef * m (40 KB per CTA at ef = 512 whatever n is, but 15-45 % slower: probes past the first slot are extra L2 round
     // trips on a pop's critical path) for larger shards and tighter devices.
     const uint64_t bitmap_bytes = (g.n + 31) / 32 * 4 * 32ull * static_cast<uint64_t>(ix->num_sms);
-    int vis = (smem_hash <= ix->smem_optin && ctas >= 20) ? kVisSmemHash
-            : ((bitmap_bytes <= (32ull << 30) && !ix->bitmap_oom) ? kVisGlobalBitmap : kVisGlobalHash);
-    if (ix->visited_mode == 1) vis = kVisSmemHash;
-    if (ix->visited_mode == 2) vis = kVisGlobalBitmap;
-    if (ix->visited_mode == 3) vis = kVisGlobalHash;
-    return vis;
+    v.vis = (v.smem_hash <= ix->smem_optin && ctas_for(v.smem_hash) >= 20) ? kVisSmemHash
+          : ((bitmap_bytes <= (32ull << 30) && !ix->bitmap_oom) ? kVisGlobalBitmap : kVisGlobalHash);
+    if (ix->visited_mode == 1) v.vis = kVisSmemHash;
+    if (ix->visited_mode == 2) v.vis = kVisGlobalBitmap;
+    if (ix->visited_mode == 3) v.vis = kVisGlobalHash;
+    return v;
 }
 
-// The receiving side of a fused sharded step (zvdb_search_batch_exchange): see SearchParams.
-struct FusedExchange {
-    uint32_t *peer_qflags[8];
-    const uint32_t *qflags;
-    const uint8_t *gather;
-    uint64_t block_bytes;
-    uint64_t *m_ids; float *m_dist; uint32_t *m_counts;
-    uint32_t world, rank, epoch;
-    // record form (128-byte self-validating lines): ll_lines > 0
-    uint8_t *peer_ll[8] = {};
-    const uint8_t *ll_local = nullptr;
-    uint32_t ll_lines = 0, ll_pitch = 0, ll_nq = 0;
-    // gather-to-owner (zvdb_search_batch_exchange_host): q_per > 0
-    uint32_t q_per = 0;
-    const float *peer_q[8] = {};
-    uint32_t *peer_sflags[8] = {};
-    const uint32_t *sflags = nullptr;
-    uint32_t sflag_pitch = 0;
-};
-
 // Device buffers in, device buffers out, no synchronisation. Caller holds the lock and has synced
-// the device copy.
+// the device copy. exch = a sharded step: its exchange section of SearchParams (peer_blocks / n_peers, and for the
+// fused step everything from peer_qflags on that launch_search does not size itself), the rest is filled here.
 static int launch_search(zvdb_index *ix, const float *d_q, uint64_t nq, uint32_t k, uint32_t ef, uint64_t *d_ids,
                          float *d_dist, uint32_t *d_counts, uint32_t *d_pops, uint32_t *d_evals, uint64_t id_stride,
-                         uint64_t id_base, cudaStream_t s, uint8_t *const *peer_blocks = nullptr, uint32_t n_peers = 0,
-                         const FusedExchange *fx = nullptr) {
+                         uint64_t id_base, cudaStream_t s, const SearchParams *exch = nullptr) {
     const HostGraph &g = ix->g;
     if (nq == 0) return ZVDB_OK;
     if (nq > 0x7FFFFFFFull) return fail(ZVDB_ERR_UNSUPPORTED, "nq exceeds 2^31-1 queries per launch");
@@ -389,22 +383,20 @@ static int launch_search(zvdb_index *ix, const float *d_q, uint64_t nq, uint32_t
     // arena. The row format is the storage value.
     static_assert(ZVDB_STORAGE_F16 == kRowF16 && ZVDB_STORAGE_SQ8 == kRowSQ8, "storage values name the row formats");
     const int rowf = g.n > 0 ? ix->storage : kRowF32;
-    const bool exch = n_peers != 0 || fx != nullptr;
-    if (int rcr = refuse_row_form(rowf, g.row_floats, exch)) return rcr;
+    if (int rcr = refuse_row_form(rowf, g.row_floats, exch != nullptr)) return rcr;
     if (rowf != kRowF32) {
-        int rcf = ix->row_copy.sync(rowf, g, ix->d_arena, ix->n_dev, ix->cap_rows, ix->num_sms, ix->stream, ix->launches);
+        int rcf = ix->row_copy.sync(rowf, g, ix->d_arena.p, ix->n_dev, ix->cap_rows, ix->num_sms, ix->stream, ix->launches);
         if (rcf) return rcf;
     }
-    SearchParams p{};
-    p.arena = reinterpret_cast<const float4 *>(ix->d_arena);
+    SearchParams p = exch ? *exch : SearchParams{};
+    const bool fused = p.ex_world != 0;
+    p.arena = reinterpret_cast<const float4 *>(ix->d_arena.p);
     p.arena16 = rowf == kRowF16 ? ix->row_copy.search_rows<kRowF16>(g.row_floats) : nullptr;
     p.arena8 = rowf == kRowSQ8 ? ix->row_copy.search_rows<kRowSQ8>(g.row_floats) : nullptr;
-    p.adj = ix->d_adj;
+    p.adj = ix->d_adj.p;
     p.queries = d_q;
     p.ids = d_ids; p.dist = d_dist; p.counts = d_counts; p.pops = d_pops; p.evals = d_evals;
     p.id_stride = id_stride; p.id_base = id_base;
-    p.n_peers = n_peers;
-    for (uint32_t i = 0; i < n_peers && i < 8; ++i) p.peer_blocks[i] = peer_blocks[i];
     p.row_chunks = g.row_floats / 4;
     p.m = g.m; p.n = static_cast<uint32_t>(g.n); p.entry = static_cast<uint32_t>(g.entry); p.dim = g.dim;
     p.nq = static_cast<uint32_t>(nq); p.k = k; p.ef = ef;
@@ -423,12 +415,7 @@ static int launch_search(zvdb_index *ix, const float *d_q, uint64_t nq, uint32_t
     if (p.row_chunks > 8 * 32) return fail(ZVDB_ERR_UNSUPPORTED, "dim > 1024 is not built into the search kernel");
     const int cpl = cpl_for(p.row_chunks * 4);
 
-    const uint64_t bound = std::max<uint64_t>(1, std::min<uint64_t>(g.n, 1ull + static_cast<uint64_t>(ef) * g.m));   // visited-set maximum
-    const uint64_t slots = bound + bound / 4 + 16;
-    const uint64_t hash_words = (slots + 3) & ~3ull;                   // tables are wiped 16 bytes at a time
-    const uint64_t cand_cap = std::max<uint64_t>(2, next_pow2(ef));   // >= ef, even (alignment), reused by the final sort
-    const uint64_t smem_lists = (((static_cast<uint64_t>(ef) + 1) & ~1ull) + cand_cap) * 8 + kPoolCap * 8 + 32 * 4 + kPoolCap * 4 + 16;
-    const uint64_t smem_hash = smem_lists + slots * 4;
+    const VisitedPlan v = plan_visited(ix, ef);
     // K1L: a small plain batch gets one CTA per query (search_team_kernel.cuh: the latency form, same results bit for bit).
     // Automatic while every query of the batch finds a resident CTA at once: full teams (256 threads) with the per-slot
     // adjacency cache when that fits (82 KB per query at ef = 64, m = 16: 2 per SM), full teams without it (3 per SM), then
@@ -436,12 +423,12 @@ static int launch_search(zvdb_index *ix, const float *d_q, uint64_t nq, uint32_t
     // (profiles/r02_c5_team_sweep.jsonl). team_mode 1 / 2 / 3 = never / full teams whenever the shape fits / half teams.
     // (A forced visited-set or prefetch variant is a request for the one-warp kernel: those knobs exist only there.)
     const bool team_auto = ix->team_mode == 0 && ix->visited_mode == 0 && ix->prefetch_mode == 0;
-    if (!fx && n_peers == 0 && g.n > 0 && ef > 0 && (team_auto || ix->team_mode >= 2)) {
+    if (!exch && g.n > 0 && ef > 0 && (team_auto || ix->team_mode >= 2)) {
         const uint32_t ucpl = static_cast<uint32_t>(cpl);
         const uint64_t cap256 = team_cand_cap(ef, g.m, 256), cap128 = team_cand_cap(ef, g.m, 128);
-        const uint64_t smem_plain = team_smem_bytes(cap256, ef, hash_words, ucpl, g.m, false);
-        const uint64_t smem_cache = team_smem_bytes(cap256, ef, hash_words, ucpl, g.m, true);
-        const uint64_t smem_half = team_smem_bytes(cap128, ef, hash_words, ucpl, g.m, false);
+        const uint64_t smem_plain = team_smem_bytes(cap256, ef, v.hash_words, ucpl, g.m, false);
+        const uint64_t smem_cache = team_smem_bytes(cap256, ef, v.hash_words, ucpl, g.m, true);
+        const uint64_t smem_half = team_smem_bytes(cap128, ef, v.hash_words, ucpl, g.m, false);
         const uint64_t regs256 = cpl <= 1 ? 3 : (cpl <= 4 ? 2 : 1);              // 256 threads x 62-78 / 80-128 / 164+ registers
         const uint64_t regs128 = cpl <= 1 ? 7 : (cpl <= 2 ? 6 : (cpl <= 4 ? 4 : 2));   // 128 threads x 72 / 82 / 118 / 194 registers
         auto resident = [&](uint64_t smem, uint64_t by_regs) { return std::min<uint64_t>(by_regs, (227ull * 1024) / (smem + 1024)) * ix->num_sms; };
@@ -464,7 +451,7 @@ static int launch_search(zvdb_index *ix, const float *d_q, uint64_t nq, uint32_t
                 ix->launches++;
                 ZV_CUDA(e);
             }
-            p.slots = static_cast<uint32_t>(slots); p.hash_words = static_cast<uint32_t>(hash_words);
+            p.slots = static_cast<uint32_t>(v.slots); p.hash_words = static_cast<uint32_t>(v.hash_words);
             p.cand_cap = static_cast<uint32_t>(team_cap);
             if (ix->mailbox_dev && nq == 1) { p.done_flag = ix->mailbox_dev; p.done_seq = ix->mailbox_seq; ix->mailbox_armed = true; }
             e = launch_team(rowf, g.metric, cpl, adjc, threads, p, static_cast<unsigned>(nq), static_cast<size_t>(team_smem), s);
@@ -476,28 +463,27 @@ static int launch_search(zvdb_index *ix, const float *d_q, uint64_t nq, uint32_t
     }
     // fused exchange: the merge of world * k candidates needs its own scratch (keys + global ids) behind the search's
     uint64_t merge_smem = 0;
-    if (fx) {
-        const uint64_t total = static_cast<uint64_t>(fx->world) * k;
+    if (fused) {
+        const uint64_t total = static_cast<uint64_t>(p.ex_world) * k;
         if (total > 4096) return fail(ZVDB_ERR_UNSUPPORTED, "merge: G*k > 4096");
         p.merge_p2 = next_pow2(static_cast<uint32_t>(total));
         merge_smem = (total * 12 + 8 * 4 + 15) & ~15ull;     // global ids u64 + distance words u32 per candidate, 8 list lengths
     }
-    auto ctas_for = [](uint64_t smem) { return std::min<uint64_t>(32, (227ull * 1024) / (smem + 1024)); };
-    int vis = plan_visited(ix, ef);
+    int vis = v.vis;
     if (vis == kVisGlobalBitmap && ix->visited_mode == 0) {
         // reserve the bitmaps now; if the device cannot hold them, fall back to the hash (whose footprint does not grow with n)
         const uint64_t resident0 = std::min<uint64_t>(nq, 32ull * ix->num_sms);
         const uint64_t need0 = resident0 * ((g.n + 31) / 32);
         if (need0 > ix->bitmap_buf.cap) {
             cudaError_t eb = ix->bitmap_buf.reserve(need0);
-            if (eb == cudaErrorMemoryAllocation) { cudaGetLastError(); ix->bitmap_oom = true; vis = plan_visited(ix, ef); }
+            if (eb == cudaErrorMemoryAllocation) { cudaGetLastError(); ix->bitmap_oom = true; vis = plan_visited(ix, ef).vis; }
             else { ZV_CUDA(eb); ZV_CUDA(cudaMemsetAsync(ix->bitmap_buf.p, 0, ix->bitmap_buf.cap * sizeof(uint32_t), s)); }
         }
     }
     const uint64_t res_cap = (static_cast<uint64_t>(ef) + 1) & ~1ull;
     // global modes: the popped-key list moves to per-CTA global scratch when it would cost residency (see the kernel)
-    const bool res_global = vis != kVisSmemHash && ctas_for(smem_lists + merge_smem) < 32;
-    uint64_t smem = vis == kVisSmemHash ? smem_hash : (res_global ? smem_lists - res_cap * 8 : smem_lists);
+    const bool res_global = vis != kVisSmemHash && ctas_for(v.smem_lists + merge_smem) < 32;
+    uint64_t smem = vis == kVisSmemHash ? v.smem_hash : (res_global ? v.smem_lists - res_cap * 8 : v.smem_lists);
     smem = (smem + 15) & ~15ull;
     p.merge_off = static_cast<uint32_t>(smem);
     smem += merge_smem;
@@ -507,13 +493,13 @@ static int launch_search(zvdb_index *ix, const float *d_q, uint64_t nq, uint32_t
                  static_cast<unsigned long long>(smem), ef, g.m, ix->smem_optin);
         return fail(ZVDB_ERR_UNSUPPORTED, buf);
     }
-    p.slots = static_cast<uint32_t>(slots); p.hash_words = static_cast<uint32_t>(hash_words);
+    p.slots = static_cast<uint32_t>(v.slots); p.hash_words = static_cast<uint32_t>(v.hash_words);
     // L2 prefetch, automatic = the rows of a pop's later gather batches, in the global modes with rows of at most 1 KiB
     // (+2..4 % on a graph that reaches every row; wider rows are bandwidth bound); off in shared-hash mode (small
     // ef: the extra issue slots cost 1-2 %). Prefetching the evaluated neighbours' adjacency rows measured no gain
     // anywhere and stays a variant. A/B: profiles/r01_k1_prefetch_ab.jsonl.
     p.prefetch = ix->prefetch_mode == 0 ? ((vis != kVisSmemHash && cpl <= 2) ? 1u : 0u) : ix->prefetch_mode - 1u;
-    p.cand_cap = static_cast<uint32_t>(cand_cap);
+    p.cand_cap = static_cast<uint32_t>(v.cand_cap);
     // One warp per query; CTAs resident per SM: 32 (16 beyond 256 floats per row: registers), fewer if shared memory binds.
     const uint64_t resident = std::min<uint64_t>(ctas_for(smem), cpl <= 2 ? 32 : 16) * ix->num_sms;
     unsigned grid = static_cast<unsigned>(nq);
@@ -533,14 +519,14 @@ static int launch_search(zvdb_index *ix, const float *d_q, uint64_t nq, uint32_t
                 ZV_CUDA(ix->bitmap_buf.reserve(need));
                 ZV_CUDA(cudaMemsetAsync(ix->bitmap_buf.p, 0, ix->bitmap_buf.cap * sizeof(uint32_t), s));
             }
-            const uint64_t log_cap = (bound + 3) & ~3ull;                          // 16-byte aligned logs (read back as uint4)
+            const uint64_t log_cap = (v.bound + 3) & ~3ull;                         // 16-byte aligned logs (read back as uint4)
             ZV_CUDA(ix->vlog_buf.reserve(grid * log_cap));
             p.gbitmap = ix->bitmap_buf.p; p.glog = ix->vlog_buf.p;
             p.bm_words = static_cast<uint32_t>(bm_words); p.log_cap = static_cast<uint32_t>(log_cap);
         } else {
             // every slot reads kInvalidId between queries: the kernel leaves the tables it used wiped, whatever their
             // pitch was, so only fresh memory is initialised here
-            const uint64_t need = grid * hash_words;
+            const uint64_t need = grid * v.hash_words;
             if (need > ix->gtable_buf.cap) {
                 ZV_CUDA(ix->gtable_buf.reserve(need));
                 ZV_CUDA(cudaMemsetAsync(ix->gtable_buf.p, 0xFF, ix->gtable_buf.cap * sizeof(uint32_t), s));
@@ -552,19 +538,9 @@ static int launch_search(zvdb_index *ix, const float *d_q, uint64_t nq, uint32_t
             p.gres = ix->res_buf.p; p.res_cap = static_cast<uint32_t>(res_cap);
         }
     }
-    if (fx) {
-        for (uint32_t i = 0; i < fx->world; ++i) p.peer_qflags[i] = fx->peer_qflags[i];
-        p.qflags = fx->qflags; p.gather = fx->gather; p.block_bytes = fx->block_bytes;
-        p.m_ids = fx->m_ids; p.m_dist = fx->m_dist; p.m_counts = fx->m_counts;
-        p.ex_world = fx->world; p.ex_rank = fx->rank; p.ex_epoch = fx->epoch;
-        p.ll_local = fx->ll_local; p.ll_lines = fx->ll_lines; p.ll_pitch = fx->ll_pitch; p.ll_nq = fx->ll_nq;
-        for (uint32_t i = 0; i < fx->world; ++i) p.peer_ll[i] = fx->peer_ll[i];
-        p.q_per = fx->q_per; p.sflags = fx->sflags; p.sflag_pitch = fx->sflag_pitch;
-        for (uint32_t i = 0; i < fx->world; ++i) { p.peer_q[i] = fx->peer_q[i]; p.peer_sflags[i] = fx->peer_sflags[i]; }
-        if (vis == kVisSmemHash) {                        // CTA b searches query b and merges query b - lag, one wave behind
-            p.merge_lag = static_cast<uint32_t>(std::min<uint64_t>(resident, nq));
-            grid = static_cast<unsigned>(nq + p.merge_lag);
-        }
+    if (fused && vis == kVisSmemHash) {                   // CTA b searches query b and merges query b - lag, one wave behind
+        p.merge_lag = static_cast<uint32_t>(std::min<uint64_t>(resident, nq));
+        grid = static_cast<unsigned>(nq + p.merge_lag);
     }
     cudaError_t e;
     if (p.seeds) {                                        // K2 first: one warp per query, 4 per CTA
@@ -574,9 +550,9 @@ static int launch_search(zvdb_index *ix, const float *d_q, uint64_t nq, uint32_t
         ix->launches++;
         ZV_CUDA(e);
     }
-    if (vis == kVisSmemHash) e = launch_k1<kVisSmemHash>(exch, rowf, g.metric, cpl, p, grid, smem, s);
-    else if (vis == kVisGlobalBitmap) e = launch_k1<kVisGlobalBitmap>(exch, rowf, g.metric, cpl, p, grid, smem, s);
-    else e = launch_k1<kVisGlobalHash>(exch, rowf, g.metric, cpl, p, grid, smem, s);
+    if (vis == kVisSmemHash) e = launch_k1<kVisSmemHash>(exch != nullptr, rowf, g.metric, cpl, p, grid, smem, s);
+    else if (vis == kVisGlobalBitmap) e = launch_k1<kVisGlobalBitmap>(exch != nullptr, rowf, g.metric, cpl, p, grid, smem, s);
+    else e = launch_k1<kVisGlobalHash>(exch != nullptr, rowf, g.metric, cpl, p, grid, smem, s);
     ix->launches++;
     ZV_CUDA(e);
     if (vis != kVisSmemHash || p.seeds) ZV_CUDA(cudaEventRecord(ix->bitmap_ev, s));
@@ -780,7 +756,7 @@ static int launch_bruteforce(zvdb_index *ix, const float *d_q, uint64_t nq, uint
         ZV_CUDA(ix->bf_xlo.reserve(n * pitch));
         ZV_CUDA(ix->bf_xnorm.reserve(n));
         const unsigned blocks = static_cast<unsigned>(std::min<uint64_t>((n + 7) / 8, 148ull * 16));
-        bf::split_tf32_kernel<<<blocks, 256, 0, s>>>(ix->d_arena, pitch, pitch, n, ix->bf_xhi.p, ix->bf_xlo.p, pitch, ix->bf_xnorm.p);
+        bf::split_tf32_kernel<<<blocks, 256, 0, s>>>(ix->d_arena.p, pitch, pitch, n, ix->bf_xhi.p, ix->bf_xlo.p, pitch, ix->bf_xnorm.p);
         ix->launches++;
         ZV_CUDA(cudaGetLastError());
         ix->bf_rows = n;
@@ -876,7 +852,7 @@ static int launch_bruteforce(zvdb_index *ix, const float *d_q, uint64_t nq, uint
     ZV_CUDA(cudaGetLastError());
     // (4) merge the splits, exact re-rank, write k
     bf::BfFinalParams fp{};
-    fp.arena = reinterpret_cast<const float4 *>(ix->d_arena);
+    fp.arena = reinterpret_cast<const float4 *>(ix->d_arena.p);
     fp.queries = d_q; fp.part_keys = p.part_keys;
     fp.ids = d_ids; fp.dist = d_dist; fp.counts = d_counts;
     fp.id_stride = id_stride; fp.id_base = id_base;
@@ -899,7 +875,6 @@ static int launch_bruteforce(zvdb_index *ix, const float *d_q, uint64_t nq, uint
 // frontier's length. 16 bytes per node and 4.
 struct ReachScratch {
     DevBuf<uint32_t> depth, parent, q0, q1, count;
-    ~ReachScratch() { depth.free_(); parent.free_(); q0.free_(); q1.free_(); count.free_(); }
 };
 
 // Level-synchronous BFS over the device table from the entry point (device current, n > 0): depth, parent, and the
@@ -924,7 +899,7 @@ static int reach_locked(zvdb_index *ix, ReachScratch &r, uint64_t &reached) {
         ZV_CUDA(cudaMemsetAsync(r.count.p, 0, sizeof(uint32_t), s));
         const uint64_t total = static_cast<uint64_t>(count) * g.m;
         const unsigned blocks = static_cast<unsigned>(std::min<uint64_t>((total + 255) / 256, 148ull * 16));
-        bfs_level_kernel<<<blocks, 256, 0, s>>>(ix->d_adj, g.m, n, cur, count, level, r.depth.p, r.parent.p, next, r.count.p);
+        bfs_level_kernel<<<blocks, 256, 0, s>>>(ix->d_adj.p, g.m, n, cur, count, level, r.depth.p, r.parent.p, next, r.count.p);
         ix->launches++;
         ZV_CUDA(cudaGetLastError());
         ZV_CUDA(cudaMemcpyAsync(&count, r.count.p, sizeof count, cudaMemcpyDeviceToHost, s));
@@ -939,13 +914,75 @@ static int reach_locked(zvdb_index *ix, ReachScratch &r, uint64_t &reached) {
 struct ConnectScratch {
     DevBuf<float> q, dist;
     DevBuf<uint64_t> ids, best;
-    DevBuf<uint32_t> unreached, cnt, accepted, cursor, target, won, counters, rows, touched;
+    DevBuf<uint32_t> unreached, cnt, accepted, cursor, target, won, counters, touched;
     DevBuf<uint8_t> eligible, tmp;
-    ~ConnectScratch() {
-        q.free_(); dist.free_(); ids.free_(); best.free_(); unreached.free_(); cnt.free_(); accepted.free_(); cursor.free_();
-        target.free_(); won.free_(); counters.free_(); rows.free_(); touched.free_(); eligible.free_(); tmp.free_();
-    }
 };
+
+// Graph search of nq device-resident queries (dim floats each), k results each, in launches of at most 2^31-1 queries.
+static int search_all(zvdb_index *ix, const float *d_q, uint64_t nq, uint32_t k, uint32_t ef, uint64_t *d_ids, float *d_dist,
+                      uint32_t *d_counts, cudaStream_t s) {
+    for (uint64_t q0 = 0; q0 < nq; q0 += 0x7FFFFFFFull) {
+        const uint64_t cnt = std::min<uint64_t>(nq - q0, 0x7FFFFFFFull);
+        int rc = launch_search(ix, d_q + q0 * ix->g.dim, cnt, k, ef, d_ids + q0 * k, d_dist + q0 * k, d_counts + q0, nullptr,
+                               nullptr, 1, 0, s);
+        if (rc) return rc;
+    }
+    return ZVDB_OK;
+}
+
+// The device table's rows d_ids[0..count) (host_ids: the same ids on the host) into the host's layer-0 table: one
+// gather on the device, one copy.
+static int download_rows(zvdb_index *ix, const uint32_t *d_ids, uint32_t count, const uint32_t *host_ids, const char *what) {
+    HostGraph &g = ix->g;
+    cudaStream_t s = ix->stream;
+    std::vector<uint32_t> rows;
+    try { rows.resize(static_cast<size_t>(count) * g.m); }
+    catch (const std::bad_alloc &) { return fail(ZVDB_ERR_OUT_OF_MEMORY, std::string(what) + ": out of memory"); }
+    DevBuf<uint32_t> d_rows;
+    ZV_CUDA(d_rows.reserve(std::max<size_t>(rows.size(), 1)));
+    const unsigned blocks = static_cast<unsigned>(std::min<uint64_t>((rows.size() + 255) / 256 + 1, 148ull * 8));
+    gather_adj_rows_kernel<<<blocks, 256, 0, s>>>(d_rows.p, ix->d_adj.p, d_ids, count, g.m); ix->launches++;
+    ZV_CUDA(cudaGetLastError());
+    ZV_CUDA(cudaMemcpyAsync(rows.data(), d_rows.p, rows.size() * sizeof(uint32_t), cudaMemcpyDeviceToHost, s));
+    ZV_CUDA(cudaStreamSynchronize(s));
+    for (uint32_t t = 0; t < count; ++t)
+        std::memcpy(g.adj0.data() + static_cast<size_t>(host_ids[t]) * g.m, rows.data() + static_cast<size_t>(t) * g.m, g.m * sizeof(uint32_t));
+    return ZVDB_OK;
+}
+
+// Reverse lists of the forward lists fw[rows][m] (ids < n) for K6 and K7: cnt[j] = in-degree of node j (cnt[n] = 0),
+// off[0..n] their exclusive scan (off[n] = the edge count), rev[off[j] ..) the rows linking to j, in atomic order.
+// rev is allocated at its exact size (off[n] read back).
+struct ReverseLists {
+    DevBuf<uint32_t> cnt;     // [n + 1] counts, then [n] fill cursors
+    DevBuf<uint64_t> off;     // [n + 1]
+    DevBuf<uint32_t> rev;
+    DevBuf<uint8_t> tmp;      // the scan's scratch
+};
+static int build_reverse_lists(zvdb_index *ix, const uint32_t *fw, uint64_t rows, uint64_t n, ReverseLists &r) {
+    cudaStream_t s = ix->stream;
+    const uint32_t m = ix->g.m;
+    ZV_CUDA(r.cnt.reserve(2 * n + 1));
+    ZV_CUDA(r.off.reserve(n + 1));
+    ZV_CUDA(cudaMemsetAsync(r.cnt.p, 0, (2 * n + 1) * sizeof(uint32_t), s));
+    const uint64_t total = rows * m;
+    const unsigned blocks = static_cast<unsigned>(std::min<uint64_t>((total + 255) / 256, 148ull * 16));
+    count_reverse_kernel<<<blocks, 256, 0, s>>>(fw, total, r.cnt.p); ix->launches++;
+    ZV_CUDA(cudaGetLastError());
+    auto widened = thrust::make_transform_iterator(r.cnt.p, WidenU32{});
+    size_t bytes = 0;
+    ZV_CUDA(cub::DeviceScan::ExclusiveSum(nullptr, bytes, widened, r.off.p, static_cast<int64_t>(n + 1), s));
+    ZV_CUDA(r.tmp.reserve(std::max<size_t>(bytes, 1)));
+    ZV_CUDA(cub::DeviceScan::ExclusiveSum(r.tmp.p, bytes, widened, r.off.p, static_cast<int64_t>(n + 1), s));
+    ix->launches++;
+    uint64_t edges = 0;
+    ZV_CUDA(cudaMemcpyAsync(&edges, r.off.p + n, sizeof edges, cudaMemcpyDeviceToHost, s));
+    ZV_CUDA(cudaStreamSynchronize(s));
+    ZV_CUDA(r.rev.reserve(std::max<uint64_t>(edges, 1)));
+    fill_reverse_kernel<<<blocks, 256, 0, s>>>(fw, total, m, r.off.p, r.cnt.p + n + 1, r.rev.p); ix->launches++;
+    ZV_CUDA(cudaGetLastError());
+    return ZVDB_OK;
+}
 
 // rows[0..count) = the ids v < n with pred(v), ascending (CUB select over the node ids); returns count.
 template <typename Pred>
@@ -985,17 +1022,13 @@ static int connect_locked(zvdb_index *ix, uint32_t K, uint32_t ef, uint32_t max_
     st.searched = nu;
     ZV_CUDA(c.q.reserve(static_cast<size_t>(nu) * g.dim));
     const unsigned qblocks = static_cast<unsigned>(std::min<uint64_t>((static_cast<uint64_t>(nu) * g.dim + 255) / 256, 148ull * 8));
-    gather_query_rows_kernel<<<qblocks, 256, 0, s>>>(c.q.p, ix->d_arena, g.row_floats, c.unreached.p, nu, g.dim); ix->launches++;
+    gather_query_rows_kernel<<<qblocks, 256, 0, s>>>(c.q.p, ix->d_arena.p, g.row_floats, c.unreached.p, nu, g.dim); ix->launches++;
     ZV_CUDA(cudaGetLastError());
     ZV_CUDA(c.ids.reserve(static_cast<size_t>(nu) * K));
     ZV_CUDA(c.dist.reserve(static_cast<size_t>(nu) * K));
     ZV_CUDA(c.cnt.reserve(nu));
-    for (uint64_t q0 = 0; q0 < nu; q0 += 0x7FFFFFFFull) {   // launch_search's per-launch query limit
-        const uint64_t cnt = std::min<uint64_t>(nu - q0, 0x7FFFFFFFull);
-        rc = launch_search(ix, c.q.p + q0 * g.dim, cnt, K, ef, c.ids.p + q0 * K, c.dist.p + q0 * K, c.cnt.p + q0, nullptr, nullptr,
-                           1, 0, s);
-        if (rc) return rc;
-    }
+    rc = search_all(ix, c.q.p, nu, K, ef, c.ids.p, c.dist.p, c.cnt.p, s);
+    if (rc) return rc;
     c.q.free_();
     // the matching state
     ZV_CUDA(c.accepted.reserve(n));
@@ -1007,8 +1040,8 @@ static int connect_locked(zvdb_index *ix, uint32_t K, uint32_t ef, uint32_t max_
     ZV_CUDA(c.counters.reserve(2));
     ZV_CUDA(cudaMemsetAsync(c.accepted.p, 0, static_cast<size_t>(n) * sizeof(uint32_t), s));
     ConnectParams cp{};
-    cp.arena = reinterpret_cast<const float4 *>(ix->d_arena);
-    cp.row_chunks = g.row_floats / 4; cp.n = n; cp.m = g.m; cp.adj = ix->d_adj;
+    cp.arena = reinterpret_cast<const float4 *>(ix->d_arena.p);
+    cp.row_chunks = g.row_floats / 4; cp.n = n; cp.m = g.m; cp.adj = ix->d_adj.p;
     cp.depth = r.depth.p; cp.parent = r.parent.p; cp.unreached = c.unreached.p; cp.nu = nu;
     cp.cand = c.ids.p; cp.cand_dist = c.dist.p; cp.K = K; cp.max_new = max_new;
     cp.accepted = c.accepted.p; cp.eligible = c.eligible.p; cp.best = c.best.p; cp.cursor = c.cursor.p; cp.target = c.target.p;
@@ -1057,19 +1090,51 @@ static int connect_locked(zvdb_index *ix, uint32_t K, uint32_t ef, uint32_t max_
     rc = select_rows(n, AcceptedRow{c.accepted.p}, c.touched, c.tmp, nt, ix);
     if (rc) return rc;
     st.rows_rewritten = nt;
-    std::vector<uint32_t> touched, rows;
-    try { touched.resize(nt); rows.resize(static_cast<size_t>(nt) * g.m); }
-    catch (const std::bad_alloc &) { return fail(ZVDB_ERR_OUT_OF_MEMORY, "connect: out of memory"); }
-    ZV_CUDA(c.rows.reserve(std::max<size_t>(rows.size(), 1)));
-    const unsigned gblocks = static_cast<unsigned>(std::min<uint64_t>((rows.size() + 255) / 256 + 1, 148ull * 8));
-    gather_adj_rows_kernel<<<gblocks, 256, 0, s>>>(c.rows.p, ix->d_adj, c.touched.p, nt, g.m); ix->launches++;
-    ZV_CUDA(cudaGetLastError());
+    std::vector<uint32_t> touched;
+    try { touched.resize(nt); } catch (const std::bad_alloc &) { return fail(ZVDB_ERR_OUT_OF_MEMORY, "connect: out of memory"); }
     ZV_CUDA(cudaMemcpyAsync(touched.data(), c.touched.p, nt * sizeof(uint32_t), cudaMemcpyDeviceToHost, s));
-    ZV_CUDA(cudaMemcpyAsync(rows.data(), c.rows.p, rows.size() * sizeof(uint32_t), cudaMemcpyDeviceToHost, s));
-    ZV_CUDA(cudaStreamSynchronize(s));
-    for (uint32_t t = 0; t < nt; ++t)
-        std::memcpy(g.adj0.data() + static_cast<size_t>(touched[t]) * g.m, rows.data() + static_cast<size_t>(t) * g.m, g.m * sizeof(uint32_t));
+    return download_rows(ix, c.touched.p, nt, touched.data(), "connect");
+}
+
+// ---- the search entry points' shared host steps ----------------------------------------------------
+
+// The argument checks of every search entry point, in this order; `what` names the call in the message. ef (graph
+// searches only; null for exact k-NN): 0 = k.
+static int check_search_args(const char *what, const void *queries, const void *ids, const void *dist, const void *counts,
+                             uint32_t k, uint32_t *ef) {
+    if (!queries || !ids || !dist || !counts) return fail(ZVDB_ERR_INVALID, std::string(what) + ": null buffer");
+    if (k == 0) return fail(ZVDB_ERR_INVALID, std::string(what) + ": k must be >= 1");
+    if (ef && *ef == 0) *ef = k;
+    if (ef && *ef < k) return fail(ZVDB_ERR_INVALID, std::string(what) + ": ef must be >= k");
     return ZVDB_OK;
+}
+
+// The result of a search of an empty index, which is not an error (test_hnsw.zig:43-53): count 0, ids ~0, distance 0,
+// and pops / evals 0 where the call reports them. Host buffers, and device buffers (enqueued on s).
+static void empty_result_host(uint64_t nq, uint32_t k, uint64_t *ids, float *dist, uint32_t *counts, uint32_t *pops = nullptr,
+                              uint32_t *evals = nullptr) {
+    for (uint64_t i = 0; i < nq; ++i) counts[i] = 0;
+    for (uint64_t i = 0; i < nq * k; ++i) { ids[i] = ZVDB_INVALID_ID; dist[i] = 0.0f; }
+    if (pops) for (uint64_t i = 0; i < nq; ++i) pops[i] = 0;
+    if (evals) for (uint64_t i = 0; i < nq; ++i) evals[i] = 0;
+}
+static int empty_result_device(uint64_t nq, uint32_t k, uint64_t *ids, float *dist, uint32_t *counts, uint32_t *pops,
+                               uint32_t *evals, cudaStream_t s) {
+    ZV_CUDA(cudaMemsetAsync(counts, 0, nq * sizeof(uint32_t), s));
+    ZV_CUDA(cudaMemsetAsync(ids, 0xFF, nq * k * sizeof(uint64_t), s));
+    ZV_CUDA(cudaMemsetAsync(dist, 0, nq * k * sizeof(float), s));
+    if (pops) ZV_CUDA(cudaMemsetAsync(pops, 0, nq * sizeof(uint32_t), s));
+    if (evals) ZV_CUDA(cudaMemsetAsync(evals, 0, nq * sizeof(uint32_t), s));
+    return ZVDB_OK;
+}
+
+// Whether host memory `ptr` is page-locked and mapped into the device, and if so its device address.
+static bool mapped_device_pointer(const void *ptr, void **dptr) {
+    cudaPointerAttributes a{};
+    if (cudaPointerGetAttributes(&a, ptr) != cudaSuccess) { cudaGetLastError(); return false; }
+    if (a.type != cudaMemoryTypeHost || a.devicePointer == nullptr) return false;
+    *dptr = a.devicePointer;
+    return true;
 }
 
 }  // namespace zvdb
@@ -1126,14 +1191,8 @@ void zvdb_destroy(zvdb_index *ix) {
     for (int i = 0; i < 8; ++i) if (ix->in_ev[i]) cudaEventDestroy(ix->in_ev[i]);
     if (ix->bitmap_ev) cudaEventDestroy(ix->bitmap_ev);
     if (ix->bf_ev) cudaEventDestroy(ix->bf_ev);
-    cudaFree(ix->d_arena); cudaFree(ix->d_adj);
     if (ix->h_stage) cudaFreeHost(ix->h_stage);
-    ix->row_copy.release();
-    ix->q_buf.free_(); ix->dist_buf.free_(); ix->ids_buf.free_(); ix->cnt_buf.free_();
-    ix->pops_buf.free_(); ix->evals_buf.free_(); ix->scat_rows.free_(); ix->scat_ids.free_(); ix->bitmap_buf.free_(); ix->vlog_buf.free_(); ix->res_buf.free_(); ix->gtable_buf.free_();
-    ix->d_level.free_(); ix->d_upper_base.free_(); ix->d_upper_adj.free_(); ix->seeds_buf.free_();
-    ix->bf_xhi.free_(); ix->bf_xlo.free_(); ix->bf_xnorm.free_(); ix->bf_qhi.free_(); ix->bf_qlo.free_(); ix->bf_part.free_(); ix->bf_glists.free_(); ix->bf_segs.free_(); ix->bf_seg_off.free_();
-    delete ix;
+    delete ix;   // the device buffers go with their owners, on this device and behind the synchronised streams
 }
 
 int zvdb_set_level_seed(zvdb_index *ix, uint64_t seed) {
@@ -1314,12 +1373,7 @@ static int set_points_locked(zvdb_index *ix, const float *points, uint64_t n, ui
         g.level.assign(n, 0);
         g.upper_off.assign(n, ~0ull);
     } catch (const std::bad_alloc &) { return fail(ZVDB_ERR_OUT_OF_MEMORY, "out of memory"); }
-    const uint64_t nchunks = (n + g.rows_per_chunk - 1) / g.rows_per_chunk;
-    for (uint64_t c = 0; c < nchunks; ++c) {
-        float *p = nullptr;
-        ZV_CUDA(cudaHostAlloc(&p, static_cast<size_t>(g.rows_per_chunk) * g.row_floats * sizeof(float), cudaHostAllocDefault));
-        g.chunks.push_back(p);
-    }
+    if (!g.reserve_rows(n)) return fail(ZVDB_ERR_OUT_OF_MEMORY, "out of memory");
     g.n = n;
     for (uint64_t i = 0; i < n; ++i) g.store_row(g.point_mut(i), points + i * dim);
     g.has_entry = n > 0; g.entry = entry; g.max_level = 0;
@@ -1388,18 +1442,9 @@ int zvdb_save(const zvdb_index *cix, const char *path) {
     hd.row_floats = g.row_floats; hd.max_level = g.max_level; hd.has_entry = g.has_entry ? 1u : 0u;
     hd.n = g.n; hd.entry = g.entry; hd.top_node = g.top_node; hd.rng = g.rng; hd.n_lists = g.upper_lists();
     cf.write(&hd, sizeof hd);
-    for (uint64_t r = 0; r < g.n;) {
-        const uint64_t end = std::min<uint64_t>(g.n, (r / g.rows_per_chunk + 1) * g.rows_per_chunk);
-        cf.write(g.point(r), (end - r) * g.row_floats * sizeof(float));
-        r = end;
-    }
-    if (g.dtype != 0) {
-        for (uint64_t r = 0; r < g.n;) {
-            const uint64_t end = std::min<uint64_t>(g.n, (r / g.rows_per_chunk + 1) * g.rows_per_chunk);
-            cf.write(g.typed_point(r), (end - r) * g.dim * g.elem_size());
-            r = end;
-        }
-    }
+    g.for_each_span(0, g.n, [&](uint64_t r, uint64_t end) { cf.write(g.point(r), (end - r) * g.row_floats * sizeof(float)); return 0; });
+    if (g.dtype != 0)
+        g.for_each_span(0, g.n, [&](uint64_t r, uint64_t end) { cf.write(g.typed_point(r), (end - r) * g.dim * g.elem_size()); return 0; });
     cf.write(g.adj0.data(), g.n * g.m * sizeof(uint32_t));
     cf.write(g.level.data(), g.n);
     std::vector<uint32_t> base(g.n), flat(hd.n_lists * g.m);
@@ -1428,8 +1473,7 @@ int zvdb_load(zvdb_index *ix, const char *path) {
         if (fread(&stored, 1, sizeof stored, cf.f) != sizeof stored || stored != cf.h) return fail(ZVDB_ERR_INVALID, "load: truncated file or checksum mismatch");
         cudaSetDevice(ix->device);
         g.reset_nodes();
-        g.dim = 0; g.row_floats = 0; g.rows_per_chunk = 0;
-        if (hd.dim) g.fix_dim(hd.dim);
+        g.fix_dim(hd.dim);
         g.ef_construction = hd.ef_construction; g.rng = hd.rng; g.dtype = 0;
         forget_device_rows(ix);
         return ZVDB_OK;
@@ -1444,30 +1488,14 @@ int zvdb_load(zvdb_index *ix, const char *path) {
     try {
         fresh.adj0.resize(hd.n * fresh.m); fresh.level.resize(hd.n); fresh.upper_off.assign(hd.n, ~0ull);
     } catch (const std::bad_alloc &) { return fail(ZVDB_ERR_OUT_OF_MEMORY, "load: out of memory"); }
-    const uint64_t nchunks = (hd.n + fresh.rows_per_chunk - 1) / fresh.rows_per_chunk;
-    for (uint64_t c = 0; c < nchunks; ++c) {
-        float *pc = nullptr;
-        ZV_CUDA(cudaHostAlloc(&pc, static_cast<size_t>(fresh.rows_per_chunk) * fresh.row_floats * sizeof(float), cudaHostAllocDefault));
-        fresh.chunks.push_back(pc);
-    }
+    if (!fresh.reserve_rows(hd.n)) return fail(ZVDB_ERR_OUT_OF_MEMORY, "load: out of memory");
     fresh.n = hd.n;
-    for (uint64_t r = 0; r < hd.n;) {
-        const uint64_t end = std::min<uint64_t>(hd.n, (r / fresh.rows_per_chunk + 1) * fresh.rows_per_chunk);
-        cf.read(fresh.point_mut(r), (end - r) * fresh.row_floats * sizeof(float));
-        r = end;
-    }
-    if (fresh.dtype != 0) {
-        for (uint64_t c = 0; c < nchunks; ++c) {
-            unsigned char *tc = static_cast<unsigned char *>(std::malloc(static_cast<size_t>(fresh.rows_per_chunk) * fresh.dim * fresh.elem_size()));
-            if (!tc) return fail(ZVDB_ERR_OUT_OF_MEMORY, "load: out of memory");
-            fresh.typed_chunks.push_back(tc);
-        }
-        for (uint64_t r = 0; r < hd.n;) {
-            const uint64_t end = std::min<uint64_t>(hd.n, (r / fresh.rows_per_chunk + 1) * fresh.rows_per_chunk);
+    fresh.for_each_span(0, hd.n, [&](uint64_t r, uint64_t end) { cf.read(fresh.point_mut(r), (end - r) * fresh.row_floats * sizeof(float)); return 0; });
+    if (fresh.dtype != 0)
+        fresh.for_each_span(0, hd.n, [&](uint64_t r, uint64_t end) {
             cf.read(const_cast<void *>(fresh.typed_point(r)), (end - r) * fresh.dim * fresh.elem_size());
-            r = end;
-        }
-    }
+            return 0;
+        });
     cf.read(fresh.adj0.data(), hd.n * fresh.m * sizeof(uint32_t));
     cf.read(fresh.level.data(), hd.n);
     uint64_t lists = 0;
@@ -1502,7 +1530,7 @@ int zvdb_load(zvdb_index *ix, const char *path) {
     fresh.rng = hd.rng;
     // swap the new state in; the device copy is rebuilt by the next search
     g.release();
-    g.dim = fresh.dim; g.row_floats = fresh.row_floats; g.rows_per_chunk = fresh.rows_per_chunk; g.ef_construction = fresh.ef_construction;
+    g.fix_dim(fresh.dim); g.ef_construction = fresh.ef_construction;
     g.dtype = fresh.dtype; g.typed_chunks.swap(fresh.typed_chunks);
     g.n = fresh.n; g.chunks.swap(fresh.chunks); g.adj0.swap(fresh.adj0); g.level.swap(fresh.level);
     g.upper_off.swap(fresh.upper_off); g.upper.swap(fresh.upper);
@@ -1610,19 +1638,10 @@ static int build_from_candidates_locked(zvdb_index *ix, uint64_t n, const uint32
     HostGraph &g = ix->g;
     int rc = ensure_capacity(ix, n);
     if (rc) return rc;
+    rc = upload_rows(ix, 0, n);
+    if (rc) return rc;
     cudaStream_t s = ix->stream;
-    for (uint64_t r = 0; r < n;) {                       // arena rows up
-        const uint64_t chunk = r / g.rows_per_chunk;
-        const uint64_t end = std::min<uint64_t>(n, (chunk + 1) * g.rows_per_chunk);
-        ZV_CUDA(cudaMemcpyAsync(ix->d_arena + r * g.row_floats, g.point(r), (end - r) * g.row_floats * sizeof(float), cudaMemcpyHostToDevice, s));
-        r = end;
-    }
-    DevBuf<uint32_t> d_cand, d_fw, d_indeg, d_rev;
-    DevBuf<uint64_t> d_off;
-    struct Cleanup {                                     // every exit frees the build scratch
-        DevBuf<uint32_t> &a, &b, &c, &d; DevBuf<uint64_t> &e;
-        ~Cleanup() { a.free_(); b.free_(); c.free_(); d.free_(); e.free_(); }
-    } cleanup{d_cand, d_fw, d_indeg, d_rev, d_off};
+    DevBuf<uint32_t> d_cand, d_fw;
     const uint32_t *cand_dev = cand;
     if (!cand_on_device) {
         ZV_CUDA(d_cand.reserve(n * K));
@@ -1630,13 +1649,10 @@ static int build_from_candidates_locked(zvdb_index *ix, uint64_t n, const uint32
         cand_dev = d_cand.p;
     }
     ZV_CUDA(d_fw.reserve(n * g.m));
-    ZV_CUDA(d_indeg.reserve(2 * n));
-    ZV_CUDA(d_off.reserve(n + 1));
-    ZV_CUDA(cudaMemsetAsync(d_indeg.p, 0, 2 * n * sizeof(uint32_t), s));
     BuildParams bp{};
-    bp.arena = reinterpret_cast<const float4 *>(ix->d_arena);
+    bp.arena = reinterpret_cast<const float4 *>(ix->d_arena.p);
     bp.row_chunks = g.row_floats / 4; bp.n = static_cast<uint32_t>(n); bp.m = g.m;
-    bp.cand = cand_dev; bp.K = K; bp.fw = d_fw.p; bp.adj = ix->d_adj;
+    bp.cand = cand_dev; bp.K = K; bp.fw = d_fw.p; bp.adj = ix->d_adj.p;
     auto launch_build = [&](bool forward) {               // K6: forward lists, then the final lists
         return dispatch(g.metric, cpl_for(g.row_floats), [&](auto fm) {
             using Fm = decltype(fm);
@@ -1646,24 +1662,13 @@ static int build_from_candidates_locked(zvdb_index *ix, uint64_t n, const uint32
     };
     cudaError_t e = launch_build(true); ix->launches++;
     ZV_CUDA(e);
-    const uint64_t total = n * g.m;
-    const unsigned blocks = static_cast<unsigned>(std::min<uint64_t>((total + 255) / 256, 148ull * 16));
-    count_reverse_kernel<<<blocks, 256, 0, s>>>(d_fw.p, total, d_indeg.p); ix->launches++;
-    std::vector<uint32_t> indeg;
-    std::vector<uint64_t> off;
-    try { indeg.resize(n); off.resize(n + 1); }
-    catch (const std::bad_alloc &) { return fail(ZVDB_ERR_OUT_OF_MEMORY, "build: out of memory"); }
-    ZV_CUDA(cudaMemcpyAsync(indeg.data(), d_indeg.p, n * sizeof(uint32_t), cudaMemcpyDeviceToHost, s));
-    ZV_CUDA(cudaStreamSynchronize(s));
-    off[0] = 0;
-    for (uint64_t i = 0; i < n; ++i) off[i + 1] = off[i] + indeg[i];
-    ZV_CUDA(d_rev.reserve(std::max<uint64_t>(off[n], 1)));
-    ZV_CUDA(cudaMemcpyAsync(d_off.p, off.data(), (n + 1) * sizeof(uint64_t), cudaMemcpyHostToDevice, s));
-    fill_reverse_kernel<<<blocks, 256, 0, s>>>(d_fw.p, total, g.m, d_off.p, d_indeg.p + n, d_rev.p); ix->launches++;
-    bp.rev_off = d_off.p; bp.rev = d_rev.p;
+    ReverseLists r;
+    rc = build_reverse_lists(ix, d_fw.p, n, n, r);
+    if (rc) return rc;
+    bp.rev_off = r.off.p; bp.rev = r.rev.p;
     e = launch_build(false); ix->launches++;
     ZV_CUDA(e);
-    ZV_CUDA(cudaMemcpyAsync(g.adj0.data(), ix->d_adj, n * g.m * sizeof(uint32_t), cudaMemcpyDeviceToHost, s));
+    ZV_CUDA(cudaMemcpyAsync(g.adj0.data(), ix->d_adj.p, n * g.m * sizeof(uint32_t), cudaMemcpyDeviceToHost, s));
     ZV_CUDA(cudaStreamSynchronize(s));
     return ZVDB_OK;
 }
@@ -1701,40 +1706,28 @@ static int append_locked(zvdb_index *ix, uint64_t n0, uint32_t K, uint32_t ef, s
     const uint64_t n = g.n, nb = n - n0;
     int rc = ensure_capacity(ix, n);
     if (rc) return rc;
+    rc = upload_rows(ix, n0, n);                          // the batch's arena rows (no links yet: nothing reaches them)
+    if (rc) return rc;
     cudaStream_t s = ix->stream;
-    for (uint64_t r = n0; r < n;) {                      // the batch's arena rows up (no links yet: nothing reaches them)
-        const uint64_t chunk = r / g.rows_per_chunk;
-        const uint64_t end = std::min<uint64_t>(n, (chunk + 1) * g.rows_per_chunk);
-        ZV_CUDA(cudaMemcpyAsync(ix->d_arena + r * g.row_floats, g.point(r), (end - r) * g.row_floats * sizeof(float), cudaMemcpyHostToDevice, s));
-        r = end;
-    }
     DevBuf<float> d_q, d_dist;
-    DevBuf<uint64_t> d_ids, d_off;
-    DevBuf<uint32_t> d_cnt, d_fw, d_indeg, d_rev, d_touched, d_rows;
+    DevBuf<uint64_t> d_ids;
+    DevBuf<uint32_t> d_cnt, d_fw, d_touched;
     DevBuf<uint8_t> d_tmp;
-    struct Cleanup {                                     // every exit frees the append scratch
-        DevBuf<float> &a, &b; DevBuf<uint64_t> &c, &d; DevBuf<uint32_t> &e, &f, &g, &h, &i, &j; DevBuf<uint8_t> &k;
-        ~Cleanup() { a.free_(); b.free_(); c.free_(); d.free_(); e.free_(); f.free_(); g.free_(); h.free_(); i.free_(); j.free_(); k.free_(); }
-    } cleanup{d_q, d_dist, d_ids, d_off, d_cnt, d_fw, d_indeg, d_rev, d_touched, d_rows, d_tmp};
     // 1. search: the batch's stored rows as queries (dim floats each), on the graph as it was
     ZV_CUDA(d_q.reserve(nb * g.dim));
-    ZV_CUDA(cudaMemcpy2DAsync(d_q.p, g.dim * sizeof(float), ix->d_arena + n0 * g.row_floats, g.row_floats * sizeof(float),
+    ZV_CUDA(cudaMemcpy2DAsync(d_q.p, g.dim * sizeof(float), ix->d_arena.p + n0 * g.row_floats, g.row_floats * sizeof(float),
                               g.dim * sizeof(float), nb, cudaMemcpyDeviceToDevice, s));
     ZV_CUDA(d_ids.reserve(nb * K));
     ZV_CUDA(d_dist.reserve(nb * K));
     ZV_CUDA(d_cnt.reserve(nb));
-    for (uint64_t q0 = 0; q0 < nb; q0 += 0x7FFFFFFFull) {   // launch_search's per-launch query limit
-        const uint64_t cnt = std::min<uint64_t>(nb - q0, 0x7FFFFFFFull);
-        rc = launch_search(ix, d_q.p + q0 * g.dim, cnt, K, ef, d_ids.p + q0 * K, d_dist.p + q0 * K, d_cnt.p + q0, nullptr, nullptr,
-                           1, 0, s);
-        if (rc) return rc;
-    }
+    rc = search_all(ix, d_q.p, nb, K, ef, d_ids.p, d_dist.p, d_cnt.p, s);
+    if (rc) return rc;
     // 2. forward lists of the batch
     ZV_CUDA(d_fw.reserve(nb * g.m));
     AppendParams ap{};
-    ap.arena = reinterpret_cast<const float4 *>(ix->d_arena);
+    ap.arena = reinterpret_cast<const float4 *>(ix->d_arena.p);
     ap.row_chunks = g.row_floats / 4; ap.n = static_cast<uint32_t>(n); ap.n0 = static_cast<uint32_t>(n0); ap.m = g.m;
-    ap.cand = d_ids.p; ap.K = K; ap.fw = d_fw.p; ap.adj = ix->d_adj;
+    ap.cand = d_ids.p; ap.K = K; ap.fw = d_fw.p; ap.adj = ix->d_adj.p;
     const int cpl = cpl_for(g.row_floats);
     cudaError_t e = dispatch(g.metric, cpl, [&](auto fm) {
         using Fm = decltype(fm);
@@ -1742,39 +1735,18 @@ static int append_locked(zvdb_index *ix, uint64_t n0, uint32_t K, uint32_t ef, s
     });
     ix->launches++;
     ZV_CUDA(e);
-    // 3. reverse rows: per-node counts (K6's kernels), offsets by a scan over the counts, the touched rows by a select
-    ZV_CUDA(d_indeg.reserve(2 * n));
-    ZV_CUDA(d_off.reserve(n));
-    ZV_CUDA(cudaMemsetAsync(d_indeg.p, 0, 2 * n * sizeof(uint32_t), s));
-    const uint64_t total = nb * g.m;
-    const unsigned blocks = static_cast<unsigned>(std::min<uint64_t>((total + 255) / 256, 148ull * 16));
-    count_reverse_kernel<<<blocks, 256, 0, s>>>(d_fw.p, total, d_indeg.p); ix->launches++;
-    ZV_CUDA(cudaGetLastError());
-    const uint64_t touched_cap = std::min<uint64_t>(n, nb + total);
-    ZV_CUDA(d_touched.reserve(touched_cap + 1));          // + the select's count word
-    uint32_t *d_nsel = d_touched.p + touched_cap;
-    auto widened = thrust::make_transform_iterator(d_indeg.p, WidenU32{});
-    const thrust::counting_iterator<uint32_t> node_ids(0);
-    const TouchedRow pick{d_indeg.p, static_cast<uint32_t>(n0)};
-    size_t scan_bytes = 0, select_bytes = 0;
-    ZV_CUDA(cub::DeviceScan::ExclusiveSum(nullptr, scan_bytes, widened, d_off.p, static_cast<int64_t>(n), s));
-    ZV_CUDA(cub::DeviceSelect::If(nullptr, select_bytes, node_ids, d_touched.p, d_nsel, static_cast<int64_t>(n), pick, s));
-    ZV_CUDA(d_tmp.reserve(std::max<size_t>(std::max(scan_bytes, select_bytes), 1)));
-    ZV_CUDA(cub::DeviceScan::ExclusiveSum(d_tmp.p, scan_bytes, widened, d_off.p, static_cast<int64_t>(n), s));
-    ix->launches++;
-    ZV_CUDA(d_rev.reserve(std::max<uint64_t>(total, 1)));
-    fill_reverse_kernel<<<blocks, 256, 0, s>>>(d_fw.p, total, g.m, d_off.p, d_indeg.p + n, d_rev.p); ix->launches++;
-    ZV_CUDA(cudaGetLastError());
-    ZV_CUDA(cub::DeviceSelect::If(d_tmp.p, select_bytes, node_ids, d_touched.p, d_nsel, static_cast<int64_t>(n), pick, s));
-    ix->launches++;
+    // 3. reverse rows (K6's), and the touched rows by a select
+    ReverseLists r;
+    rc = build_reverse_lists(ix, d_fw.p, nb, n, r);
+    if (rc) return rc;
     uint32_t nt = 0;
-    ZV_CUDA(cudaMemcpyAsync(&nt, d_nsel, sizeof nt, cudaMemcpyDeviceToHost, s));
-    ZV_CUDA(cudaStreamSynchronize(s));
+    rc = select_rows(static_cast<uint32_t>(n), TouchedRow{r.cnt.p, static_cast<uint32_t>(n0)}, d_touched, d_tmp, nt, ix);
+    if (rc) return rc;
     try { touched_host.resize(nt); } catch (const std::bad_alloc &) { return fail(ZVDB_ERR_OUT_OF_MEMORY, "append: out of memory"); }
     ZV_CUDA(cudaMemcpyAsync(touched_host.data(), d_touched.p, nt * sizeof(uint32_t), cudaMemcpyDeviceToHost, s));
     ZV_CUDA(cudaStreamSynchronize(s));
     // 4. final lists of the touched rows, in place
-    ap.touched = d_touched.p; ap.rev_off = d_off.p; ap.rev_cnt = d_indeg.p; ap.rev = d_rev.p;
+    ap.touched = d_touched.p; ap.rev_off = r.off.p; ap.rev_cnt = r.cnt.p; ap.rev = r.rev.p;
     final_started = true;
     e = dispatch(g.metric, cpl, [&](auto fm) {
         using Fm = decltype(fm);
@@ -1782,18 +1754,7 @@ static int append_locked(zvdb_index *ix, uint64_t n0, uint32_t K, uint32_t ef, s
     });
     ix->launches++;
     ZV_CUDA(e);
-    // the touched rows back: gather on the device, one copy, scatter into the host table
-    std::vector<uint32_t> rows;
-    try { rows.resize(static_cast<size_t>(nt) * g.m); } catch (const std::bad_alloc &) { return fail(ZVDB_ERR_OUT_OF_MEMORY, "append: out of memory"); }
-    ZV_CUDA(d_rows.reserve(std::max<size_t>(rows.size(), 1)));
-    const unsigned gblocks = static_cast<unsigned>(std::min<uint64_t>((rows.size() + 255) / 256 + 1, 148ull * 8));
-    gather_adj_rows_kernel<<<gblocks, 256, 0, s>>>(d_rows.p, ix->d_adj, d_touched.p, nt, g.m); ix->launches++;
-    ZV_CUDA(cudaGetLastError());
-    ZV_CUDA(cudaMemcpyAsync(rows.data(), d_rows.p, rows.size() * sizeof(uint32_t), cudaMemcpyDeviceToHost, s));
-    ZV_CUDA(cudaStreamSynchronize(s));
-    for (uint32_t t = 0; t < nt; ++t)
-        std::memcpy(g.adj0.data() + static_cast<size_t>(touched_host[t]) * g.m, rows.data() + static_cast<size_t>(t) * g.m, g.m * sizeof(uint32_t));
-    return ZVDB_OK;
+    return download_rows(ix, d_touched.p, nt, touched_host.data(), "append");
 }
 
 int zvdb_append_batch(zvdb_index *ix, const float *points, uint64_t n, uint32_t dim, uint32_t K, uint32_t ef) {
@@ -1852,7 +1813,6 @@ int zvdb_reachable(zvdb_index *ix, uint8_t *mask, uint64_t *count) {
     if (rc) return rc;
     if (mask) {
         DevBuf<uint8_t> d_mask;
-        struct Cleanup { DevBuf<uint8_t> &m; ~Cleanup() { m.free_(); } } cleanup{d_mask};
         ZV_CUDA(d_mask.reserve(g.n));
         const unsigned blocks = static_cast<unsigned>(std::min<uint64_t>((g.n + 255) / 256, 148ull * 16));
         reach_mask_kernel<<<blocks, 256, 0, ix->stream>>>(r.depth.p, g.n, d_mask.p); ix->launches++;
@@ -1921,21 +1881,11 @@ int zvdb_search_batch_device(zvdb_index *ix, const float *d_queries, uint64_t nq
                              uint64_t id_stride, uint64_t id_base, void *stream) {
     if (!ix) return fail(ZVDB_ERR_INVALID, "null index");
     if (nq == 0) return ZVDB_OK;
-    if (!d_queries || !d_ids || !d_dist || !d_counts) return fail(ZVDB_ERR_INVALID, "search: null buffer");
-    if (k == 0) return fail(ZVDB_ERR_INVALID, "search: k must be >= 1");
-    if (ef == 0) ef = k;
-    if (ef < k) return fail(ZVDB_ERR_INVALID, "search: ef must be >= k");
+    if (int rc = check_search_args("search", d_queries, d_ids, d_dist, d_counts, k, &ef)) return rc;
     std::lock_guard<std::mutex> lk(ix->mu);   // hnsw.zig:195-196
     ZV_CUDA(cudaSetDevice(ix->device));
     cudaStream_t s = static_cast<cudaStream_t>(stream);
-    if (ix->g.n == 0 || !ix->g.has_entry) {   // empty index: empty result, not an error (test_hnsw.zig:43-53)
-        ZV_CUDA(cudaMemsetAsync(d_counts, 0, nq * sizeof(uint32_t), s));
-        ZV_CUDA(cudaMemsetAsync(d_ids, 0xFF, nq * k * sizeof(uint64_t), s));
-        ZV_CUDA(cudaMemsetAsync(d_dist, 0, nq * k * sizeof(float), s));
-        if (d_pops) ZV_CUDA(cudaMemsetAsync(d_pops, 0, nq * sizeof(uint32_t), s));
-        if (d_evals) ZV_CUDA(cudaMemsetAsync(d_evals, 0, nq * sizeof(uint32_t), s));
-        return ZVDB_OK;
-    }
+    if (ix->g.n == 0 || !ix->g.has_entry) return empty_result_device(nq, k, d_ids, d_dist, d_counts, d_pops, d_evals, s);
     int rc = sync_device_locked(ix);
     if (rc) return rc;
     return launch_search(ix, d_queries, nq, k, ef, d_ids, d_dist, d_counts, d_pops, d_evals, id_stride, id_base, s);
@@ -1945,17 +1895,11 @@ int zvdb_search_batch(zvdb_index *ix, const float *queries, uint64_t nq, uint32_
                       uint64_t *ids, float *dist, uint32_t *counts, uint32_t *pops, uint32_t *evals) {
     if (!ix) return fail(ZVDB_ERR_INVALID, "null index");
     if (nq == 0) return ZVDB_OK;
-    if (!queries || !ids || !dist || !counts) return fail(ZVDB_ERR_INVALID, "search: null buffer");
-    if (k == 0) return fail(ZVDB_ERR_INVALID, "search: k must be >= 1");
-    if (ef == 0) ef = k;
-    if (ef < k) return fail(ZVDB_ERR_INVALID, "search: ef must be >= k");
+    if (int rc = check_search_args("search", queries, ids, dist, counts, k, &ef)) return rc;
     std::lock_guard<std::mutex> lk(ix->mu);   // hnsw.zig:195-196
     ZV_CUDA(cudaSetDevice(ix->device));       // no device, no search: there is no CPU path
     if (ix->g.n == 0 || !ix->g.has_entry) {
-        for (uint64_t i = 0; i < nq; ++i) counts[i] = 0;
-        for (uint64_t i = 0; i < nq * k; ++i) { ids[i] = ZVDB_INVALID_ID; dist[i] = 0.0f; }
-        if (pops) for (uint64_t i = 0; i < nq; ++i) pops[i] = 0;
-        if (evals) for (uint64_t i = 0; i < nq; ++i) evals[i] = 0;
+        empty_result_host(nq, k, ids, dist, counts, pops, evals);
         return ZVDB_OK;
     }
     if (dim != ix->g.dim) return fail(ZVDB_ERR_DIM_MISMATCH, "Mismatched dimensions in distance calculation");
@@ -1965,17 +1909,11 @@ int zvdb_search_batch(zvdb_index *ix, const float *queries, uint64_t nq, uint32_
     // The search kernel reads each query straight from host memory when its warp starts (one 16-byte load per lane,
     // ~2 us over PCIe against ~100 us of search per query) and writes its k results straight back, so both
     // transfers ride under the compute of the other ~4 700 resident queries: one launch, no copy calls.
-    auto mapped = [](const void *ptr, void **dptr) {
-        cudaPointerAttributes a{};
-        if (cudaPointerGetAttributes(&a, ptr) != cudaSuccess) { cudaGetLastError(); return false; }
-        if (a.type != cudaMemoryTypeHost || a.devicePointer == nullptr) return false;
-        *dptr = a.devicePointer;
-        return true;
-    };
     if (!ix->stage_host_buffers) {
         void *dq = nullptr, *di = nullptr, *dd = nullptr, *dc = nullptr, *dp = nullptr, *de = nullptr;
-        if (mapped(queries, &dq) && mapped(ids, &di) && mapped(dist, &dd) && mapped(counts, &dc) &&
-            (!pops || mapped(pops, &dp)) && (!evals || mapped(evals, &de))) {
+        if (mapped_device_pointer(queries, &dq) && mapped_device_pointer(ids, &di) && mapped_device_pointer(dist, &dd) &&
+            mapped_device_pointer(counts, &dc) && (!pops || mapped_device_pointer(pops, &dp)) &&
+            (!evals || mapped_device_pointer(evals, &de))) {
             rc = launch_search(ix, static_cast<const float *>(dq), nq, k, ef, static_cast<uint64_t *>(di), static_cast<float *>(dd),
                                static_cast<uint32_t *>(dc), static_cast<uint32_t *>(dp), static_cast<uint32_t *>(de), 1, 0, ix->stream);
             if (rc) return rc;
@@ -2046,7 +1984,7 @@ int zvdb_search_batch(zvdb_index *ix, const float *queries, uint64_t nq, uint32_
         if (cudaPointerGetAttributes(&a, ptr) != cudaSuccess) { cudaGetLastError(); return false; }
         return a.type == cudaMemoryTypeHost;
     };
-    const uint64_t nchunks = (nq >= 4096 && plan_visited(ix, ef) == kVisSmemHash && pinned(queries) && pinned(ids) && pinned(dist)) ? 4 : 1;
+    const uint64_t nchunks = (nq >= 4096 && plan_visited(ix, ef).vis == kVisSmemHash && pinned(queries) && pinned(ids) && pinned(dist)) ? 4 : 1;
     const uint64_t per = (nq + nchunks - 1) / nchunks;
     if (nchunks > 1) {   // all copies in go down their own stream, back to back; kernels and copies out alternate between two others
         for (uint64_t c = 0, off = 0; off < nq; ++c, off += per) {
@@ -2098,17 +2036,11 @@ int zvdb_bruteforce_knn_device(zvdb_index *ix, const float *d_queries, uint64_t 
                                float *d_dist, uint32_t *d_counts, uint64_t id_stride, uint64_t id_base, void *stream) {
     if (!ix) return fail(ZVDB_ERR_INVALID, "null index");
     if (nq == 0) return ZVDB_OK;
-    if (!d_queries || !d_ids || !d_dist || !d_counts) return fail(ZVDB_ERR_INVALID, "bruteforce: null buffer");
-    if (k == 0) return fail(ZVDB_ERR_INVALID, "bruteforce: k must be >= 1");
+    if (int rc = check_search_args("bruteforce", d_queries, d_ids, d_dist, d_counts, k, nullptr)) return rc;
     std::lock_guard<std::mutex> lk(ix->mu);
     ZV_CUDA(cudaSetDevice(ix->device));
     cudaStream_t s = static_cast<cudaStream_t>(stream);
-    if (ix->g.n == 0) {
-        ZV_CUDA(cudaMemsetAsync(d_counts, 0, nq * sizeof(uint32_t), s));
-        ZV_CUDA(cudaMemsetAsync(d_ids, 0xFF, nq * k * sizeof(uint64_t), s));
-        ZV_CUDA(cudaMemsetAsync(d_dist, 0, nq * k * sizeof(float), s));
-        return ZVDB_OK;
-    }
+    if (ix->g.n == 0) return empty_result_device(nq, k, d_ids, d_dist, d_counts, nullptr, nullptr, s);
     int rc = sync_device_locked(ix);
     if (rc) return rc;
     return launch_bruteforce(ix, d_queries, nq, k, d_ids, d_dist, d_counts, id_stride, id_base, s);
@@ -2118,13 +2050,11 @@ int zvdb_bruteforce_knn(zvdb_index *ix, const float *queries, uint64_t nq, uint3
                         float *dist, uint32_t *counts) {
     if (!ix) return fail(ZVDB_ERR_INVALID, "null index");
     if (nq == 0) return ZVDB_OK;
-    if (!queries || !ids || !dist || !counts) return fail(ZVDB_ERR_INVALID, "bruteforce: null buffer");
-    if (k == 0) return fail(ZVDB_ERR_INVALID, "bruteforce: k must be >= 1");
+    if (int rc = check_search_args("bruteforce", queries, ids, dist, counts, k, nullptr)) return rc;
     std::lock_guard<std::mutex> lk(ix->mu);
     ZV_CUDA(cudaSetDevice(ix->device));
     if (ix->g.n == 0) {
-        for (uint64_t i = 0; i < nq; ++i) counts[i] = 0;
-        for (uint64_t i = 0; i < nq * k; ++i) { ids[i] = ZVDB_INVALID_ID; dist[i] = 0.0f; }
+        empty_result_host(nq, k, ids, dist, counts);
         return ZVDB_OK;
     }
     if (dim != ix->g.dim) return fail(ZVDB_ERR_DIM_MISMATCH, "Mismatched dimensions in distance calculation");
@@ -2187,22 +2117,51 @@ struct zvdb_exchange {
     int device = 0;
     uint32_t world = 1, rank = 0;
     uint64_t cap_bytes = 0;          // bytes of one parity half: world blocks
-    uint8_t *local = nullptr;        // [2][world][block] | flags
+    DevBuf<uint8_t> local;           // [2][world][block] | flags (exported to the peers whole: cudaIpcGetMemHandle)
     uint64_t flags_off = 0;
     uint8_t *peer[8] = {nullptr, nullptr, nullptr, nullptr, nullptr, nullptr, nullptr, nullptr};
-    uint32_t **d_peer_flags = nullptr;   // device array of world pointers
+    DevBuf<uint32_t *> d_peer_flags; // device array of world pointers
     uint64_t qflags_off = 0;         // per-query flag rows [nq_max][8] u32 (fused step): slot r of row q = last epoch rank r published for q
     uint64_t nq_max = 0;
     uint64_t ll_off = 0;             // fused step, record form: [2][world][nq_max][ll_pitch] lines of 128 bytes
     uint32_t ll_pitch = 0;           // lines reserved per record: ceil((2 * k_max + 1) / 30)
     uint64_t qbuf_off = 0;           // host step: [2][nq_max][dim_max] f32, this rank's slice of the query batch (by epoch parity)
     uint32_t dim_max = 0;
-    uint64_t *d_out_ids = nullptr; float *d_out_dist = nullptr; uint32_t *d_out_counts = nullptr;   // host step with pageable result buffers: staging
-    uint64_t out_cap = 0;
+    DevBuf<uint64_t> d_out_ids;      // host step with pageable result buffers: staging, [nq][k] / [nq]
+    DevBuf<float> d_out_dist;
+    DevBuf<uint32_t> d_out_counts;
     uint32_t epoch = 0;
     bool opened = false;
 };
 static constexpr uint32_t kFlagPitch = 32;   // one flag per 128 bytes
+
+// Lines of a record of k results: 2k + 1 payload words, 30 to a 128-byte line.
+static uint32_t record_lines(uint32_t k) { return (2 * k + 1 + 29) / 30; }
+
+// SearchParams' exchange section for step `epoch` of `ex`, results of `block` bytes per rank: this rank's block in every
+// peer's gather buffer, in the epoch's parity half (a peer may already be one call ahead). That is all of it for the
+// three-launch step (variant bit 12); the fused step (`fused`) adds the per-query flag rows, the merge's local gather
+// buffer and outputs, and the record lines of the same half unless the handle uses the block form (variant bit 13).
+static SearchParams exchange_section(const zvdb_index *ix, const zvdb_exchange *ex, uint32_t epoch, uint64_t block, uint32_t k,
+                                     bool fused, uint64_t *m_ids, float *m_dist, uint32_t *m_counts) {
+    SearchParams p{};
+    const uint64_t half = (epoch & 1) * ex->cap_bytes;
+    for (uint32_t g = 0; g < ex->world; ++g) p.peer_blocks[g] = ex->peer[g] + half + block * ex->rank;
+    p.n_peers = ex->world;
+    if (!fused) return p;
+    for (uint32_t g = 0; g < ex->world; ++g) p.peer_qflags[g] = reinterpret_cast<uint32_t *>(ex->peer[g] + ex->qflags_off);
+    p.qflags = reinterpret_cast<const uint32_t *>(ex->local.p + ex->qflags_off);
+    p.gather = ex->local.p + half; p.block_bytes = block;
+    p.m_ids = m_ids; p.m_dist = m_dist; p.m_counts = m_counts;
+    p.ex_world = ex->world; p.ex_rank = ex->rank; p.ex_epoch = epoch;
+    if (!ix->exchange_blocks) {
+        const uint64_t llhalf = ex->ll_off + (epoch & 1) * static_cast<uint64_t>(ex->world) * ex->nq_max * ex->ll_pitch * 128;
+        for (uint32_t g = 0; g < ex->world; ++g) p.peer_ll[g] = ex->peer[g] + llhalf;
+        p.ll_local = ex->local.p + llhalf; p.ll_lines = record_lines(k); p.ll_pitch = ex->ll_pitch;
+        p.ll_nq = static_cast<uint32_t>(ex->nq_max);
+    }
+    return p;
+}
 
 int zvdb_exchange_create(zvdb_exchange **out, int device, uint32_t world, uint32_t rank, uint64_t nq_max, uint32_t k_max) {
     return zvdb_exchange_create_host(out, device, world, rank, nq_max, k_max, 0);
@@ -2222,15 +2181,15 @@ int zvdb_exchange_create_host(zvdb_exchange **out, int device, uint32_t world, u
     ex->qflags_off = ex->flags_off + static_cast<size_t>(8) * kFlagPitch * sizeof(uint32_t);
     ex->nq_max = nq_max;
     ex->ll_off = (ex->qflags_off + static_cast<size_t>(nq_max) * 8 * sizeof(uint32_t) + 255) / 256 * 256;
-    ex->ll_pitch = (2 * k_max + 1 + 29) / 30;
+    ex->ll_pitch = record_lines(k_max);
     ex->qbuf_off = ex->ll_off + 2 * static_cast<size_t>(world) * nq_max * ex->ll_pitch * 128;
     ex->dim_max = dim_max;
     const size_t total = ex->qbuf_off + 2 * static_cast<size_t>(nq_max) * dim_max * sizeof(float);
-    cudaError_t e = cudaMalloc(&ex->local, total);
-    if (e == cudaSuccess) e = cudaMemset(ex->local, 0, total);
-    if (e == cudaSuccess) e = cudaMalloc(&ex->d_peer_flags, 8 * sizeof(uint32_t *));
-    if (e != cudaSuccess) { cudaFree(ex->local); delete ex; ZV_CUDA(e); }
-    ex->peer[rank] = ex->local;
+    cudaError_t e = ex->local.reserve(total);
+    if (e == cudaSuccess) e = cudaMemset(ex->local.p, 0, total);
+    if (e == cudaSuccess) e = ex->d_peer_flags.reserve(8);
+    if (e != cudaSuccess) { delete ex; ZV_CUDA(e); }
+    ex->peer[rank] = ex->local.p;
     *out = ex;
     return ZVDB_OK;
 }
@@ -2240,7 +2199,7 @@ int zvdb_exchange_ipc_handle(zvdb_exchange *ex, void *handle64) {
     static_assert(sizeof(cudaIpcMemHandle_t) == 64, "IPC handle size");
     ZV_CUDA(cudaSetDevice(ex->device));
     cudaIpcMemHandle_t h;
-    ZV_CUDA(cudaIpcGetMemHandle(&h, ex->local));
+    ZV_CUDA(cudaIpcGetMemHandle(&h, ex->local.p));
     std::memcpy(handle64, &h, 64);
     return ZVDB_OK;
 }
@@ -2258,7 +2217,7 @@ int zvdb_exchange_open_peers(zvdb_exchange *ex, const void *handles) {
     }
     uint32_t *pf[8] = {};
     for (uint32_t g = 0; g < ex->world; ++g) pf[g] = reinterpret_cast<uint32_t *>(ex->peer[g] + ex->flags_off);
-    ZV_CUDA(cudaMemcpy(ex->d_peer_flags, pf, sizeof(pf), cudaMemcpyHostToDevice));
+    ZV_CUDA(cudaMemcpy(ex->d_peer_flags.p, pf, sizeof(pf), cudaMemcpyHostToDevice));
     ex->opened = true;
     return ZVDB_OK;
 }
@@ -2269,9 +2228,6 @@ void zvdb_exchange_destroy(zvdb_exchange *ex) {
     cudaDeviceSynchronize();
     for (uint32_t g = 0; g < ex->world; ++g)
         if (g != ex->rank && ex->peer[g]) cudaIpcCloseMemHandle(ex->peer[g]);
-    cudaFree(ex->d_peer_flags);
-    cudaFree(ex->local);
-    cudaFree(ex->d_out_ids); cudaFree(ex->d_out_dist); cudaFree(ex->d_out_counts);
     delete ex;
 }
 
@@ -2280,10 +2236,7 @@ int zvdb_search_batch_exchange(zvdb_index *ix, zvdb_exchange *ex, const float *d
     if (!ix || !ex) return fail(ZVDB_ERR_INVALID, "null argument");
     if (!ex->opened && ex->world > 1) return fail(ZVDB_ERR_INVALID, "exchange: peers not opened");
     if (nq == 0) return ZVDB_OK;
-    if (!d_queries || !out_ids || !out_dist || !out_counts) return fail(ZVDB_ERR_INVALID, "search: null buffer");
-    if (k == 0) return fail(ZVDB_ERR_INVALID, "search: k must be >= 1");
-    if (ef == 0) ef = k;
-    if (ef < k) return fail(ZVDB_ERR_INVALID, "search: ef must be >= k");
+    if (int rc = check_search_args("search", d_queries, out_ids, out_dist, out_counts, k, &ef)) return rc;
     const uint64_t block = zvdb_shard_block_bytes(nq, k);
     if (block * ex->world > ex->cap_bytes) return fail(ZVDB_ERR_INVALID, "exchange: nq * k exceeds the capacity the exchange was created with");
     std::lock_guard<std::mutex> lk(ix->mu);
@@ -2291,44 +2244,32 @@ int zvdb_search_batch_exchange(zvdb_index *ix, zvdb_exchange *ex, const float *d
     ZV_CUDA(cudaSetDevice(ix->device));
     cudaStream_t s = static_cast<cudaStream_t>(stream);
     const uint32_t epoch = ++ex->epoch;
-    const uint64_t half = (epoch & 1) * ex->cap_bytes;           // double buffered: a peer may already be one call ahead
-    uint8_t *blocks[8];
-    for (uint32_t g = 0; g < ex->world; ++g) blocks[g] = ex->peer[g] + half + block * ex->rank;
+    const uint64_t half = (epoch & 1) * ex->cap_bytes;
     const bool empty = ix->g.n == 0 || !ix->g.has_entry;
     if (!empty) {
         int rc = sync_device_locked(ix);
         if (rc) return rc;
     }
-    const bool records = !ix->exchange_blocks;
-    if (!ix->legacy_exchange && nq <= ex->nq_max && (!records || (2 * k + 1 + 29) / 30 <= ex->ll_pitch)) {
+    const bool fused = !ix->legacy_exchange && nq <= ex->nq_max && (ix->exchange_blocks || record_lines(k) <= ex->ll_pitch);
+    const SearchParams xp = exchange_section(ix, ex, epoch, block, k, fused, out_ids, out_dist, out_counts);
+    if (fused) {
         // ONE launch: search, peer stores, per-query flags, and -- one wave behind -- the merge of every query whose
         // flag row is complete (an empty shard runs the same kernel and publishes zero results per query)
-        FusedExchange fx{};
-        for (uint32_t g = 0; g < ex->world; ++g) fx.peer_qflags[g] = reinterpret_cast<uint32_t *>(ex->peer[g] + ex->qflags_off);
-        fx.qflags = reinterpret_cast<const uint32_t *>(ex->local + ex->qflags_off);
-        fx.gather = ex->local + half; fx.block_bytes = block;
-        fx.m_ids = out_ids; fx.m_dist = out_dist; fx.m_counts = out_counts;
-        fx.world = ex->world; fx.rank = ex->rank; fx.epoch = epoch;
-        if (!ix->exchange_blocks) {
-            const uint64_t llhalf = ex->ll_off + (epoch & 1) * static_cast<uint64_t>(ex->world) * ex->nq_max * ex->ll_pitch * 128;
-            for (uint32_t g = 0; g < ex->world; ++g) fx.peer_ll[g] = ex->peer[g] + llhalf;
-            fx.ll_local = ex->local + llhalf; fx.ll_lines = (2 * k + 1 + 29) / 30; fx.ll_pitch = ex->ll_pitch; fx.ll_nq = static_cast<uint32_t>(ex->nq_max);
-        }
-        return launch_search(ix, d_queries, nq, k, ef, nullptr, nullptr, nullptr, nullptr, nullptr, ex->world, ex->rank, s, blocks, ex->world, &fx);
+        return launch_search(ix, d_queries, nq, k, ef, nullptr, nullptr, nullptr, nullptr, nullptr, ex->world, ex->rank, s, &xp);
     }
     if (empty) {
         // an empty shard still publishes count 0 for every query (memset through the peer mappings)
-        for (uint32_t g = 0; g < ex->world; ++g) ZV_CUDA(cudaMemsetAsync(blocks[g] + nq * k * 12, 0, nq * sizeof(uint32_t), s));
+        for (uint32_t g = 0; g < ex->world; ++g) ZV_CUDA(cudaMemsetAsync(xp.peer_blocks[g] + nq * k * 12, 0, nq * sizeof(uint32_t), s));
     } else {
-        int rc = launch_search(ix, d_queries, nq, k, ef, nullptr, nullptr, nullptr, nullptr, nullptr, ex->world, ex->rank, s, blocks, ex->world);
+        int rc = launch_search(ix, d_queries, nq, k, ef, nullptr, nullptr, nullptr, nullptr, nullptr, ex->world, ex->rank, s, &xp);
         if (rc) return rc;
     }
-    exchange_signal_kernel<<<1, 32, 0, s>>>(ex->d_peer_flags, ex->world, ex->rank, kFlagPitch, epoch);
+    exchange_signal_kernel<<<1, 32, 0, s>>>(ex->d_peer_flags.p, ex->world, ex->rank, kFlagPitch, epoch);
     ix->launches++;
     ZV_CUDA(cudaGetLastError());
-    const uint8_t *b = ex->local + half;
+    const uint8_t *b = ex->local.p + half;
     int rc = launch_merge(b + nq * k * 8, b, b + nq * k * 12, block, block, block, ex->world, nq, k, out_dist, out_ids, out_counts, s,
-                          reinterpret_cast<const uint32_t *>(ex->local + ex->flags_off), kFlagPitch, epoch);
+                          reinterpret_cast<const uint32_t *>(ex->local.p + ex->flags_off), kFlagPitch, epoch);
     ix->launches++;
     return rc;
 }
@@ -2338,13 +2279,10 @@ int zvdb_search_batch_exchange_host(zvdb_index *ix, zvdb_exchange *ex, const flo
     if (!ix || !ex) return fail(ZVDB_ERR_INVALID, "null argument");
     if (!ex->opened && ex->world > 1) return fail(ZVDB_ERR_INVALID, "exchange: peers not opened");
     if (nq == 0) return ZVDB_OK;
-    if (!h_queries || !h_ids || !h_dist || !h_counts) return fail(ZVDB_ERR_INVALID, "search: null buffer");
-    if (k == 0) return fail(ZVDB_ERR_INVALID, "search: k must be >= 1");
-    if (ef == 0) ef = k;
-    if (ef < k) return fail(ZVDB_ERR_INVALID, "search: ef must be >= k");
+    if (int rc = check_search_args("search", h_queries, h_ids, h_dist, h_counts, k, &ef)) return rc;
     if (dim == 0 || dim > ex->dim_max || nq > ex->nq_max)
         return fail(ZVDB_ERR_INVALID, "exchange: created without a query buffer for this dim / batch size (zvdb_exchange_create_host)");
-    if (!ix->exchange_blocks && (2 * k + 1 + 29) / 30 > ex->ll_pitch)
+    if (!ix->exchange_blocks && record_lines(k) > ex->ll_pitch)
         return fail(ZVDB_ERR_INVALID, "exchange: k exceeds the k_max the exchange was created with");
     const uint64_t block = zvdb_shard_block_bytes(nq, k);
     if (block * ex->world > ex->cap_bytes) return fail(ZVDB_ERR_INVALID, "exchange: nq * k exceeds the capacity the exchange was created with");
@@ -2359,61 +2297,40 @@ int zvdb_search_batch_exchange_host(zvdb_index *ix, zvdb_exchange *ex, const flo
     }
     cudaStream_t s = static_cast<cudaStream_t>(stream);
     const uint32_t epoch = ++ex->epoch;
-    const uint64_t half = (epoch & 1) * ex->cap_bytes;
     const uint64_t per = (nq + ex->world - 1) / ex->world;                       // queries per slice; rank r owns [r*per, (r+1)*per)
     const uint64_t lo = std::min<uint64_t>(nq, per * ex->rank), hi = std::min<uint64_t>(nq, lo + per);
     const uint64_t qhalf = ex->qbuf_off + (epoch & 1) * ex->nq_max * static_cast<uint64_t>(ex->dim_max) * sizeof(float);
     // (1) this rank's slice of the batch: the only host-to-device bytes of the step on this PCIe link
     if (hi > lo)
-        ZV_CUDA(cudaMemcpyAsync(ex->local + qhalf + lo * dim * sizeof(float), h_queries + lo * dim, (hi - lo) * dim * sizeof(float),
+        ZV_CUDA(cudaMemcpyAsync(ex->local.p + qhalf + lo * dim * sizeof(float), h_queries + lo * dim, (hi - lo) * dim * sizeof(float),
                                 cudaMemcpyHostToDevice, s));
     // (2) results: straight into the caller's buffers when they are page-locked, else through device staging
-    auto mapped = [](const void *ptr, void **dptr) {
-        cudaPointerAttributes a{};
-        if (cudaPointerGetAttributes(&a, ptr) != cudaSuccess) { cudaGetLastError(); return false; }
-        if (a.type != cudaMemoryTypeHost || a.devicePointer == nullptr) return false;
-        *dptr = a.devicePointer;
-        return true;
-    };
     void *di = nullptr, *dd = nullptr, *dc = nullptr;
-    const bool direct = mapped(h_ids, &di) && mapped(h_dist, &dd) && mapped(h_counts, &dc);
+    const bool direct = mapped_device_pointer(h_ids, &di) && mapped_device_pointer(h_dist, &dd) && mapped_device_pointer(h_counts, &dc);
     if (!direct) {
-        if (nq * k > ex->out_cap) {
-            ZV_CUDA(cudaStreamSynchronize(s));
-            cudaFree(ex->d_out_ids); cudaFree(ex->d_out_dist); cudaFree(ex->d_out_counts);
-            ex->d_out_ids = nullptr; ex->d_out_dist = nullptr; ex->d_out_counts = nullptr; ex->out_cap = 0;
-            ZV_CUDA(cudaMalloc(&ex->d_out_ids, nq * k * sizeof(uint64_t)));
-            ZV_CUDA(cudaMalloc(&ex->d_out_dist, nq * k * sizeof(float)));
-            ZV_CUDA(cudaMalloc(&ex->d_out_counts, nq * k * sizeof(uint32_t)));
-            ex->out_cap = nq * k;
+        if (nq * k > ex->d_out_ids.cap || nq > ex->d_out_counts.cap) {
+            ZV_CUDA(cudaStreamSynchronize(s));   // (the staging being replaced may still be read by the previous step's copies)
+            ZV_CUDA(ex->d_out_ids.reserve(nq * k));
+            ZV_CUDA(ex->d_out_dist.reserve(nq * k));
+            ZV_CUDA(ex->d_out_counts.reserve(nq));
         }
-        di = ex->d_out_ids; dd = ex->d_out_dist; dc = ex->d_out_counts;
+        di = ex->d_out_ids.p; dd = ex->d_out_dist.p; dc = ex->d_out_counts.p;
     }
     // (3) ONE launch: search on queries read from their owners, top-k to the owner only, the owner merges its slice
-    uint8_t *blocks[8];
-    for (uint32_t g = 0; g < ex->world; ++g) blocks[g] = ex->peer[g] + half + block * ex->rank;
-    FusedExchange fx{};
+    SearchParams xp = exchange_section(ix, ex, epoch, block, k, true, static_cast<uint64_t *>(di), static_cast<float *>(dd),
+                                       static_cast<uint32_t *>(dc));
     for (uint32_t g = 0; g < ex->world; ++g) {
-        fx.peer_qflags[g] = reinterpret_cast<uint32_t *>(ex->peer[g] + ex->qflags_off);
-        fx.peer_q[g] = reinterpret_cast<const float *>(ex->peer[g] + qhalf);
-        fx.peer_sflags[g] = reinterpret_cast<uint32_t *>(ex->peer[g] + ex->flags_off);
+        xp.peer_q[g] = reinterpret_cast<const float *>(ex->peer[g] + qhalf);
+        xp.peer_sflags[g] = reinterpret_cast<uint32_t *>(ex->peer[g] + ex->flags_off);
     }
-    fx.qflags = reinterpret_cast<const uint32_t *>(ex->local + ex->qflags_off);
-    fx.sflags = reinterpret_cast<const uint32_t *>(ex->local + ex->flags_off); fx.sflag_pitch = kFlagPitch;
-    fx.gather = ex->local + half; fx.block_bytes = block;
-    fx.m_ids = static_cast<uint64_t *>(di); fx.m_dist = static_cast<float *>(dd); fx.m_counts = static_cast<uint32_t *>(dc);
-    fx.world = ex->world; fx.rank = ex->rank; fx.epoch = epoch; fx.q_per = static_cast<uint32_t>(per);
-    if (!ix->exchange_blocks) {
-        const uint64_t llhalf = ex->ll_off + (epoch & 1) * static_cast<uint64_t>(ex->world) * ex->nq_max * ex->ll_pitch * 128;
-        for (uint32_t g = 0; g < ex->world; ++g) fx.peer_ll[g] = ex->peer[g] + llhalf;
-        fx.ll_local = ex->local + llhalf; fx.ll_lines = (2 * k + 1 + 29) / 30; fx.ll_pitch = ex->ll_pitch; fx.ll_nq = static_cast<uint32_t>(ex->nq_max);
-    }
-    int rc = launch_search(ix, nullptr, nq, k, ef, nullptr, nullptr, nullptr, nullptr, nullptr, ex->world, ex->rank, s, blocks, ex->world, &fx);
+    xp.sflags = reinterpret_cast<const uint32_t *>(ex->local.p + ex->flags_off); xp.sflag_pitch = kFlagPitch;
+    xp.q_per = static_cast<uint32_t>(per);
+    int rc = launch_search(ix, nullptr, nq, k, ef, nullptr, nullptr, nullptr, nullptr, nullptr, ex->world, ex->rank, s, &xp);
     if (rc) return rc;
     if (!direct && hi > lo) {
-        ZV_CUDA(cudaMemcpyAsync(h_ids + lo * k, ex->d_out_ids + lo * k, (hi - lo) * k * sizeof(uint64_t), cudaMemcpyDeviceToHost, s));
-        ZV_CUDA(cudaMemcpyAsync(h_dist + lo * k, ex->d_out_dist + lo * k, (hi - lo) * k * sizeof(float), cudaMemcpyDeviceToHost, s));
-        ZV_CUDA(cudaMemcpyAsync(h_counts + lo, ex->d_out_counts + lo, (hi - lo) * sizeof(uint32_t), cudaMemcpyDeviceToHost, s));
+        ZV_CUDA(cudaMemcpyAsync(h_ids + lo * k, ex->d_out_ids.p + lo * k, (hi - lo) * k * sizeof(uint64_t), cudaMemcpyDeviceToHost, s));
+        ZV_CUDA(cudaMemcpyAsync(h_dist + lo * k, ex->d_out_dist.p + lo * k, (hi - lo) * k * sizeof(float), cudaMemcpyDeviceToHost, s));
+        ZV_CUDA(cudaMemcpyAsync(h_counts + lo, ex->d_out_counts.p + lo, (hi - lo) * sizeof(uint32_t), cudaMemcpyDeviceToHost, s));
     }
     return ZVDB_OK;
 }

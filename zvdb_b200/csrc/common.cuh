@@ -40,10 +40,22 @@ __host__ __device__ __forceinline__ uint32_t next_pow2(uint32_t v) {
     return p;
 }
 
+// One device allocation of at least `cap` elements, owned: freed when the buffer goes (move-only). reserve() and
+// free_() release the old memory without a synchronisation, so a buffer that work still in flight reads is only
+// regrown or dropped behind a synchronise.
 template <typename T>
 struct DevBuf {
     T *p = nullptr;
     size_t cap = 0;
+    DevBuf() = default;
+    DevBuf(const DevBuf &) = delete;
+    DevBuf &operator=(const DevBuf &) = delete;
+    DevBuf(DevBuf &&o) noexcept : p(o.p), cap(o.cap) { o.p = nullptr; o.cap = 0; }
+    DevBuf &operator=(DevBuf &&o) noexcept {
+        if (this != &o) { free_(); p = o.p; cap = o.cap; o.p = nullptr; o.cap = 0; }
+        return *this;
+    }
+    ~DevBuf() { free_(); }
     cudaError_t reserve(size_t count) {
         if (count <= cap) return cudaSuccess;
         if (p) cudaFree(p);

@@ -13,6 +13,7 @@
 // building is the reference's sequential unfused f32 sum (this file is compiled with
 // -ffp-contract=off), so the produced graph is the reference's graph.
 #pragma once
+#include <algorithm>
 #include <cstdint>
 #include <cstring>
 #include <cstdlib>
@@ -73,12 +74,41 @@ struct HostGraph {
         rows_uploaded = 0; dirty.clear(); adj_all_dirty = true;
     }
 
+    // d = 0: no dim yet (the first insert fixes it).
     void fix_dim(uint32_t d) {
         dim = d;
         row_floats = (d + 31u) / 32u * 32u;
         const uint64_t target = 16ull << 20;   // 16 MiB chunks
-        uint64_t r = target / (static_cast<uint64_t>(row_floats) * 4u);
-        rows_per_chunk = r < 1 ? 1u : static_cast<uint32_t>(r);
+        rows_per_chunk = d ? static_cast<uint32_t>(std::max<uint64_t>(1, target / (static_cast<uint64_t>(row_floats) * 4u))) : 0;
+    }
+
+    // Chunks covering rows [0, rows): pinned f32 chunks, and for f64 / i32 indexes the typed ones. false when an
+    // allocation fails (the chunks already added stay for the next call).
+    bool reserve_rows(uint64_t rows) {
+        const uint64_t need = (rows + rows_per_chunk - 1) / rows_per_chunk;
+        while (chunks.size() < need) {
+            float *c = nullptr;
+            if (cudaHostAlloc(&c, static_cast<size_t>(rows_per_chunk) * row_floats * sizeof(float),
+                              cudaHostAllocDefault) != cudaSuccess) { cudaGetLastError(); return false; }
+            chunks.push_back(c);
+        }
+        while (dtype != 0 && typed_chunks.size() < need) {
+            unsigned char *c = static_cast<unsigned char *>(std::malloc(static_cast<size_t>(rows_per_chunk) * dim * elem_size()));
+            if (!c) return false;
+            typed_chunks.push_back(c);
+        }
+        return true;
+    }
+    // f(r, end) for each run [r, end) of rows [r0, r1) that lies in one chunk (contiguous in memory, in both the f32
+    // and the typed chunks); stops at, and returns, the first nonzero result.
+    template <typename F>
+    int for_each_span(uint64_t r0, uint64_t r1, F &&f) const {
+        for (uint64_t r = r0; r < r1;) {
+            const uint64_t end = std::min<uint64_t>(r1, (r / rows_per_chunk + 1) * rows_per_chunk);
+            if (int rc = f(r, end)) return rc;
+            r = end;
+        }
+        return 0;
     }
 
     const float *point(uint64_t id) const {
@@ -203,20 +233,8 @@ struct HostGraph {
         const uint64_t id = n;                                                   // :77
         const uint32_t lv = forced_level >= 0 ? static_cast<uint32_t>(forced_level > 31 ? 31 : forced_level)
                                               : random_level();                  // :78
-        if (id / rows_per_chunk >= chunks.size()) {
-            float *c = nullptr;
-            if (cudaHostAlloc(&c, static_cast<size_t>(rows_per_chunk) * row_floats * sizeof(float),
-                              cudaHostAllocDefault) != cudaSuccess) { cudaGetLastError(); return 1; }
-            chunks.push_back(c);
-        }
-        if (dtype != 0) {
-            if (id / rows_per_chunk >= typed_chunks.size()) {
-                unsigned char *c = static_cast<unsigned char *>(std::malloc(static_cast<size_t>(rows_per_chunk) * dim * elem_size()));
-                if (!c) return 1;
-                typed_chunks.push_back(c);
-            }
-            std::memcpy(const_cast<void *>(typed_point(id)), typed, static_cast<size_t>(dim) * elem_size());
-        }
+        if (!reserve_rows(id + 1)) return 1;
+        if (dtype != 0) std::memcpy(const_cast<void *>(typed_point(id)), typed, static_cast<size_t>(dim) * elem_size());
         const size_t upper_before = upper.size();
         try {
             adj0.resize((id + 1) * m, kInvalidId);
@@ -282,13 +300,7 @@ struct HostGraph {
             level.resize(n0 + count, 0);
             upper_off.resize(n0 + count, ~0ull);
         } catch (const std::bad_alloc &) { truncate(n0); return 1; }
-        const uint64_t need = (n0 + count + rows_per_chunk - 1) / rows_per_chunk;
-        while (chunks.size() < need) {
-            float *c = nullptr;
-            if (cudaHostAlloc(&c, static_cast<size_t>(rows_per_chunk) * row_floats * sizeof(float),
-                              cudaHostAllocDefault) != cudaSuccess) { cudaGetLastError(); truncate(n0); return 1; }
-            chunks.push_back(c);
-        }
+        if (!reserve_rows(n0 + count)) { truncate(n0); return 1; }
         for (uint64_t r = 0; r < count; ++r) store_row(point_mut(n0 + r), pts + r * dim);
         n = n0 + count;
         return 0;

@@ -74,7 +74,7 @@ __global__ void arena_to_sq8_kernel(uint32_t *__restrict__ dst, const float4 *__
 //        codes [cap_rows][row_floats] (the kernels find the codebook in front of the codes).
 // Rows [0, covered) of it are current.
 struct RowCopy {
-    unsigned char *d = nullptr;
+    DevBuf<unsigned char> d;
     uint64_t covered = 0;
     bool trained = false;           // cb belongs to the contents (else the next SQ8 search trains it)
     std::vector<float> cb;          // the SQ8 codebook as on the device, [2][row_floats]
@@ -83,9 +83,9 @@ struct RowCopy {
 
     // Capacity growth: the copy is sized like the arena, so it goes; the next search rebuilds it (SQ8: same codebook).
     int drop() {
-        if (!d) return ZVDB_OK;
+        if (!d.p) return ZVDB_OK;
         ZV_CUDA(cudaDeviceSynchronize());
-        cudaFree(d); d = nullptr; covered = 0;
+        d.free_(); covered = 0;
         return ZVDB_OK;
     }
     // The contents were replaced: nothing is covered, and the next SQ8 search trains a codebook for them.
@@ -97,13 +97,13 @@ struct RowCopy {
     // so the next search trains one, and leaving SQ8 leaves none to read back. Searches enqueued on caller streams may
     // still read what changes here.
     int set_format(int from, int to, int device) {
-        const bool free_copy = d && from != to;
-        if (free_copy || (d && trained)) {
+        const bool free_copy = d.p && from != to;
+        if (free_copy || (d.p && trained)) {
             ZV_CUDA(cudaSetDevice(device));
             ZV_CUDA(cudaDeviceSynchronize());
         }
-        if (free_copy) { cudaFree(d); d = nullptr; }
-        if (!d || to != kRowF16) covered = 0;
+        if (free_copy) d.free_();
+        if (!d.p || to != kRowF16) covered = 0;
         trained = false; cb.clear();
         return ZVDB_OK;
     }
@@ -145,23 +145,23 @@ struct RowCopy {
                     cb[i] = (hi - lo) / 255.0f;           // (built without contraction: two IEEE operations)
                     cb[rf + i] = lo;
                 }
-                trained = true; covered = 0; upload = d != nullptr;   // an existing copy is re-encoded below
+                trained = true; covered = 0; upload = d.p != nullptr;   // an existing copy is re-encoded below
             }
         }
-        if (bad_row == ~0u && !d) {                       // (first search in the format, or after capacity growth)
-            ZV_CUDA(cudaMalloc(&d, sq8 ? 8ull * rf + cap_rows * rf : cap_rows * rf * 2));
+        if (bad_row == ~0u && !d.p) {                     // (first search in the format, or after capacity growth)
+            ZV_CUDA(d.reserve(sq8 ? 8ull * rf + cap_rows * rf : cap_rows * rf * 2));
             covered = 0; upload = sq8;
         }
-        if (upload) ZV_CUDA(cudaMemcpyAsync(d, cb.data(), cb.size() * sizeof(float), cudaMemcpyHostToDevice, s));
+        if (upload) ZV_CUDA(cudaMemcpyAsync(d.p, cb.data(), cb.size() * sizeof(float), cudaMemcpyHostToDevice, s));
         if (bad_row == ~0u && covered < n_dev) {
             const uint64_t total = (n_dev - covered) * row_chunks;
             const unsigned blocks = static_cast<unsigned>(std::min<uint64_t>((total + 255) / 256, static_cast<uint64_t>(num_sms) * 8));
             const float4 *src = reinterpret_cast<const float4 *>(arena);
             if (sq8)
-                arena_to_sq8_kernel<<<blocks, 256, 0, s>>>(reinterpret_cast<uint32_t *>(d + 8ull * rf), src, reinterpret_cast<const float4 *>(d),
+                arena_to_sq8_kernel<<<blocks, 256, 0, s>>>(reinterpret_cast<uint32_t *>(d.p + 8ull * rf), src, reinterpret_cast<const float4 *>(d.p),
                                                            covered, n_dev, row_chunks, bad.p);
             else
-                arena_to_f16_kernel<<<blocks, 256, 0, s>>>(reinterpret_cast<uint2 *>(d), src, covered, n_dev, row_chunks, bad.p);
+                arena_to_f16_kernel<<<blocks, 256, 0, s>>>(reinterpret_cast<uint2 *>(d.p), src, covered, n_dev, row_chunks, bad.p);
             launches++;
             ZV_CUDA(cudaGetLastError());
             ZV_CUDA(cudaMemcpyAsync(&bad_row, bad.p, sizeof bad_row, cudaMemcpyDeviceToHost, s));
@@ -179,12 +179,10 @@ struct RowCopy {
 
     // The rows a search in format ROWF gathers (SearchParams::arena16 / arena8).
     template <int ROWF> const RowChunk<ROWF> *search_rows(uint32_t row_floats) const {
-        return reinterpret_cast<const RowChunk<ROWF> *>(ROWF == kRowSQ8 ? d + 8ull * row_floats : d);
+        return reinterpret_cast<const RowChunk<ROWF> *>(ROWF == kRowSQ8 ? d.p + 8ull * row_floats : d.p);
     }
     // The SQ8 codebook of the contents, [2][row_floats] (scales, then offsets), or nullptr when none is trained.
     const float *codebook() const { return trained ? cb.data() : nullptr; }
-
-    void release() { cudaFree(d); d = nullptr; bad.free_(); minmax.free_(); }
 };
 
 }  // namespace zvdb
